@@ -2,7 +2,7 @@
 """MPC solves/sec of the B200 path on the BASELINE.json workloads.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config c1|c2|c3|c4|c5] [--batch B]
-                    [--scaling weak|strong] [--impl reference] [--no-cpu-baseline]
+                    [--scaling weak|strong] [--impl reference] [--no-cpu-baseline] [--dump-outputs DIR]
 
 Default = configs[2] (C3): 4096 independent CaltechACN 54-EVSE x 288-period instances per GPU.  A step = one pass of the
 whole hot path over the batch, as SURVEY.md 8(d) defines a solve: pack -> iterate (to the certified 1e-4 gap) ->
@@ -20,6 +20,9 @@ polish -> postprocess (continuous pilot projection).
              tests/golden/make_bench_golden.py (objective within 1e-4 |f*|, violation, energy, bounds).
 * `--impl reference`: the CPU oracle (float64 restatement of the reference's cvxpy/ECOS path, which cannot run here:
              cvxpy / ECOS / acnportal are not installed) on ALL host cores, one persistent pool.
+* `--dump-outputs DIR`: after the timed steps, what the last timed step of `value` handed to its caller (C4: the last
+             control step of the replay) is written as DIR/<name>.npy, float32 or float64, rank 0's instances.  The
+             inputs depend on the arguments only, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -334,6 +337,39 @@ def latency_lines():
     return out
 
 
+# ----------------------------------------------------------------------------------------------- --dump-outputs
+DUMP_BYTES = 64 << 20  # what --dump-outputs writes in all, at most
+
+
+def dump_outputs(out_dir, outs, seed=0):
+    """Writes `outs` (name -> tensor whose first axis is the instance) as out_dir/<name>.npy: float32 where the tensor is
+    float32, float64 otherwise.  When that would exceed DUMP_BYTES, every array keeps the same fixed, seeded sample of
+    instances; instance.npy holds the batch index of each instance written."""
+    import torch
+
+    B = len(next(iter(outs.values())))
+    itemsize = {name: 4 if t.dtype == torch.float32 else 8 for name, t in outs.items()}
+    per_instance = 8 + sum(itemsize[name] * (t.numel() // B) for name, t in outs.items())
+    k = min(B, (DUMP_BYTES - 4096) // per_instance)  # (4096: room for the .npy headers)
+    idx = np.arange(B) if k == B else np.sort(np.random.default_rng(seed).choice(B, k, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "instance.npy"), idx.astype(np.float64))
+    for name, t in outs.items():
+        a = t[torch.from_numpy(idx).to(t.device)].cpu().numpy()
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float32 if itemsize[name] == 4 else np.float64))
+
+
+def batch_outputs(bac):
+    """The device results of the last call on a BatchedAdaptiveCharging, the fields of its BatchResult."""
+    import torch
+
+    def cat(field):
+        return torch.cat([field(ch) for ch in bac.chunks])
+
+    return dict(pilots=cat(lambda ch: ch.pilots), status=cat(lambda ch: ch.status), iters=cat(lambda ch: ch.iters),
+                T=cat(lambda ch: ch.packed["T"]), stats=cat(lambda ch: ch.stats))
+
+
 # ----------------------------------------------------------------------------------------------- GPU arm
 def main():
     ap = argparse.ArgumentParser()
@@ -347,7 +383,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-latency", action="store_true")
     ap.add_argument("--groups", type=int, default=8, help="c4: independent groups of sites per GPU, each on its own stream")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; the reference arm has none to write")
     if args.batch is None:
         args.batch = CONFIGS[args.config]["batch"]
     if args.config == "c4":
@@ -432,6 +472,9 @@ def main():
     barrier()
     clk = clocks.stop() if rank == 0 else None
     ms = sharding.max_over_ranks(ms, dev)
+    if args.dump_outputs and rank == 0:
+        # (before the isolated steps below, which solve again into res_a)
+        dump_outputs(args.dump_outputs, batch_outputs(res_a if (steps - 1) % 2 == 0 else res_b))
     # the solve kernel alone: isolated steps (one stream, nothing else in flight), CUDA events on the stream the kernel is
     # launched on around acb_solve_batch, and around the whole step for the kernel's share of it
     iso_solve, iso_step = [], []
@@ -591,6 +634,12 @@ def run_c4(args, world, rank, local, dev, barrier):
     barrier()
     clk = clocks.stop() if rank == 0 else None
     ms = sharding.max_over_ranks(ms, dev)
+    if args.dump_outputs and rank == 0:
+        # the last control step of every site of the rank (the groups are consecutive ranges of sites) and the peaks so far
+        outs = [batch_outputs(rp._bac) for rp in rps]
+        outs = {k: torch.cat([o[k] for o in outs]) for k in outs[0]}
+        outs["prev_peak"] = torch.cat([rp._d["prev_peak"] for rp in rps])
+        dump_outputs(args.dump_outputs, outs)
     s1 = summary()
     summ = torch.tensor([s1["site_steps"] - s0["site_steps"], s1["unsolved"] - s0["unsolved"], s1["iters"] - s0["iters"], t_enq],
                         dtype=torch.float64, device=dev)
