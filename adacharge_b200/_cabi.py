@@ -14,10 +14,11 @@ LIB_PATH = os.path.join(_HERE, "libadacharge_b200.so")
 ACB_SOC, ACB_LINEAR = 0, 1
 ACB_SOLVED, ACB_MAX_ITER, ACB_INFEASIBLE, ACB_NUMERICAL, ACB_INVALID = 0, 1, 2, 3, 4
 ACB_NSTATS = 8
+ACB_PILOTS_DISCRETE, ACB_PILOTS_REALLOCATE = 1, 2  # acb_quantize_pilots modes
 EXPORTS = [
     "acb_site_create", "acb_site_destroy", "acb_site_dims", "acb_site_max_horizon", "acb_default_options",
     "acb_solve_batch", "acb_charging_rate_bounds", "acb_project_continuous", "acb_project_discrete",
-    "acb_reallocate", "acb_constraints_feasible", "acb_min_rate_admission", "acb_pack_sessions", "acb_preprocess_sessions", "acb_fleet_sessions", "acb_fleet_apply", "acb_last_error", "acb_version",
+    "acb_reallocate", "acb_quantize_pilots", "acb_constraints_feasible", "acb_min_rate_admission", "acb_pack_sessions", "acb_preprocess_sessions", "acb_fleet_sessions", "acb_fleet_apply", "acb_last_error", "acb_version",
 ]
 ACB_MAX_COMPONENTS = 16
 # acb_objective.kind values (include/adacharge_b200.h)
@@ -97,6 +98,7 @@ def lib():
     L.acb_project_continuous.argtypes = [_P, _P, _P, C.c_int, C.c_int, _P]
     L.acb_project_discrete.argtypes = [_P, _P, _P, C.c_int, C.c_int, _P]
     L.acb_reallocate.argtypes = [_P, C.c_int, _P, _P, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P]
+    L.acb_quantize_pilots.argtypes = [_P, C.c_int, C.POINTER(Sessions), C.c_double, C.POINTER(Batch), _P, _P]
     L.acb_constraints_feasible.argtypes = [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P]
     L.acb_min_rate_admission.argtypes = [_P, C.c_int, C.c_int, _P, _P, _P, _P, _P]
     L.acb_preprocess_sessions.argtypes = [_P, C.POINTER(Sessions), C.c_int, _P, _P]

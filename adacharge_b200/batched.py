@@ -1,12 +1,14 @@
 """Batched form of the per-step MPC path: many independent instances of ONE site per call.
 
 ``BatchedAdaptiveCharging.schedule(sessions, ...)`` is what ``AdaptiveSchedulingAlgorithm.schedule``
-(reference adacharge/adacharge.py:135-193: build -> solve -> project_into_continuous_feasible_pilots -> max(., 0))
+(reference adacharge/adacharge.py:135-193: build -> solve -> project the pilots -> max(., 0))
 does for one site and one control step, for B instances at once (sites, scenarios, sweep points): the caller hands
 over the raw session tables and the interface quantities as host arrays; this class stages them in pinned memory,
 copies them to the device, packs them there (``acb_pack_sessions``: horizon, energy rows, the ObjectiveComponent
 list -> cost vectors, reference aco.py:200-284, 363-408), solves (``acb_solve_batch``, whose epilogue also does the
-continuous pilot projection, postprocessing.py:77-94) and copies the float64 pilots back.  The batch is cut into
+continuous pilot projection, postprocessing.py:77-94) and copies the float64 pilots back.  With ``quantize`` (and
+``reallocate``) the solve skips that projection and one more launch (``acb_quantize_pilots``) writes the discrete pilots
+of project_into_discrete_feasible_pilots (postprocessing.py:97-118) or diff_based_reallocation (:189-258) instead.  The batch is cut into
 chunks on their own streams so that the copies of one chunk overlap the solve of another.
 
 Only the built-in objective functions are packed on the device (by identity, as the drop-in class recognises them);
@@ -31,6 +33,20 @@ _KIND_OF = {
 }
 SESSION_FIELDS = (("station", np.int32), ("arrival_offset", np.int32), ("remaining_time", np.int32),
                   ("remaining_demand", np.float64), ("min_rate", np.float64), ("max_rate", np.float64))
+
+
+def pilot_mode(quantize, reallocate, infrastructure) -> int:
+    """The acb_quantize_pilots mode for AdaptiveSchedulingAlgorithm's `quantize` / `reallocate` flags (0 = continuous
+    pilots), with the reference's rule (ada.py:101-105) and a check that every EVSE has its allowable pilots."""
+    if reallocate and not quantize:
+        raise ValueError("reallocate cannot be true without quantize. Otherwise there is nothing to reallocate :).")
+    if not quantize:
+        return 0
+    ap = getattr(infrastructure, "allowable_pilots", None)
+    n = len(infrastructure.station_ids)
+    if ap is None or len(ap) != n or any(a is None or len(a) == 0 for a in ap):
+        raise ValueError("quantize=True needs allowable_pilots for every EVSE of the infrastructure")
+    return _cabi.ACB_PILOTS_REALLOCATE if reallocate else _cabi.ACB_PILOTS_DISCRETE
 
 
 def objective_components(objective: Sequence[aco.ObjectiveComponent]):
@@ -58,7 +74,7 @@ def objective_components(objective: Sequence[aco.ObjectiveComponent]):
 
 @dataclass
 class BatchResult:
-    pilots: np.ndarray   # [B, N, Tp] float64, max(min(rates, max_pilot), 0); columns >= T[b] are zero
+    pilots: np.ndarray   # [B, N, Tp] float64, the pilots schedule() returns per EVSE (continuous or quantised); columns >= T[b] are zero
     status: np.ndarray   # [B] acb status
     iters: np.ndarray    # [B]
     T: np.ndarray        # [B] horizon of each instance (aco.py:243-245)
@@ -101,7 +117,7 @@ class _Chunk:
             d["sess_quad"] = mk((B, S), f32)
         self.packed = d
         self.rates = mk((B, N, Tp), f32)
-        self.pilots = mk((B, N, Tp), torch.float64)
+        self.pilots = mk((B, N, Tp), torch.float64)  # continuous: the solve's epilogue; quantised: acb_quantize_pilots
         self.status, self.iters = mk((B,), i32), mk((B,), i32)
         self.stats = mk((B, _cabi.ACB_NSTATS), f32)
         self.work = mk((B, N + max(R, 1), Tp), f32)
@@ -112,7 +128,8 @@ class _Chunk:
         b.B, b.Tp, b.S_max, b.multi_session = B, Tp, S, int(owner.multi_session)
         for k, t in d.items():
             setattr(b, k, p(t))
-        b.work, b.rates, b.pilots, b.status, b.iters, b.stats = p(self.work), p(self.rates), p(self.pilots), p(self.status), p(self.iters), p(self.stats)
+        b.work, b.rates, b.status, b.iters, b.stats = p(self.work), p(self.rates), p(self.status), p(self.iters), p(self.stats)
+        b.pilots = None if owner.pilot_mode else p(self.pilots)  # quantised pilots are not first projected continuously
         self.batch = b
         s = _cabi.Sessions()
         s.B, s.S_max = B, S
@@ -145,12 +162,15 @@ class BatchedAdaptiveCharging:
         multi_session: an EVSE may hold more than one session within the horizon.
         demand_charge: $/kW (interface.get_demand_charge) when it is the same for every instance; per-instance values
             are passed to ``schedule``.
+        quantize, reallocate: as AdaptiveSchedulingAlgorithm's (ada.py:101-113, 177-190): pilots rounded down into each
+            EVSE's allowable set (every EVSE needs one), and with ``reallocate`` the first period's rounding loss given
+            back greedily.  Bit-identical to the drop-in class with the same flags.
     """
 
     def __init__(self, objective: List[aco.ObjectiveComponent], infrastructure, period, batch: int, max_sessions: int, horizon: int,
                  constraint_type="SOC", enforce_energy_equality=False, peak_limit=False, multi_session=False, demand_charge=0.0,
                  per_instance_demand_charge=False, solver_options: Optional[dict] = None, device=None, chunks: int = 4,
-                 enforce_pilot_limit=True, estimate_max_rate=False):
+                 enforce_pilot_limit=True, estimate_max_rate=False, quantize=False, reallocate=False):
         from .interface import InfrastructureInfo
 
         if isinstance(infrastructure, dict):
@@ -158,6 +178,7 @@ class BatchedAdaptiveCharging:
             infrastructure = InfrastructureInfo(np.asarray(i["constraint_matrix"]), np.asarray(i["constraint_limits"]), np.asarray(i["phases"]),
                                                 np.asarray(i["voltages"]), i["constraint_ids"], i["station_ids"], np.asarray(i["max_pilot"]),
                                                 np.asarray(i["min_pilot"]), i.get("allowable_pilots"), i.get("is_continuous"))
+        self.pilot_mode = pilot_mode(quantize, reallocate, infrastructure)
         self.components = objective_components(objective)
         kinds = {k for k, _, _ in self.components}
         K = _cabi.OBJ_KIND
@@ -192,9 +213,10 @@ class BatchedAdaptiveCharging:
         self.h2d_bytes = sum(c.h2d_bytes for c in self.chunks)
         self.d2h_bytes = sum(t.numel() * t.element_size() for t in (self.host_pilots, self.host_status, self.host_iters, self.host_T, self.host_stats))
         # own kernels per call and chunk: the packer + the solve (three launches when phased: solve, relaunch list, solve;
-        # the general path launches per phase and is not counted here)
+        # the general path launches per phase and is not counted here) + the preprocessing + the quantised pilots
         phased = self.options.phase_iters > 0 and self.options.phase_iters < self.options.max_iter
-        self.kernel_launches_per_call = len(self.chunks) * (1 + (3 if phased else 1) + int(self.enforce_pilot_limit or self.estimate_max_rate))
+        self.kernel_launches_per_call = len(self.chunks) * (1 + (3 if phased else 1) + int(self.enforce_pilot_limit or self.estimate_max_rate)
+                                                            + int(self.pilot_mode != 0))
 
     # ------------------------------------------------------------------------------------------------
     def _stage(self, ch: _Chunk, arrays: Dict[str, np.ndarray]):
@@ -221,7 +243,7 @@ class BatchedAdaptiveCharging:
                 d[...] = a[ch.lo:ch.hi]
 
     def enqueue(self, ch: _Chunk, from_device_raw=False, events=None):
-        """H2D of the raw arrays (unless they are already on the device), pack, solve, D2H — on the chunk's stream.
+        """H2D of the raw arrays (unless they are already on the device), pack, solve, quantise (if asked), D2H — on the chunk's stream.
         `events`: a list that receives a (start, end) pair of CUDA events around the solve launch(es)."""
         L = _cabi.lib()
         st = C.c_void_p(ch.stream.cuda_stream)
@@ -241,6 +263,9 @@ class BatchedAdaptiveCharging:
             if events is not None:
                 ev[1].record(ch.stream)
                 events.append(ev)
+            if self.pilot_mode:
+                _cabi.check(L.acb_quantize_pilots(self.site.handle, self.pilot_mode, C.byref(ch.sessions), float(self.period), C.byref(ch.batch),
+                                                  engine._ptr(ch.pilots), st), "acb_quantize_pilots")
             if not from_device_raw:
                 self.host_pilots[ch.lo:ch.hi].copy_(ch.pilots, non_blocking=True)
                 self.host_status[ch.lo:ch.hi].copy_(ch.status, non_blocking=True)
@@ -354,4 +379,4 @@ def sessions_to_arrays(session_lists, infrastructure, S_max: Optional[int] = Non
     return out
 
 
-__all__ = ["BatchedAdaptiveCharging", "BatchResult", "sessions_to_arrays", "objective_components"]
+__all__ = ["BatchedAdaptiveCharging", "BatchResult", "sessions_to_arrays", "objective_components", "pilot_mode"]

@@ -58,6 +58,13 @@ struct SiteDev {
     const double* volt;     // [N] voltages (V), float64 for the device packer
     const int* allow_off;   // [N+1]
     const double* allow_vals;
+    // sparsity of the SOC rows (entries where a_cos or a_sin is nonzero), for the reallocation greedy
+    const int* evse_row_off;  // [N+1] rows with a nonzero coefficient at EVSE i: evse_rows[evse_row_off[i] ..]
+    const int* evse_rows;
+    const int* row_col_off;   // [M+1] nonzero columns of row j, ascending: row_cols[row_col_off[j] ..]
+    const int* row_cols;
+    const double* row_cos;    // a_cos / a_sin at those entries
+    const double* row_sin;
 };
 
 struct acb_site {

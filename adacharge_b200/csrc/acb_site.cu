@@ -311,6 +311,24 @@ extern "C" int acb_site_create(acb_site** out, int device, int N, int M, const d
     }
     UP(acos_, a_cos) UP(asin_, a_sin) UP(lim64, limits) UP(mp, max_pilot) UP(aoff, allow_off) UP(avals, allow_vals)
     {
+        // CSR of the nonzero entries of the SOC rows, by row (columns ascending) and by EVSE (rows ascending)
+        std::vector<int> rc_off(M + 1, 0), rc_col, er_cnt(N + 1, 0), er_off(N + 1, 0), er_rows;
+        std::vector<double> rc_cos, rc_sin;
+        for (int j = 0; j < M; ++j) {
+            for (int i = 0; i < N; ++i) {
+                const double c = acos_[(size_t)j * N + i], sn = asin_[(size_t)j * N + i];
+                if (c != 0.0 || sn != 0.0) { rc_col.push_back(i); rc_cos.push_back(c); rc_sin.push_back(sn); ++er_cnt[i + 1]; }
+            }
+            rc_off[j + 1] = (int)rc_col.size();
+        }
+        for (int i = 0; i < N; ++i) er_off[i + 1] = er_off[i] + er_cnt[i + 1];
+        er_rows.resize(rc_col.size());
+        std::vector<int> fill(er_off.begin(), er_off.end() - 1);
+        for (int j = 0; j < M; ++j)
+            for (int p = rc_off[j]; p < rc_off[j + 1]; ++p) er_rows[fill[rc_col[p]]++] = j;
+        UP(er_off, evse_row_off) UP(er_rows, evse_rows) UP(rc_off, row_col_off) UP(rc_col, row_cols) UP(rc_cos, row_cos) UP(rc_sin, row_sin)
+    }
+    {
         std::vector<double> volt64(voltages, voltages + N);
         UP(volt64, volt)
     }

@@ -39,12 +39,13 @@ class FleetStats:
 
 class FleetReplay:
     """`n_sites` copies of one site, `days` seeded days of EVs each (day d of site s is
-    `synthetic_day(seed0 + s * days + d)` shifted by d * steps_per_day periods)."""
+    `synthetic_day(seed0 + s * days + d)` shifted by d * steps_per_day periods).  `quantize` / `reallocate` are
+    AdaptiveSchedulingAlgorithm's flags: the EVs are charged with pilots from each EVSE's allowable set."""
 
     def __init__(self, infra: Dict, objective: List[ObjectiveComponent], n_sites: int, steps_per_day: int = 288, days: int = 1,
                  period: float = 5, prices: Optional[np.ndarray] = None, demand_charge: float = 15.51, seed0: int = 0,
                  warm_start: bool = True, solver_options: Optional[dict] = None, device=None, mean_sessions: int = 40,
-                 Tp: int = 288, site_offset: int = 0):
+                 Tp: int = 288, site_offset: int = 0, quantize: bool = False, reallocate: bool = False):
         self.infra, self.objective, self.n_sites, self.period = infra, objective, n_sites, period
         self.steps_per_day, self.days, self.steps = steps_per_day, days, steps_per_day * days
         self.warm_start, self.device, self.Tp = warm_start, device, Tp
@@ -62,6 +63,9 @@ class FleetReplay:
             np.asarray(infra["constraint_matrix"]), np.asarray(infra["constraint_limits"]), np.asarray(infra["phases"]),
             self.volt, infra["constraint_ids"], infra["station_ids"], np.asarray(infra["max_pilot"]), np.asarray(infra["min_pilot"]),
             infra.get("allowable_pilots"), infra.get("is_continuous"))
+        from .batched import pilot_mode
+
+        self.pilot_mode = pilot_mode(quantize, reallocate, self.info)
         cols = {k: [] for k in ("site", "station", "arr", "dep", "req", "maxrate")}
         for s in range(n_sites):
             for d in range(days):
@@ -195,7 +199,7 @@ class FleetReplay:
         if self.warm_start and self._prev is not None:
             pb.warm = self._shifted_warm(idx_d, s_d, pos_d, pb)
         pb.upload().solve(self.options)
-        pilots = engine.project_continuous(self.site, pb.rates.to(torch.float64))  # pp.py:77-94 on device
+        pilots = self._project(pb.rates.to(torch.float64), h, idx, s, pos)
         first = pilots[:, :, 0].contiguous().cpu().numpy()
         it, stt = pb.iters.cpu().numpy(), pb.status.cpu().numpy()
         ev1.record()
@@ -217,6 +221,25 @@ class FleetReplay:
         st_.device_ms.append(ev0.elapsed_time(ev1))
         st_.host_ms.append((t1 - t0 + time.perf_counter() - t2) * 1e3)
         return first
+
+    def _project(self, rates, h, idx, s, pos):
+        """The pilots of the step's schedule (pp.py:77-118, 189-258 on the device)."""
+        if self.pilot_mode:
+            pilots = self._project_quantized(rates, h, idx, s, pos)
+            pilots[torch.from_numpy(h["n_sessions"] == 0).to(pilots.device)] = 0.0  # idle sites: no pilots (as acb_quantize_pilots)
+            return pilots
+        return engine.project_continuous(self.site, rates)
+
+    def _project_quantized(self, rates, h, idx, s, pos):
+        if self.pilot_mode == _cabi.ACB_PILOTS_REALLOCATE:
+            # sessions in slot order (the EV table's), all starting now; ramp = interface.remaining_amp_periods
+            B, S_ = h["sess_row"].shape
+            ramp, max0 = np.zeros((B, S_)), np.zeros((B, S_))
+            rem = self.ev_req[idx] - self.ev_dlv[idx]
+            ramp[s, pos] = rem * 1000 / self.volt[self.ev_station[idx]] * (60 / self.period)
+            max0[s, pos] = self.ev_max[idx]
+            return engine.reallocate(self.site, 1, rates, h["n_sessions"], h["sess_row"], h["sess_start"], ramp, max0)
+        return engine.project_discrete(self.site, rates)
 
     def _shifted_warm(self, idx_d, s_d, pos_d, pb):
         """Previous state shifted by one period (column t of the new problem is column t+1 of the
@@ -260,7 +283,8 @@ class DeviceFleetReplay(FleetReplay):
     the energy delivered, the previous peaks and the per-EV warm-start multipliers stay in device arrays; a step is four
     launches on one stream -- active sessions (acb_fleet_sessions), packing (acb_pack_sessions), the warm-started solve
     whose prologue reads the previous state one column ahead (acb_batch.warm_shift) and whose epilogue projects the
-    pilots, and the simulator update (acb_fleet_apply) -- with no host synchronisation between steps.  Same schedules,
+    pilots, and the simulator update (acb_fleet_apply) -- with no host synchronisation between steps.  Quantised pilots
+    take a fifth launch (acb_quantize_pilots) between the solve and the update.  Same schedules,
     bit for bit, as FleetReplay (tests/test_gpu_replay.py)."""
 
     def __init__(self, *a, **kw):
@@ -273,7 +297,8 @@ class DeviceFleetReplay(FleetReplay):
         opts = {**REPLAY_SOLVER_DEFAULTS, **(kw.get("solver_options") or {})}
         self._bac = BatchedAdaptiveCharging(self.objective, self.info, self.period, batch=self.n_sites, max_sessions=self.N, horizon=self.Tp,
                                             demand_charge=self.demand_charge, solver_options=opts, device=self.device, chunks=1,
-                                            enforce_pilot_limit=False)
+                                            enforce_pilot_limit=False, quantize=self.pilot_mode != 0,
+                                            reallocate=self.pilot_mode == _cabi.ACB_PILOTS_REALLOCATE)
         if self._bac.Tp != self.Tp:
             raise ValueError(f"Tp = {self.Tp} is not a padded horizon of the solve path")
         self.site = self._bac.site
@@ -332,8 +357,14 @@ class DeviceFleetReplay(FleetReplay):
         _cabi.check(L.acb_fleet_sessions(self.site.handle, C.byref(self._fleet), t, C.byref(ch.sessions), p(d["sess_ev"]), p(d["warm_mu"]), st), "acb_fleet_sessions")
         _cabi.check(L.acb_pack_sessions(self.site.handle, C.byref(ch.sessions), C.byref(o), C.byref(b), p(ch.flags), st), "acb_pack_sessions")
         _cabi.check(L.acb_solve_batch(self.site.handle, C.byref(b), C.byref(self._bac.options), st), "acb_solve_batch")
+        if self.pilot_mode:  # the solve skipped the continuous projection (batch.pilots NULL); acb_fleet_apply reads batch.pilots
+            _cabi.check(L.acb_quantize_pilots(self.site.handle, self.pilot_mode, C.byref(ch.sessions), float(self.period), C.byref(b), p(ch.pilots), st),
+                        "acb_quantize_pilots")
+            b.pilots = p(ch.pilots)
         _cabi.check(L.acb_fleet_apply(self.site.handle, C.byref(self._fleet), t, float(self.period), C.byref(b), p(d["sess_ev"]),
                                       p(d["first"]) if want_first else None, p(d["stats"]), st), "acb_fleet_apply")
+        if self.pilot_mode:
+            b.pilots = None
         self._k = 1 - self._k
         self._started = True
         return d["first"].cpu().numpy() if want_first else None

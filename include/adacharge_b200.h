@@ -19,6 +19,8 @@
  *   acb_project_discrete        project_into_discrete_feasible_pilots     postprocessing.py:97-118
  *   acb_reallocate              index_based_reallocation / diff_based_reallocation
  *                                                                 postprocessing.py:121-258
+ *   acb_quantize_pilots         project_into_discrete_feasible_pilots / diff_based_reallocation for a solved batch
+ *                                                                 postprocessing.py:97-118, 189-258
  *   acb_constraints_feasible    infrastructure_constraints_feasible       utils.py:5-12
  *   acb_pack_sessions           the host work before the solver: horizon, energy rows, build_objective
  *                                                                 ...optimization.py:114-122, 200-218, 243-245, 363-408
@@ -161,7 +163,8 @@ typedef struct acb_batch {
     /* results */
     float* rates;                /* [B][N][Tp] */
     double* pilots;              /* optional [B][N][Tp]: max(min(rates, max_pilot), 0) in float64, i.e. the solve's epilogue also does
-                                  * project_into_continuous_feasible_pilots (postprocessing.py:77-94); NULL = skip */
+                                  * project_into_continuous_feasible_pilots (postprocessing.py:77-94); NULL = skip (quantised pilots:
+                                  * acb_quantize_pilots after the solve) */
     float* rate_est;             /* optional [B]: estimated distance (A) of the schedule to its limit point when the rate polish ran, else -1 */
     int32_t* status;             /* [B] */
     int32_t* iters;              /* [B] */
@@ -238,6 +241,18 @@ int acb_reallocate(acb_site* site, int mode, const double* rates_in, double* rat
                    int S_max, const int32_t* n_sessions, const int32_t* sess_row, const int32_t* sess_start,
                    const double* sess_ramp, const double* sess_max0, const int32_t* order,
                    const double* peak_limit, void* stream);
+
+/* Quantised pilots of a solved batch, in one launch: what AdaptiveSchedulingAlgorithm(quantize=True[, reallocate=True])
+ * does after the solve (adacharge/adacharge.py:177-190), for every instance.  Reads batch->rates (float32 [B][N][Tp]),
+ * batch->T, batch->n_sessions (an instance without sessions gets all-zero pilots) and, for ACB_PILOTS_REALLOCATE, the raw session tables (after acb_preprocess_sessions, if used); writes
+ * pilots [B][N][Tp] float64, bit-identical to the reference applied to rates[:, :T] in float64 and then np.maximum(., 0).
+ * Columns >= T[b] are 0.  The reallocation takes the sessions in slot order (empty slots, station < 0, skipped) and their
+ * ramp as interface.remaining_amp_periods: remaining_demand * 1000 / voltage * (60 / period).  The site needs
+ * allowable_pilots; sessions->B must equal batch->B. */
+#define ACB_PILOTS_DISCRETE 1   /* project_into_discrete_feasible_pilots   postprocessing.py:97-118 */
+#define ACB_PILOTS_REALLOCATE 2 /* diff_based_reallocation                 postprocessing.py:189-258 */
+int acb_quantize_pilots(acb_site* site, int mode, const acb_sessions* sessions, double period, const acb_batch* batch,
+                        double* pilots, void* stream);
 
 /* feasible[b] = 1 iff every SOC line current of column `col` is <= limit + 1e-7. */
 int acb_constraints_feasible(acb_site* site, const double* rates, int B, int T, int col, int32_t* feasible, void* stream);
