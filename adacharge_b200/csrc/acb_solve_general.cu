@@ -70,6 +70,9 @@ __global__ void k_setup(SiteDev S, acb_batch B, acb_options opt, GenWork W, GenD
     const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = blockDim.x >> 5;
     const int nS = B.n_sessions[b], Tb = B.T[b], Tp = D.Tp;
     __shared__ float red[32];
+    // (warm_shift / warm_had: see the on-chip kernel)
+    const int wsh = B.warm_shift;
+    const bool hadW = !B.warm_had || B.warm_had[b] != 0;
     for (int i = tid; i < D.N; i += blockDim.x) { W.row_first[(size_t)b * D.N + i] = 0; W.row_cnt[(size_t)b * D.N + i] = 0; }
     __syncthreads();
     // per-row session runs (sessions are sorted by row)
@@ -82,7 +85,7 @@ __global__ void k_setup(SiteDev S, acb_batch B, acb_options opt, GenWork W, GenD
             W.row_first[(size_t)b * D.N + row] = s;
             W.row_cnt[(size_t)b * D.N + row] = c;
         }
-        W.MU[(size_t)b * B.S_max + s] = B.warm_mu ? B.warm_mu[(size_t)b * B.S_max + s] : 0.f;
+        W.MU[(size_t)b * B.S_max + s] = (B.warm_mu && hadW) ? B.warm_mu[(size_t)b * B.S_max + s] : 0.f;
     }
     // cost scale and scaled cost vectors
     float m = 0.f;
@@ -130,9 +133,8 @@ __global__ void k_setup(SiteDev S, acb_batch B, acb_options opt, GenWork W, GenD
         // (2 Gamma u^2 with u = su * (Khat r)_u): at rho ~ Gamma su^2 the row's prox is balanced; a 1000-EVSE
         // load-flattening instance goes from > 1000 iterations at rho0 to the first check
         const float su0 = D.has_u ? S.row_scale[D.rU] : 0.f;
-        const bool hadW0 = !B.warm_had || B.warm_had[b] != 0;
-        sc[GS_RHO] = (B.warm_scal && hadW0 && B.warm_scal[b * 2] > 0.f) ? B.warm_scal[b * 2] : fmaxf(opt.rho0, opt.rho_curv * B.gamma[b] * cs * su0 * su0);
-        sc[GS_PLEVEL] = B.warm_scal ? fmaxf(hadW0 ? B.warm_scal[b * 2 + 1] : 0.f, B.peak_p0[b]) : B.peak_p0[b];
+        sc[GS_RHO] = (B.warm_scal && hadW && B.warm_scal[b * 2] > 0.f) ? B.warm_scal[b * 2] : fmaxf(opt.rho0, opt.rho_curv * B.gamma[b] * cs * su0 * su0);
+        sc[GS_PLEVEL] = (B.warm_scal && hadW) ? fmaxf(B.warm_scal[b * 2 + 1], B.peak_p0[b]) : B.peak_p0[b];
         sc[GS_CS] = cs;
         sc[GS_QD] = B.qd[b] * cs; sc[GS_GAMMA] = B.gamma[b] * cs; sc[GS_PKW] = B.peak_w[b] * cs; sc[GS_PKP0] = B.peak_p0[b];
         sc[GS_E1] = sc[GS_E2] = sc[GS_XMAX] = sc[GS_YMAX] = sc[GS_VIOL] = sc[GS_UMAX] = sc[GS_ZUMAX] = sc[GS_GAP] = sc[GS_RP] = sc[GS_RD] = 0.f;
@@ -145,9 +147,6 @@ __global__ void k_setup(SiteDev S, acb_batch B, acb_options opt, GenWork W, GenD
         W.iters[b] = 0;
     }
     // state of the coupling rows (the EVSE rows' v: k_rows<Q, 6>)
-    // (warm_shift / warm_had: see the on-chip kernel)
-    const int wsh = B.warm_shift;
-    const bool hadW = !B.warm_had || B.warm_had[b] != 0;
     for (int i = tid; i < D.R * Tp; i += blockDim.x) {
         size_t k = (size_t)b * D.R * Tp + i;
         const int t = i % Tp;
@@ -338,7 +337,7 @@ __global__ void __launch_bounds__(Q > 0 ? 128 : 256, Q > 0 ? 5 : 1) k_rows(SiteD
                 for (int q = 0; q < nq; ++q) {
                     const int t = lane + 32 * q;
                     const float lo = rs.LB(q), hi = rs.UB(q);
-                    W.V[base + 32 * q] = B.warm_v1 ? ((hadW && t + wsh < Tp) ? B.warm_v1[base + 32 * q + wsh] : 0.f) : clampf(0.f, lo, hi);
+                    W.V[base + 32 * q] = (B.warm_v1 && hadW) ? ((t + wsh < Tp) ? B.warm_v1[base + 32 * q + wsh] : 0.f) : clampf(0.f, lo, hi);
                     const float c = AL[t] + kgc * BE[t];
                     dsum += (double)fmaxf(c * lo, c * hi) + (double)qd * (double)fmaxf(lo * lo, hi * hi);
                     add_part(q, hi);
@@ -1038,7 +1037,7 @@ __global__ void k_rescale_vc(SiteDev S, acb_batch B, GenWork W, GenDims D) {
 
 __global__ void k_clear_check(GenWork W, int B_) {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= B_) return;
+    if (b >= B_ || W.status[b] >= 0) return;  // a finished instance keeps its last violation for the stats
     float* sc = W.scal + (size_t)b * GS_N;
     sc[GS_VIOL] = 0.f;  // encoded as viol + 4 by the atomic max
     sc[GS_E1] = sc[GS_E2] = sc[GS_XMAX] = sc[GS_YMAX] = 0.f;
@@ -1054,7 +1053,8 @@ __global__ void k_finish(acb_batch B, GenWork W, GenDims D) {
     float* o = B.stats + (size_t)b * ACB_NSTATS;
     o[0] = sc[GS_RP]; o[1] = sc[GS_RD]; o[2] = sc[GS_GAP]; o[3] = sc[GS_VIOL]; o[4] = sc[GS_RHO]; o[5] = sc[GS_CS]; o[6] = 0.f; o[7] = 0.f;
     if (B.out_scal) { B.out_scal[b * 2] = sc[GS_RHO]; B.out_scal[b * 2 + 1] = sc[GS_PLEVEL]; }
-    if (B.out_mu) for (int s = 0; s < B.S_max; ++s) B.out_mu[(size_t)b * B.S_max + s] = W.MU[(size_t)b * B.S_max + s];
+    if (B.out_mu)  // (empty session slots: 0, as on chip; k_setup leaves their W.MU unset)
+        for (int s = 0; s < B.S_max; ++s) B.out_mu[(size_t)b * B.S_max + s] = s < B.n_sessions[b] ? W.MU[(size_t)b * B.S_max + s] : 0.f;
 }
 
 template <int Q>

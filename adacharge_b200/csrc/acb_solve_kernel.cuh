@@ -223,9 +223,11 @@ __global__ void __launch_bounds__(TPW == 2 ? 1024 : (FAST ? ACB_FAST_THREADS : 7
     // ------------------------------------------------------------------ prologue
     for (int i = tid; i < 2 * N * Tp; i += nthreads) LB[i] = 0.f;  // LB (FAST: v) and UB are contiguous
     // warm start of a closed-loop replay: the previous step's state is read `warm_shift` columns ahead (column t of this
-    // problem was column t + 1 of the previous one), and instances whose site was idle before start cold (warm_had)
+    // problem was column t + 1 of the previous one), and instances whose site was idle before start cold (warm_had = 0:
+    // no warm array is read, the same start as a solve without warm arrays)
     const int wsh = B.warm_shift;
     const bool hadW = !B.warm_had || B.warm_had[b] != 0;
+    const float* warm_v1 = hadW ? B.warm_v1 : nullptr;
     for (int i = tid; i < R * Tp; i += nthreads) {
         const int t = i % Tp;
         VC[i] = (B.warm_vc && hadW && t + wsh < Tp) ? B.warm_vc[(size_t)b * R * Tp + i + wsh] : 0.f;
@@ -246,7 +248,7 @@ __global__ void __launch_bounds__(TPW == 2 ? 1024 : (FAST ? ACB_FAST_THREADS : 7
         SESS_A[i] = ok ? B.sess_start[k] : 0;
         SESS_B[i] = ok ? B.sess_start[k] + B.sess_len[k] : 0;
         SESS_E[i] = ok ? B.sess_energy[k] : 0.f;
-        SESS_MU[i] = (ok && B.warm_mu) ? B.warm_mu[k] : 0.f;
+        SESS_MU[i] = (ok && B.warm_mu && hadW) ? B.warm_mu[k] : 0.f;
         SESS_MU2[i] = 0.f;
         SESS_NF[i] = 0.f;
         SESS_Q[i] = (ok && B.sess_quad) ? B.sess_quad[k] : 0.f;  // (scaled by the cost scale below)
@@ -345,7 +347,7 @@ __global__ void __launch_bounds__(TPW == 2 ? 1024 : (FAST ? ACB_FAST_THREADS : 7
         const float su0 = S.has_u ? S.row_scale[rU] : 0.f;
         SCAL[SC_RHO] = (B.warm_scal && hadW && B.warm_scal[b * 2] > 0.f) ? B.warm_scal[b * 2]
                                                                            : fmaxf(opt.rho0, opt.rho_curv * B.gamma[b] * SCAL[SC_CS] * su0 * su0);
-        SCAL[SC_PLEVEL] = B.warm_scal ? fmaxf(hadW ? B.warm_scal[b * 2 + 1] : 0.f, B.peak_p0[b]) : B.peak_p0[b];
+        SCAL[SC_PLEVEL] = (B.warm_scal && hadW) ? fmaxf(B.warm_scal[b * 2 + 1], B.peak_p0[b]) : B.peak_p0[b];
         SCAL[SC_FLAG] = 0.f;
         SCAL[SC_NSUM] = 0.f;
         SCAL[SC_NREST] = 0.f;
@@ -455,7 +457,7 @@ __global__ void __launch_bounds__(TPW == 2 ? 1024 : (FAST ? ACB_FAST_THREADS : 7
             float v = 0.f;
             if (row >= 0) {
                 if (P.resume) v = P.st_v1[((size_t)b * N + row) * Tp + t];
-                else if (B.warm_v1) v = (hadW && t + wsh < Tp) ? B.warm_v1[((size_t)b * N + row) * Tp + t + wsh] : 0.f;
+                else if (warm_v1) v = (t + wsh < Tp) ? warm_v1[((size_t)b * N + row) * Tp + t + wsh] : 0.f;
                 else v = clampf(0.f, lbv(row, t), ubv(row, t));
                 vset(k, q, row, v);
             }
@@ -1448,7 +1450,7 @@ __global__ void __launch_bounds__(TPW == 2 ? 1024 : (FAST ? ACB_FAST_THREADS : 7
                     // start over cold, keeping the best dual bound.  (A second penalty change on cold-started solves
                     // measured worse than none.)
                     const int nresc = (int)SCAL[SC_NRESCUE];
-                    const bool canRescue = nresc < opt.max_rescues && (nresc == 0 || (nresc == 1 && B.warm_v1 != nullptr));
+                    const bool canRescue = nresc < opt.max_rescues && (nresc == 0 || (nresc == 1 && B.warm_v1 != nullptr && (!B.warm_had || B.warm_had[b] != 0)));
                     if (flag == 0.f && opt.stall_checks > 0 && SCAL[SC_STALL] >= (float)opt.stall_checks && canRescue) {
                         const bool cold = nresc > 0;
                         SCAL[SC_NEWRHO] = cold ? opt.rho0 : fminf(fmaxf(rho * 3.f, 1e-4f), 1e4f);

@@ -158,7 +158,9 @@ typedef struct acb_batch {
     const float* warm_v1; const float* warm_vc; const float* warm_mu; const float* warm_scal;
     int32_t warm_shift;          /* closed-loop replay: warm_v1 / warm_vc are read this many columns ahead (1 = the previous control
                                   * step's state: its column t + 1 is this problem's column t), zero beyond the horizon */
-    const int32_t* warm_had;     /* optional [B]: 0 = this instance starts cold although warm arrays are given (site idle before) */
+    const int32_t* warm_had;     /* optional [B]: 0 = this instance starts cold although warm arrays are given (site idle before): no
+                                  * warm array is read for it and it is solved bit for bit as without warm arrays (also in
+                                  * the choice of stagnation rescues) */
     float* out_v1; float* out_vc; float* out_mu; float* out_scal;
     /* results */
     float* rates;                /* [B][N][Tp] */

@@ -74,13 +74,17 @@ def test_device_fleet_replay_equals_host_fleet_replay(require_gpu):
     """SURVEY.md 8(f) N1: the simulator side of the step on the device (active sessions, energy delivered, previous
     peak, per-EV multipliers, warm start read one column ahead inside the solve) gives the same pilots, bit for bit,
     as the host-side replay, at every step, including idle sites and a second day."""
+    device_vs_host_fleet_replay(list(range(80, 125)) + list(range(288 + 90, 288 + 110)))
+
+
+def device_vs_host_fleet_replay(steps, solver_options=None):
     from adacharge_b200.replay_fast import DeviceFleetReplay, FleetReplay
 
     obj = [ab.ObjectiveComponent(ab.tou_energy_cost), ab.ObjectiveComponent(ab.total_energy, 0.3), ab.ObjectiveComponent(ab.demand_charge, 1 / 30)]
     infra = caltech_acn_infrastructure()
-    kw = dict(n_sites=7, steps_per_day=288, days=2, seed0=40, mean_sessions=12, Tp=160)
+    kw = dict(n_sites=7, steps_per_day=288, days=2, seed0=40, mean_sessions=12, Tp=160, solver_options=solver_options)
     host, dev = FleetReplay(infra, obj, **kw), DeviceFleetReplay(infra, obj, **kw)
-    for t in list(range(80, 125)) + list(range(288 + 90, 288 + 110)):
+    for t in steps:
         a = host.step(t)
         b = dev.step(t, want_first=True)
         np.testing.assert_array_equal(a, b, err_msg=f"first-period pilots at step {t}")
@@ -96,13 +100,17 @@ def test_warm_started_steps_match_a_cold_oracle_solve(require_gpu):
     """Every warm-started closed-loop step is an ordinary MPC instance: its schedule must be as good as a cold float64
     oracle solve of the same step (objective within 1e-4, constraints satisfied).  Small three-phase site, 15-minute
     periods, so that the oracle takes a fraction of a second per step."""
+    warm_steps_vs_cold_oracle()
+
+
+def warm_steps_vs_cold_oracle(solver_options=None):
     from adacharge_b200.generators import three_phase_balanced_network
     from oracle import mpc
 
     spec = [("tou_energy_cost", 1, {}), ("total_energy", 0.3, {}), ("demand_charge", 1 / 30, {})]
     obj = [ab.ObjectiveComponent(getattr(ab, n), c, k) for n, c, k in spec]
     infra = three_phase_balanced_network(3, 30)
-    rp = SiteReplay(infra, obj, n_sites=3, steps=96, period=15, seed0=5, warm_start=True, mean_sessions=7)
+    rp = SiteReplay(infra, obj, n_sites=3, steps=96, period=15, seed0=5, warm_start=True, mean_sessions=7, solver_options=solver_options)
     rp.keep_problems = True
     rp.run(28, 52)
     warm = [p for p in rp.problems if p[0] > 28]
