@@ -51,10 +51,13 @@ __device__ __forceinline__ float warp_max(float v) {
 }
 __device__ __forceinline__ float clampf(float v, float lo, float hi) { return fminf(fmaxf(v, lo), hi); }
 
-// projection of (a, b) onto the disc of radius lim
-__device__ __forceinline__ void proj_disc(float a, float b, float lim, float& za, float& zb) {
+// projection of (a, b) onto the disc of radius lim: (a, b) * disc_scale(a, b, lim)
+__device__ __forceinline__ float disc_scale(float a, float b, float lim) {
     float n2 = a * a + b * b;
-    float f = (n2 > lim * lim) ? lim * rsqrtf(n2) : 1.0f;
+    return (n2 > lim * lim) ? lim * rsqrtf(n2) : 1.0f;
+}
+__device__ __forceinline__ void proj_disc(float a, float b, float lim, float& za, float& zb) {
+    const float f = disc_scale(a, b, lim);
     za = a * f;
     zb = b * f;
 }
@@ -164,6 +167,10 @@ __global__ void __launch_bounds__(TPW == 2 ? 1024 : (FAST ? ACB_FAST_THREADS : 7
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int nthreads = blockDim.x, nwarps = nthreads >> 5;
     constexpr int Tp = 32 * Q;  // the host pads every batch to an instantiated horizon
+    // paired fp32 ops (FFMA2 / FADD2 / FMUL2: each half rounds as the scalar op) in the column pass and the hot row pass.
+    // Only where v lives in shared memory with three rows per warp: there the aligned register pairs fit; in the other
+    // variants they raise the spills (v in registers, or 64 registers per thread)
+    constexpr bool PAIR = FAST && TPW == 3;
     const int N = S.N, R = S.R, NG = S.NG, NP = S.NP;
     float* LB = sm + L.LB; float* UB = sm + L.UB; float* PART = sm + L.PART; float* VC = sm + L.VC;
     float* VOUT = sm + L.VOUT; float* GIN = sm + L.GIN; float* HG = sm + L.HG; float* THC = sm + L.THC; float* THA = sm + L.THA; float* ALPHA = sm + L.ALPHA; float* BETA = sm + L.BETA;
@@ -834,15 +841,20 @@ __global__ void __launch_bounds__(TPW == 2 ? 1024 : (FAST ? ACB_FAST_THREADS : 7
         for (int wk = tid; wk < nParts * Tp; wk += nthreads) {
             const int part = wk / Tp, t = wk - part * Tp;
             const int obase = part * ACB_OHT;
-            float out[ACB_OHT];
+            float2 out[ACB_OHT / 2];  // outputs (2i, 2i + 1)
 #pragma unroll
-            for (int k = 0; k < ACB_OHT; ++k) out[k] = 0.f;
+            for (int k = 0; k < ACB_OHT / 2; ++k) out[k] = make_float2(0.f, 0.f);
             auto accum = [&](int c, float in) {
                 const float4* mrow = reinterpret_cast<const float4*>(MFT + c * OP + obase);
 #pragma unroll
                 for (int h = 0; h < ACB_OHT / 4; ++h) {
                     const float4 m = mrow[h];
-                    out[4 * h + 0] += m.x * in; out[4 * h + 1] += m.y * in; out[4 * h + 2] += m.z * in; out[4 * h + 3] += m.w * in;
+                    if constexpr (PAIR) {
+                        out[2 * h] = __ffma2_rn(make_float2(m.x, m.y), make_float2(in, in), out[2 * h]);
+                        out[2 * h + 1] = __ffma2_rn(make_float2(m.z, m.w), make_float2(in, in), out[2 * h + 1]);
+                    } else {
+                        out[2 * h].x += m.x * in; out[2 * h].y += m.y * in; out[2 * h + 1].x += m.z * in; out[2 * h + 1].y += m.w * in;
+                    }
                 }
             };
             for (int g = 0; g < NG; ++g) {
@@ -860,7 +872,7 @@ __global__ void __launch_bounds__(TPW == 2 ? 1024 : (FAST ? ACB_FAST_THREADS : 7
             float* ob = HG + obase * Tp + t;  // (HG, VOUT) output block
 #pragma unroll
             for (int k = 0; k < ACB_OHT; ++k)
-                if (obase + k < NIN) ob[k * Tp] = out[k];
+                if (obase + k < NIN) ob[k * Tp] = (k & 1) ? out[k / 2].y : out[k / 2].x;
         }
         ACB_TR(1);
         __syncthreads();
@@ -984,12 +996,24 @@ __global__ void __launch_bounds__(TPW == 2 ? 1024 : (FAST ? ACB_FAST_THREADS : 7
                 const float* ubp = UB + row * Tp + lane;
                 float e = 0.f;
 #pragma unroll
-                for (int q = 0; q < Q; ++q) {
-                    const float ub = ubp[32 * q], vo = vget(k, q, row);
-                    const float z = ub * __saturatef((vo - mu0) * ih[k]);
-                    const float vn = fmaf(c3, hgp[32 * q], fmaf(c2, z, c1 * vo));
-                    vset(k, q, row, vn);
-                    e = fmaf(ub, __saturatef((vn - mu[k]) * ih[k]), e);
+                for (int q = 0; q < Q; q += PAIR ? 2 : 1) {
+                    if (PAIR && q + 1 < Q) {  // elements (q, q + 1) in paired ops; the saturating multiplies and the sum e stay scalar
+                        const float2 ub = make_float2(ubp[32 * q], ubp[32 * q + 32]), vo = make_float2(vget(k, q, row), vget(k, q + 1, row));
+                        const float2 d = __fadd2_rn(vo, make_float2(-mu0, -mu0));
+                        const float2 z = __fmul2_rn(ub, make_float2(__saturatef(d.x * ih[k]), __saturatef(d.y * ih[k])));
+                        const float2 vn = __ffma2_rn(make_float2(c3, c3), make_float2(hgp[32 * q], hgp[32 * q + 32]),
+                                                     __ffma2_rn(make_float2(c2, c2), z, __fmul2_rn(make_float2(c1, c1), vo)));
+                        vset(k, q, row, vn.x); vset(k, q + 1, row, vn.y);
+                        const float2 d1 = __fadd2_rn(vn, make_float2(-mu[k], -mu[k]));
+                        e = fmaf(ub.x, __saturatef(d1.x * ih[k]), e);
+                        e = fmaf(ub.y, __saturatef(d1.y * ih[k]), e);
+                    } else {
+                        const float ub = ubp[32 * q], vo = vget(k, q, row);
+                        const float z = ub * __saturatef((vo - mu0) * ih[k]);
+                        const float vn = fmaf(c3, hgp[32 * q], fmaf(c2, z, c1 * vo));
+                        vset(k, q, row, vn);
+                        e = fmaf(ub, __saturatef((vn - mu[k]) * ih[k]), e);
+                    }
                 }
                 E[k] = e;
             }
@@ -1026,7 +1050,7 @@ __global__ void __launch_bounds__(TPW == 2 ? 1024 : (FAST ? ACB_FAST_THREADS : 7
             // z and the partial sums of 2z - v with the stepped multipliers (verifying them on the way); the pass is
             // repeated once, without verification, if some row had to run the exact search
             for (int round = 0; round < 2; ++round) {
-                float acc[Q];
+                float2 acc[(Q + 1) / 2];  // elements (q, q + 1) of the partial row in acc[q / 2] (odd Q: the last .y is unused)
 #pragma unroll
                 for (int k = 0; k < TPW; ++k) {
                     const int row = rowk[k];
@@ -1036,19 +1060,31 @@ __global__ void __launch_bounds__(TPW == 2 ? 1024 : (FAST ? ACB_FAST_THREADS : 7
                     const float* ubp = UB + row * Tp + lane;
                     float e = 0.f;
 #pragma unroll
-                    for (int q = 0; q < Q; ++q) {
-                        const float vn = vget(k, q, row);
-                        const float zn = ubp[32 * q] * __saturatef((vn - mun[k]) * ih[k]);
-                        const float val = fmaf(2.f, zn, -vn);
-                        acc[q] = first ? val : acc[q] + val;
-                        e += zn;
+                    for (int q = 0; q < Q; q += PAIR ? 2 : 1) {
+                        if (PAIR && q + 1 < Q) {
+                            const float2 vn = make_float2(vget(k, q, row), vget(k, q + 1, row));
+                            const float2 d = __fadd2_rn(vn, make_float2(-mun[k], -mun[k]));
+                            const float2 zn = __fmul2_rn(make_float2(ubp[32 * q], ubp[32 * q + 32]),
+                                                         make_float2(__saturatef(d.x * ih[k]), __saturatef(d.y * ih[k])));
+                            const float2 val = __ffma2_rn(make_float2(2.f, 2.f), zn, make_float2(-vn.x, -vn.y));
+                            acc[q / 2] = first ? val : __fadd2_rn(acc[q / 2], val);
+                            e += zn.x;
+                            e += zn.y;
+                        } else {
+                            const float vn = vget(k, q, row);
+                            const float zn = ubp[32 * q] * __saturatef((vn - mun[k]) * ih[k]);
+                            const float val = fmaf(2.f, zn, -vn);
+                            float& a = (q & 1) ? acc[q / 2].y : acc[q / 2].x;
+                            a = first ? val : a + val;
+                            e += zn;
+                        }
                     }
                     E1[k] = e;
                     const bool last = (k == TPW - 1) || rowk[k + 1 < TPW ? k + 1 : k] < 0 || SLOT[(warp * TPW + k + 1) * 6 + 3] != 0;
                     if (last) {
                         float* pp = PART + sl[2] * Tp + lane;
 #pragma unroll
-                        for (int q = 0; q < Q; ++q) pp[32 * q] = acc[q];
+                        for (int q = 0; q < Q; ++q) pp[32 * q] = (q & 1) ? acc[q / 2].y : acc[q / 2].x;
                     }
                 }
                 if (round == 1 || (verify | exact) == 0) break;
@@ -1108,19 +1144,23 @@ __global__ void __launch_bounds__(TPW == 2 ? 1024 : (FAST ? ACB_FAST_THREADS : 7
                 if (c < nDisc) {
                     const int r = 2 * c;
                     const float lim = LIM[r];
-                    float a = VC[r * Tp + t], bb = VC[(r + 1) * Tp + t], za, zb;
-                    proj_disc(a, bb, lim, za, zb);
-                    float ka = VOUT[r * Tp + t], kb = VOUT[(r + 1) * Tp + t];
-                    float an = a + alpha * (ka - za), bn = bb + alpha * (kb - zb);
+                    // the (a, b) components in paired ops; v + alpha (k - f v) keeps k - f v as one FMA (f v is not rounded)
+                    const float2 v = make_float2(VC[r * Tp + t], VC[(r + 1) * Tp + t]);
+                    const float f = disc_scale(v.x, v.y, lim);
+                    const float2 kv = make_float2(VOUT[r * Tp + t], VOUT[(r + 1) * Tp + t]);
+                    const float2 vn = __ffma2_rn(__ffma2_rn(v, make_float2(-f, -f), kv), make_float2(alpha, alpha), v);
+                    const float an = vn.x, bn = vn.y;
                     VC[r * Tp + t] = an; VC[(r + 1) * Tp + t] = bn;
-                    float zan, zbn;
-                    proj_disc(an, bn, lim, zan, zbn);
-                    GIN[r * Tp + t] = rho * (2.f * zan - an); GIN[(r + 1) * Tp + t] = rho * (2.f * zbn - bn);
+                    const float fn = disc_scale(an, bn, lim);
+                    const float2 zn = __fmul2_rn(vn, make_float2(fn, fn));
+                    const float2 gin = __fmul2_rn(make_float2(rho, rho), __fadd2_rn(__fadd2_rn(zn, zn), make_float2(-an, -bn)));  // rho (2 z - v)
+                    GIN[r * Tp + t] = gin.x; GIN[(r + 1) * Tp + t] = gin.y;
                     if (doAvg) {
                         float* vs = VSUM + (size_t)(N + r) * Tp + t;
                         atomicAdd(vs, an); atomicAdd(vs + Tp, bn);
                     }
                     if (CHK) {
+                        const float zan = zn.x, zbn = zn.y;
                         float ya = rho * (an - zan), yb = rho * (bn - zbn);
                         VOUT[r * Tp + t] = ya; VOUT[(r + 1) * Tp + t] = yb;
                         dD -= (double)(lim * sqrtf(ya * ya + yb * yb));  // support function of the disc
