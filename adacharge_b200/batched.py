@@ -25,6 +25,7 @@ import torch
 
 from . import _cabi, engine
 from . import adaptive_charging_optimization as aco
+from .interface import infrastructure_from_dict
 
 _KIND_OF = {
     aco.quick_charge: "quick_charge", aco.equal_share: "equal_share", aco.tou_energy_cost: "tou_energy_cost",
@@ -81,12 +82,13 @@ class BatchResult:
     stats: np.ndarray    # [B, ACB_NSTATS]
 
 
-class _Chunk:
-    """Pinned staging, device buffers and the three C structs of one slice of the batch."""
+class _Chunk(engine.DeviceBatch):
+    """One slice of the batch: pinned staging and device copies of the raw arrays, the device packer's two C structs
+    (acb_sessions, acb_objective) and, as a DeviceBatch, the packed inputs that packer writes and the results."""
 
     def __init__(self, owner: "BatchedAdaptiveCharging", lo: int, hi: int):
         self.lo, self.hi = lo, hi
-        B, S, Tp, N, R = hi - lo, owner.S_max, owner.Tp, owner.site.N, owner.site.R
+        B, S, Tp = hi - lo, owner.S_max, owner.Tp
         dev = owner.device
         self.stream = torch.cuda.Stream(device=dev)
         raw = {n: ((B, S), dt) for n, dt in SESSION_FIELDS}
@@ -115,22 +117,12 @@ class _Chunk:
             d["peak_limit"] = mk((B, Tp), f32)
         if owner.need_sess_quad:
             d["sess_quad"] = mk((B, S), f32)
-        self.packed = d
-        self.rates = mk((B, N, Tp), f32)
-        self.pilots = mk((B, N, Tp), torch.float64)  # continuous: the solve's epilogue; quantised: acb_quantize_pilots
-        self.status, self.iters = mk((B,), i32), mk((B,), i32)
-        self.stats = mk((B, _cabi.ACB_NSTATS), f32)
-        self.work = mk((B, N + max(R, 1), Tp), f32)
+        # pilots: continuous from the solve's epilogue; quantised from acb_quantize_pilots, without that projection first
+        super().__init__(owner.site, d, Tp, S, multi_session=owner.multi_session, pilots=True)
+        self.bind_pilots(not owner.pilot_mode)
         self.flags = torch.zeros((1,), dtype=i32, device=dev)
         self.flags_host = torch.zeros((1,), dtype=i32).pin_memory()
         p = engine._ptr
-        b = _cabi.Batch()
-        b.B, b.Tp, b.S_max, b.multi_session = B, Tp, S, int(owner.multi_session)
-        for k, t in d.items():
-            setattr(b, k, p(t))
-        b.work, b.rates, b.status, b.iters, b.stats = p(self.work), p(self.rates), p(self.status), p(self.iters), p(self.stats)
-        b.pilots = None if owner.pilot_mode else p(self.pilots)  # quantised pilots are not first projected continuously
-        self.batch = b
         s = _cabi.Sessions()
         s.B, s.S_max = B, S
         for n, _ in SESSION_FIELDS:
@@ -147,6 +139,11 @@ class _Chunk:
         o.external_signal, o.ext_stride = p(self.dev_raw.get("external_signal")), Tp
         o.peak_limit, o.pl_stride = p(self.dev_raw.get("peak_limit")), Tp
         self.objective = o
+
+    @property
+    def batch(self) -> _cabi.Batch:
+        """The chunk's acb_batch (DeviceBatch.struct), as the entry points after the packer take it."""
+        return self.struct
 
 
 class BatchedAdaptiveCharging:
@@ -171,13 +168,8 @@ class BatchedAdaptiveCharging:
                  constraint_type="SOC", enforce_energy_equality=False, peak_limit=False, multi_session=False, demand_charge=0.0,
                  per_instance_demand_charge=False, solver_options: Optional[dict] = None, device=None, chunks: int = 4,
                  enforce_pilot_limit=True, estimate_max_rate=False, quantize=False, reallocate=False):
-        from .interface import InfrastructureInfo
-
         if isinstance(infrastructure, dict):
-            i = infrastructure
-            infrastructure = InfrastructureInfo(np.asarray(i["constraint_matrix"]), np.asarray(i["constraint_limits"]), np.asarray(i["phases"]),
-                                                np.asarray(i["voltages"]), i["constraint_ids"], i["station_ids"], np.asarray(i["max_pilot"]),
-                                                np.asarray(i["min_pilot"]), i.get("allowable_pilots"), i.get("is_continuous"))
+            infrastructure = infrastructure_from_dict(infrastructure)
         self.pilot_mode = pilot_mode(quantize, reallocate, infrastructure)
         self.components = objective_components(objective)
         kinds = {k for k, _, _ in self.components}
@@ -222,7 +214,7 @@ class BatchedAdaptiveCharging:
     def _stage(self, ch: _Chunk, arrays: Dict[str, np.ndarray]):
         """host arrays -> the chunk's pinned staging (a plain memcpy per field)."""
         # every minimum rate 0 (the usual case) is declared to the library: fastest on-chip variant
-        ch.batch.lb_zero = int(not np.any(np.asarray(arrays["min_rate"])[ch.lo:ch.hi] != 0))
+        ch.lb_zero = not np.any(np.asarray(arrays["min_rate"])[ch.lo:ch.hi] != 0)
         for k, dst in ch.host.items():
             src = arrays.get(k)
             if src is None:
@@ -255,16 +247,16 @@ class BatchedAdaptiveCharging:
             if self.enforce_pilot_limit or self.estimate_max_rate:
                 _cabi.check(L.acb_preprocess_sessions(self.site.handle, C.byref(ch.sessions), int(self.enforce_pilot_limit),
                                                       engine._ptr(ch.dev_raw.get("upper_bound")), st), "acb_preprocess_sessions")
-            _cabi.check(L.acb_pack_sessions(self.site.handle, C.byref(ch.sessions), C.byref(ch.objective), C.byref(ch.batch), engine._ptr(ch.flags), st), "acb_pack_sessions")
+            _cabi.check(L.acb_pack_sessions(self.site.handle, C.byref(ch.sessions), C.byref(ch.objective), C.byref(ch.struct), engine._ptr(ch.flags), st), "acb_pack_sessions")
             if events is not None:
                 ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
                 ev[0].record(ch.stream)
-            _cabi.check(L.acb_solve_batch(self.site.handle, C.byref(ch.batch), C.byref(self.options), st), "acb_solve_batch")
+            ch.solve(self.options, st)
             if events is not None:
                 ev[1].record(ch.stream)
                 events.append(ev)
             if self.pilot_mode:
-                _cabi.check(L.acb_quantize_pilots(self.site.handle, self.pilot_mode, C.byref(ch.sessions), float(self.period), C.byref(ch.batch),
+                _cabi.check(L.acb_quantize_pilots(self.site.handle, self.pilot_mode, C.byref(ch.sessions), float(self.period), C.byref(ch.struct),
                                                   engine._ptr(ch.pilots), st), "acb_quantize_pilots")
             if not from_device_raw:
                 self.host_pilots[ch.lo:ch.hi].copy_(ch.pilots, non_blocking=True)

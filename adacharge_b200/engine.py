@@ -246,23 +246,120 @@ def padded_horizon(T: int) -> int:
     return Tp
 
 
-class PackedBatch:
-    """Pinned host staging + device tensors of a batch; owns the acb_batch struct."""
+class DeviceBatch:
+    """Device side of one acb_batch (include/adacharge_b200.h): the packed inputs, the result and scratch tensors, and
+    the struct that points at them.  The struct is filled once, here; afterwards only the warm-start and pilots
+    pointers and the two declared flags change (set_warm, or warm / warm_out alone; bind_pilots; lb_zero,
+    multi_session), so a batch that is solved every step is not rebuilt.  Entry points that take an acb_batch get
+    ``C.byref(self.struct)``.
+
+    `packed` holds the input tensors by acb_batch field name (`T`, `n_sessions`, `sess_*`, `min_rates`, `max_rates`,
+    `alpha`, `beta`, `qd`, `gamma`, `peak_w`, `peak_p0`; `ext`, `peak_limit`, `sess_quad` optional).  `pilots`
+    allocates the float64 [B, N, Tp] pilots the solve's epilogue writes; `rate_est` the rate polish's estimate."""
+
+    def __init__(self, site: Site, packed: Dict[str, torch.Tensor], Tp: int, S_max: int, multi_session=False, lb_zero=False,
+                 pilots=False, rate_est=False):
+        B, N, R = int(packed["T"].shape[0]), site.N, site.R
+        dev = torch.device("cuda", site.device)
+        self.site, self.device, self.B, self.Tp, self.S_max, self.packed = site, dev, B, Tp, S_max, packed
+        self.rates = torch.empty((B, N, Tp), dtype=torch.float32, device=dev)
+        self.status = torch.empty((B,), dtype=torch.int32, device=dev)
+        self.iters = torch.empty((B,), dtype=torch.int32, device=dev)
+        self.stats = torch.empty((B, _cabi.ACB_NSTATS), dtype=torch.float32, device=dev)
+        self.work = torch.empty((B, N + max(R, 1), Tp), dtype=torch.float32, device=dev)
+        self.pilots = torch.empty((B, N, Tp), dtype=torch.float64, device=dev) if pilots else None
+        self.rate_est = torch.full((B,), -1.0, dtype=torch.float32, device=dev) if rate_est else None
+        s = self.struct = Batch()
+        s.B, s.Tp, s.S_max = B, Tp, S_max
+        for name, t in packed.items():
+            setattr(s, name, _ptr(t))
+        s.work, s.rates, s.status, s.iters, s.stats = _ptr(self.work), _ptr(self.rates), _ptr(self.status), _ptr(self.iters), _ptr(self.stats)
+        s.pilots, s.rate_est = _ptr(self.pilots), _ptr(self.rate_est)
+        self.multi_session, self.lb_zero = multi_session, lb_zero
+        self.set_warm()
+
+    @property
+    def multi_session(self) -> bool:
+        """Declared to the library: an EVSE may hold more than one session."""
+        return bool(self.struct.multi_session)
+
+    @multi_session.setter
+    def multi_session(self, v):
+        self.struct.multi_session = int(bool(v))
+
+    @property
+    def lb_zero(self) -> bool:
+        """Declared to the library: every minimum rate of the batch is 0 (the usual case; its fastest on-chip variant)."""
+        return bool(self.struct.lb_zero)
+
+    @lb_zero.setter
+    def lb_zero(self, v):
+        self.struct.lb_zero = int(bool(v))
+
+    def new_warm_state(self) -> Dict[str, torch.Tensor]:
+        """One zeroed set of warm-start tensors of this batch's shape: v1 [B, N, Tp], vc [B, max(R, 1), Tp], mu [B, S_max],
+        scal [B, 2] (rho, peak level)."""
+        B, Tp = self.B, self.Tp
+        mk = lambda *shape: torch.zeros(shape, dtype=torch.float32, device=self.device)  # noqa: E731
+        return dict(v1=mk(B, self.site.N, Tp), vc=mk(B, max(self.site.R, 1), Tp), mu=mk(B, self.S_max), scal=mk(B, 2))
+
+    def set_warm(self, warm: Optional[Dict[str, torch.Tensor]] = None, out: Optional[Dict[str, torch.Tensor]] = None, shift: int = 0,
+                 had: Optional[torch.Tensor] = None):
+        """Where the following solves start from and where they leave their final state (see `warm`, `warm_out`).
+        `warm` is read `shift` columns ahead (1: the previous control step's state), and an instance whose `had` [B]
+        int32 entry is 0 starts cold (its site was idle before)."""
+        self.warm, self.warm_out = warm, out
+        self.struct.warm_shift, self.struct.warm_had = shift, _ptr(had)
+        self._had = had  # the struct holds a raw pointer: keep the tensor alive
+
+    @property
+    def warm(self) -> Optional[Dict[str, torch.Tensor]]:
+        """Warm-start inputs of the following solves: a new_warm_state() set (None: a cold start)."""
+        return self._warm
+
+    @warm.setter
+    def warm(self, w: Optional[Dict[str, torch.Tensor]]):
+        s, d = self.struct, w or {}
+        s.warm_v1, s.warm_vc, s.warm_mu, s.warm_scal = _ptr(d.get("v1")), _ptr(d.get("vc")), _ptr(d.get("mu")), _ptr(d.get("scal"))
+        self._warm = w
+
+    @property
+    def warm_out(self) -> Optional[Dict[str, torch.Tensor]]:
+        """Where the following solves write their final state: a new_warm_state() set (None: not written)."""
+        return self._warm_out
+
+    @warm_out.setter
+    def warm_out(self, o: Optional[Dict[str, torch.Tensor]]):
+        s, d = self.struct, o or {}
+        s.out_v1, s.out_vc, s.out_mu, s.out_scal = _ptr(d.get("v1")), _ptr(d.get("vc")), _ptr(d.get("mu")), _ptr(d.get("scal"))
+        self._warm_out = o
+
+    def bind_pilots(self, on: bool):
+        """Point acb_batch.pilots at `self.pilots` (on) or at nothing: the solve's epilogue writes the continuous pilots
+        there, and acb_fleet_apply reads the pilots from there."""
+        self.struct.pilots = _ptr(self.pilots) if on else None
+
+    def solve(self, options: Options, stream=None):
+        """Enqueue acb_solve_batch on `stream` (a cudaStream_t; default: the current stream)."""
+        st = _stream_ptr(self.site.device) if stream is None else stream
+        _cabi.check(_cabi.lib().acb_solve_batch(self.site.handle, C.byref(self.struct), C.byref(options), st), "acb_solve_batch")
+        return self
+
+
+class PackedBatch(DeviceBatch):
+    """A batch packed on the host: pinned staging of the acb_batch inputs (`host`), copied into the device inputs by
+    upload()."""
 
     def __init__(self, site: Site, instances: Sequence[Instance], Tp: Optional[int] = None, S_max: Optional[int] = None,
                  want_warm_out=False):
-        self.site = site
         B = len(instances)
         Tmax = max(i.T for i in instances)
         if Tp is None:
             Tp = padded_horizon(Tmax)
-        self.Tp = Tp
-        self.S_max = S_max or max(4, max(len(i.sess_row) for i in instances))
-        self.B = B
-        Tp_, S_ = self.Tp, self.S_max
+        Tp_, S_ = Tp, S_max or max(4, max(len(i.sess_row) for i in instances))
         f32, i32 = np.float32, np.int32
         h = {}
-        self.multi_session = any(len(set(i.sess_row.tolist())) < len(i.sess_row) for i in instances)
+        multi_session = any(len(set(i.sess_row.tolist())) < len(i.sess_row) for i in instances)
         h["T"] = np.array([i.T for i in instances], dtype=i32)
         h["n_sessions"] = np.array([len(i.sess_row) for i in instances], dtype=i32)
         for name in ("sess_row", "sess_start", "sess_len"):
@@ -315,7 +412,7 @@ class PackedBatch:
                     raise ValueError("site was built with a peak-limit row but an instance has no peak_limit")
                 a[b, : inst.T] = np.broadcast_to(np.asarray(inst.peak_limit, dtype=np.float64), (inst.T,))
             h["peak_limit"] = a
-        self._allocate(h, want_warm_out)
+        self._stage(site, h, Tp_, S_, multi_session, want_warm_out)
 
     @classmethod
     def from_arrays(cls, site: Site, host: Dict[str, np.ndarray], Tp: int, S_max: int, multi_session=False, want_warm_out=False):
@@ -325,44 +422,24 @@ class PackedBatch:
         that keep their sessions in arrays (replay_fast) instead of SessionInfo objects."""
         if Tp % 32 != 0 or Tp <= 0 or Tp > MAX_HORIZON:
             raise ValueError(f"Tp must be a positive multiple of 32, at most {MAX_HORIZON}")
-        self = cls.__new__(cls)
-        self.site, self.Tp, self.S_max, self.B = site, Tp, S_max, int(host["T"].shape[0])
-        self.multi_session = bool(multi_session)
         if site.use_peak_row and "peak_limit" not in host:
             raise ValueError("site was built with a peak-limit row but the batch has no peak_limit")
-        self._allocate(host, want_warm_out)
+        self = cls.__new__(cls)
+        self._stage(site, host, Tp, S_max, multi_session, want_warm_out)
         return self
 
-    def _allocate(self, h: Dict[str, np.ndarray], want_warm_out: bool):
-        site, B, Tp_, S_ = self.site, self.B, self.Tp, self.S_max
+    def _stage(self, site: Site, h: Dict[str, np.ndarray], Tp: int, S_max: int, multi_session: bool, want_warm_out: bool):
         self.host = {k: torch.from_numpy(np.ascontiguousarray(v)).pin_memory() for k, v in h.items()}
         self.h2d_bytes = sum(t.numel() * t.element_size() for t in self.host.values())
         dev = torch.device("cuda", site.device)
-        self.dev: Dict[str, torch.Tensor] = {}
-        self.device = dev
-        N, R = site.N, site.R
-        self.rates = torch.empty((B, N, Tp_), dtype=torch.float32, device=dev)
-        self.status = torch.empty((B,), dtype=torch.int32, device=dev)
-        self.iters = torch.empty((B,), dtype=torch.int32, device=dev)
-        self.stats = torch.empty((B, _cabi.ACB_NSTATS), dtype=torch.float32, device=dev)
-        self.work = torch.empty((B, N + max(R, 1), Tp_), dtype=torch.float32, device=dev)
-        self.pilots = None    # set by want_pilots(): float64 continuous-feasible pilots written by the solve's epilogue
-        self.rate_est = None
+        packed = {k: torch.empty_like(t, device=dev) for k, t in self.host.items()}
         # the rate polish needs a strictly convex objective: without a quadratic term the library is told not to
         # allocate its previous-schedule scratch
         self.any_quadratic = bool(np.any(np.asarray(h["qd"]) > 0))
-        # every minimum rate 0 (the usual case): declared to the library, which then runs its fastest on-chip variant
-        self.lb_zero = not bool(np.any(np.asarray(h["min_rates"]) != 0))
-        self.warm = None
-        self.warm_out = None
+        super().__init__(site, packed, Tp, S_max, multi_session=multi_session, lb_zero=_all_zero(h["min_rates"]), rate_est=self.any_quadratic)
         if want_warm_out:
-            self.warm_out = dict(
-                v1=torch.empty((B, N, Tp_), dtype=torch.float32, device=dev),
-                vc=torch.empty((B, max(R, 1), Tp_), dtype=torch.float32, device=dev),
-                mu=torch.empty((B, S_), dtype=torch.float32, device=dev),
-                scal=torch.empty((B, 2), dtype=torch.float32, device=dev),
-            )
-        self.struct = Batch()
+            self.warm_out = self.new_warm_state()
+        self._uploaded = False
 
     def refill(self, h: Dict[str, np.ndarray]):
         """Overwrite the pinned staging buffers in place with a new batch of the same shape (same field names, shapes
@@ -376,104 +453,39 @@ class PackedBatch:
                 raise ValueError(f"refill: field {k} changed shape or dtype ({dst.shape} {dst.dtype} -> {v.shape} {v.dtype})")
             dst[...] = v
         self.any_quadratic = bool(np.any(np.asarray(h["qd"]) > 0))
-        self.lb_zero = not bool(np.any(np.asarray(h["min_rates"]) != 0))
+        self.lb_zero = _all_zero(h["min_rates"])
         return self
 
     def upload(self):
         for k, t in self.host.items():
-            d = self.dev.get(k)
-            if d is None:
-                self.dev[k] = t.to(self.device, non_blocking=True)
-            else:
-                d.copy_(t, non_blocking=True)
-        return self
-
-    def _fill_struct(self):
-        s = self.struct
-        s.B, s.Tp, s.S_max = self.B, self.Tp, self.S_max
-        s.multi_session = int(self.multi_session)
-        s.lb_zero = int(self.lb_zero)
-        for name in ("T", "n_sessions", "sess_row", "sess_start", "sess_len", "sess_energy", "sess_rate_off",
-                     "min_rates", "max_rates", "alpha", "beta", "qd", "gamma", "ext", "peak_w", "peak_p0", "peak_limit", "sess_quad"):
-            setattr(s, name, _ptr(self.dev.get(name)))
-        w = self.warm or {}
-        s.warm_v1, s.warm_vc, s.warm_mu, s.warm_scal = (_ptr(w.get(k)) for k in ("v1", "vc", "mu", "scal"))
-        o = self.warm_out or {}
-        s.out_v1, s.out_vc, s.out_mu, s.out_scal = (_ptr(o.get(k)) for k in ("v1", "vc", "mu", "scal"))
-        s.work = _ptr(self.work)
-        s.rates, s.status, s.iters, s.stats = _ptr(self.rates), _ptr(self.status), _ptr(self.iters), _ptr(self.stats)
-        s.pilots, s.rate_est = _ptr(self.pilots), _ptr(self.rate_est)
-        return s
-
-    def want_pilots(self):
-        """Have the solve also write max(min(rates, max_pilot), 0) in float64 (project_into_continuous_feasible_pilots
-        fused into the solve's epilogue) into `self.pilots` [B, N, Tp]."""
-        if self.pilots is None:
-            self.pilots = torch.empty((self.B, self.site.N, self.Tp), dtype=torch.float64, device=self.device)
+            self.packed[k].copy_(t, non_blocking=True)
+        self._uploaded = True
         return self
 
     def solve(self, options: Optional[Options] = None):
         """Enqueue the batched solve on the current stream (asynchronous)."""
-        if not self.dev:
+        if not self._uploaded:
             self.upload()
         opt = options or _cabi.default_options()
         if not self.any_quadratic and opt.rate_tol > 0:
             opt = _cabi.copy_options(opt, rate_tol=0.0)
-        elif self.any_quadratic and opt.rate_tol > 0 and self.rate_est is None:
-            self.rate_est = torch.full((self.B,), -1.0, dtype=torch.float32, device=self.device)
-        _cabi.check(
-            _cabi.lib().acb_solve_batch(self.site.handle, C.byref(self._fill_struct()), C.byref(opt), _stream_ptr(self.site.device)),
-            "acb_solve_batch",
-        )
-        return self
+        return super().solve(opt)
 
     def bounds(self):
         """charging_rate_bounds on device -> (lb, ub) tensors [B, N, Tp]."""
-        if not self.dev:
+        if not self._uploaded:
             self.upload()
         lb = torch.empty_like(self.rates)
         ub = torch.empty_like(self.rates)
         _cabi.check(
-            _cabi.lib().acb_charging_rate_bounds(self.site.handle, C.byref(self._fill_struct()), _ptr(lb), _ptr(ub), _stream_ptr(self.site.device)),
+            _cabi.lib().acb_charging_rate_bounds(self.site.handle, C.byref(self.struct), _ptr(lb), _ptr(ub), _stream_ptr(self.site.device)),
             "acb_charging_rate_bounds",
         )
         return lb, ub
 
 
-class HostPipeline:
-    """Host-to-host solve of a large batch: the instances are split into chunks, each with its own stream, so the
-    host->device copy of one chunk and the device->host copy of another overlap the solve of a third.  `run()`
-    enqueues one full pass and makes the current stream wait for it; results land in the pinned `host_rates`
-    ([B, N, Tp] float32), `host_status`, `host_iters` (valid after a synchronize of the current stream)."""
-
-    def __init__(self, site: Site, instances: Sequence[Instance], chunks: int = 4, Tp: Optional[int] = None):
-        B = len(instances)
-        chunks = max(1, min(chunks, B))
-        if Tp is None:
-            Tp = padded_horizon(max(i.T for i in instances))
-        S_max = max(4, max(len(i.sess_row) for i in instances))
-        bounds = [round(k * B / chunks) for k in range(chunks + 1)]
-        self.parts = [PackedBatch(site, instances[a:b], Tp=Tp, S_max=S_max) for a, b in zip(bounds[:-1], bounds[1:]) if b > a]
-        self.slices = [(a, b) for a, b in zip(bounds[:-1], bounds[1:]) if b > a]
-        self.streams = [torch.cuda.Stream(device=site.device) for _ in self.parts]
-        self.host_rates = torch.empty((B, site.N, Tp), dtype=torch.float32).pin_memory()
-        self.host_status = torch.empty((B,), dtype=torch.int32).pin_memory()
-        self.host_iters = torch.empty((B,), dtype=torch.int32).pin_memory()
-        self.h2d_bytes = sum(p.h2d_bytes for p in self.parts)
-        self.d2h_bytes = self.host_rates.numel() * 4 + self.host_status.numel() * 4 + self.host_iters.numel() * 4
-
-    def run(self, options: Optional[Options] = None):
-        cur = torch.cuda.current_stream(self.parts[0].site.device)
-        for p, (a, b), st in zip(self.parts, self.slices, self.streams):
-            st.wait_stream(cur)
-            with torch.cuda.stream(st):
-                p.upload().solve(options)
-                self.host_rates[a:b].copy_(p.rates, non_blocking=True)
-                self.host_status[a:b].copy_(p.status, non_blocking=True)
-                self.host_iters[a:b].copy_(p.iters, non_blocking=True)
-        for st in self.streams:  # only after everything is enqueued: the chunks must not serialise through `cur`
-            cur.wait_stream(st)
-        return self
+def _all_zero(min_rates) -> bool:
+    return not bool(np.any(np.asarray(min_rates) != 0))
 
 
 # ------------------------------------------------------------------------ postprocessing

@@ -166,6 +166,22 @@ except Exception:  # noqa: BLE001
             raise NotImplementedError
 
 
+def infrastructure_from_dict(d: Dict) -> InfrastructureInfo:
+    """InfrastructureInfo from its dict form (what the generators produce and TestingInterface holds)."""
+    return InfrastructureInfo(
+        np.array(d["constraint_matrix"]),
+        np.array(d["constraint_limits"]),
+        np.array(d["phases"]),
+        np.array(d["voltages"]),
+        d["constraint_ids"],
+        d["station_ids"],
+        np.array(d["max_pilot"]),
+        np.array(d["min_pilot"]),
+        d.get("allowable_pilots"),
+        d.get("is_continuous"),
+    )
+
+
 class TestingInterface(Interface):
     """Dict-backed Interface used by the reference tests
     (``TestingInterface({...})`` — reference tests/test_adaptive_charging_optimization.py:31-39,
@@ -195,19 +211,7 @@ class TestingInterface(Interface):
         ]
 
     def infrastructure_info(self) -> InfrastructureInfo:
-        d = self.data["infrastructure_info"]
-        return InfrastructureInfo(
-            np.array(d["constraint_matrix"]),
-            np.array(d["constraint_limits"]),
-            np.array(d["phases"]),
-            np.array(d["voltages"]),
-            d["constraint_ids"],
-            d["station_ids"],
-            np.array(d["max_pilot"]),
-            np.array(d["min_pilot"]),
-            d.get("allowable_pilots"),
-            d.get("is_continuous"),
-        )
+        return infrastructure_from_dict(self.data["infrastructure_info"])
 
     def get_prices(self, length: int, start: Optional[int] = None):
         if start is None:
@@ -240,6 +244,7 @@ __all__ = [
     "SessionInfo",
     "InfrastructureInfo",
     "TestingInterface",
+    "infrastructure_from_dict",
     "earliest_deadline_first",
     "HAVE_ACNPORTAL",
 ]

@@ -16,7 +16,7 @@ import torch
 
 from . import _cabi, engine
 from .adaptive_charging_optimization import AdaptiveChargingOptimization, ObjectiveComponent
-from .interface import InfrastructureInfo, SessionInfo, TestingInterface
+from .interface import SessionInfo, TestingInterface, infrastructure_from_dict
 
 
 REPLAY_SOLVER_DEFAULTS = dict(term_floor=1.0, stall_exit=40, alpha=1.7, stall_checks=3)  # warm-started steps: 57 vs 61 mean iterations at the library's 1.8 / 2
@@ -76,10 +76,7 @@ class SiteReplay:
         self.evs = [synthetic_day(infra, seed0 + s, steps, period, mean_sessions) for s in range(n_sites)]
         self.prev_peak = np.zeros(n_sites)  # A
         self.volt = np.asarray(infra["voltages"], dtype=float)
-        self.info = InfrastructureInfo(
-            np.asarray(infra["constraint_matrix"]), np.asarray(infra["constraint_limits"]), np.asarray(infra["phases"]),
-            self.volt, infra["constraint_ids"], infra["station_ids"], np.asarray(infra["max_pilot"]), np.asarray(infra["min_pilot"]),
-            infra.get("allowable_pilots"), infra.get("is_continuous"))
+        self.info = infrastructure_from_dict(infra)
         self.site: Optional[engine.Site] = None
         self._warm = None  # (device tensors, per-instance {session_id: mu}, site index of each batch row)
         self.keep_problems = False  # tests: record (t, site, sessions, prev_peak, schedule, status) of every solved step
@@ -114,7 +111,8 @@ class SiteReplay:
             return
         pb = engine.PackedBatch(self.site, insts, Tp=engine.SUPPORTED_HORIZONS[-1], S_max=len(self.infra["station_ids"]), want_warm_out=True)
         if self.warm_start and self._warm is not None:
-            pb.warm = self._shifted_warm(rows, sessions_of, pb)
+            warm, had = self._previous_rows(rows, sessions_of, pb)
+            pb.set_warm(warm, pb.warm_out, shift=1, had=had)
         pb.upload().solve(self.options)
         pilots = engine.project_continuous(self.site, pb.rates.to(torch.float64))  # pp.py:77-94 on device
         first = pilots[:, :, 0].cpu().numpy()
@@ -137,30 +135,23 @@ class SiteReplay:
         mu = pb.warm_out["mu"].cpu().numpy()
         self._warm = (pb.warm_out, [dict(zip(ids, mu[b, : len(ids)])) for b, ids in enumerate(sessions_of)], rows)
 
-    def _shifted_warm(self, rows, sessions_of, pb):
-        """Previous state shifted by one period: column t of the new problem is column t+1 of
-        the old one; multipliers follow their session; rho and the peak level carry over."""
+    def _previous_rows(self, rows, sessions_of, pb):
+        """The previous step's state, row by row of this batch (which holds the active sites only): multipliers follow
+        their session; the solve reads it one period ahead.  Sites without a row in the previous batch start cold.
+        Returns (warm state, had-row mask)."""
         old, old_mu, old_rows = self._warm
         pos = {s: b for b, s in enumerate(old_rows)}
         idx = [pos.get(s, -1) for s in rows]
         dev = old["v1"].device
-        have = torch.tensor([i >= 0 for i in idx], device=dev)
+        had = torch.tensor([i >= 0 for i in idx], dtype=torch.int32, device=dev)
         gather = torch.tensor([max(i, 0) for i in idx], device=dev)
-
-        def shift(x):
-            y = torch.zeros_like(x[gather])
-            y[:, :, :-1] = x[gather][:, :, 1:]
-            return y * have[:, None, None]
-
         mu = np.zeros((len(rows), pb.S_max), dtype=np.float32)
         for b, (i, ids) in enumerate(zip(idx, sessions_of)):
             if i >= 0:
                 m = old_mu[i]
                 mu[b, : len(ids)] = [m.get(sid, 0.0) for sid in ids]
-        scal = old["scal"][gather].clone()
-        scal[~have] = 0.0  # rho <= 0 => kernel falls back to rho0
-        return dict(v1=shift(old["v1"]).contiguous(), vc=shift(old["vc"]).contiguous(),
-                    mu=torch.from_numpy(mu).to(dev), scal=scal.contiguous())
+        warm = dict(v1=old["v1"][gather], vc=old["vc"][gather], mu=torch.from_numpy(mu).to(dev), scal=old["scal"][gather])
+        return warm, had
 
     def run(self, t0: int = 0, t1: Optional[int] = None) -> ReplayStats:
         stats = ReplayStats()

@@ -21,7 +21,7 @@ import torch
 
 from . import _cabi, engine
 from .adaptive_charging_optimization import ObjectiveComponent, pack_objective
-from .interface import InfrastructureInfo, TestingInterface
+from .interface import TestingInterface, infrastructure_from_dict
 from .replay import REPLAY_SOLVER_DEFAULTS, synthetic_day
 
 
@@ -59,10 +59,7 @@ class FleetReplay:
         self.demand_charge = demand_charge
         self.volt = np.asarray(infra["voltages"], dtype=float)
         self.N = len(infra["station_ids"])
-        self.info = InfrastructureInfo(
-            np.asarray(infra["constraint_matrix"]), np.asarray(infra["constraint_limits"]), np.asarray(infra["phases"]),
-            self.volt, infra["constraint_ids"], infra["station_ids"], np.asarray(infra["max_pilot"]), np.asarray(infra["min_pilot"]),
-            infra.get("allowable_pilots"), infra.get("is_continuous"))
+        self.info = infrastructure_from_dict(infra)
         from .batched import pilot_mode
 
         self.pilot_mode = pilot_mode(quantize, reallocate, self.info)
@@ -94,8 +91,9 @@ class FleetReplay:
         self._w_ev = self.volt[self.ev_station] * period / 1e3 / 60  # kWh per A-period of each EV's EVSE
         self.prev_peak = np.zeros(n_sites)  # A
         self.site: Optional[engine.Site] = None
-        self._prev = None  # (warm_out tensors, EV index / site / position of the previous step's sessions, had-sessions mask)
+        self._prev = None  # (EV index / site / position of the previous step's sessions, had-sessions mask)
         self._pb: Optional[engine.PackedBatch] = None  # one batch object for the whole replay (refilled every step)
+        self._state = None  # two sets of warm-state tensors: a step reads the previous step's set and writes the other
         self.stats = FleetStats()
 
     # ------------------------------------------------------------------ packing
@@ -185,11 +183,12 @@ class FleetReplay:
             use_u = bool((h["gamma"] > 0).any() or (h["peak_w"] > 0).any())
             self.site = engine.get_site(self.info, "SOC", False, use_u, self.device)
         if self._pb is None:
-            self._pb = engine.PackedBatch.from_arrays(self.site, h, self.Tp, self.N, multi_session=False, want_warm_out=True)
+            self._pb = engine.PackedBatch.from_arrays(self.site, h, self.Tp, self.N, multi_session=False)
+            self._state = [self._pb.new_warm_state(), self._pb.new_warm_state()]
         else:
             self._pb.refill(h)  # same shapes every step: reuse the pinned staging and the device buffers
         pb = self._pb
-        pb.warm = None
+        prev, out = self._state
         dev = pb.device
         t1 = time.perf_counter()
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -197,7 +196,9 @@ class FleetReplay:
         idx_d = torch.from_numpy(idx).to(dev)
         s_d, pos_d = torch.from_numpy(s).to(dev), torch.from_numpy(pos).to(dev)
         if self.warm_start and self._prev is not None:
-            pb.warm = self._shifted_warm(idx_d, s_d, pos_d, pb)
+            pb.set_warm(self._warm(prev, idx_d, s_d, pos_d), out, shift=1, had=self._prev[-1])
+        else:
+            pb.set_warm(None, out)
         pb.upload().solve(self.options)
         pilots = self._project(pb.rates.to(torch.float64), h, idx, s, pos)
         first = pilots[:, :, 0].contiguous().cpu().numpy()
@@ -211,7 +212,8 @@ class FleetReplay:
         e = np.minimum(first[self.ev_site[present], self.ev_station[present]] * self._w_ev[present], self.ev_req[present] - self.ev_dlv[present])
         self.ev_dlv[present] += np.maximum(e, 0.0)
         self.prev_peak = np.maximum(self.prev_peak, first.sum(axis=1))
-        self._prev = (pb.warm_out, idx_d, s_d, pos_d, torch.from_numpy(n_sess > 0).to(dev))
+        self._prev = (idx_d, s_d, pos_d, torch.from_numpy((n_sess > 0).astype(np.int32)).to(dev))
+        self._state.reverse()
         act = n_sess > 0
         st_ = self.stats
         st_.iters_mean.append(float(it[act].mean()) if act.any() else 0.0)
@@ -241,24 +243,15 @@ class FleetReplay:
             return engine.reallocate(self.site, 1, rates, h["n_sessions"], h["sess_row"], h["sess_start"], ramp, max0)
         return engine.project_discrete(self.site, rates)
 
-    def _shifted_warm(self, idx_d, s_d, pos_d, pb):
-        """Previous state shifted by one period (column t of the new problem is column t+1 of the
-        old one); multipliers follow their EV; rho and the peak level carry over.  Sites that were
-        idle in the previous step start cold, like SiteReplay."""
-        old, pidx, ps, ppos, had = self._prev
-        dev = pb.device
-
-        def shift(x):
-            y = torch.zeros_like(x)
-            y[:, :, :-1] = x[:, :, 1:]
-            return y * had[:, None, None]
-
-        mu_ev = torch.zeros(len(self.ev_req), dtype=torch.float32, device=dev)
-        mu_ev[pidx] = old["mu"][ps, ppos]
-        mu = torch.zeros((self.n_sites, pb.S_max), dtype=torch.float32, device=dev)
-        mu[s_d, pos_d] = mu_ev[idx_d] * had[s_d]
-        scal = old["scal"] * had[:, None]  # rho <= 0 => the kernel falls back to rho0
-        return dict(v1=shift(old["v1"]), vc=shift(old["vc"]), mu=mu, scal=scal.contiguous())
+    def _warm(self, prev, idx_d, s_d, pos_d):
+        """The previous step's state for this step's solve, which reads it one period ahead (sites idle before start
+        cold through warm_had); the session multipliers follow their EV."""
+        pidx, ps, ppos, _ = self._prev
+        mu_ev = torch.zeros(len(self.ev_req), dtype=torch.float32, device=prev["mu"].device)
+        mu_ev[pidx] = prev["mu"][ps, ppos]
+        mu = torch.zeros_like(prev["mu"])
+        mu[s_d, pos_d] = mu_ev[idx_d]
+        return dict(prev, mu=mu)
 
     def run(self, t0: int = 0, t1: Optional[int] = None) -> FleetStats:
         for t in range(t0, self.steps if t1 is None else t1):
@@ -326,17 +319,8 @@ class DeviceFleetReplay(FleetReplay):
         f.ev_station, f.ev_arr, f.ev_dep, f.ev_req, f.ev_max = p(d["station"]), p(d["arr"]), p(d["dep"]), p(d["req"]), p(d["mx"])
         f.ev_dlv, f.ev_mu, f.day_site_off, f.prev_peak, f.had = p(d["dlv"]), p(d["mu"]), p(d["off"]), p(d["prev_peak"]), p(d["had"])
         self._fleet = f
-        # two sets of warm-state buffers: a step reads the previous step's and writes its own
-        R = max(self.site.R, 1)
-        mk = lambda *shape: torch.zeros(shape, dtype=torch.float32, device=dev)  # noqa: E731
-        self._state = [dict(v1=mk(self.n_sites, self.N, self.Tp), vc=mk(self.n_sites, R, self.Tp), mu=mk(self.n_sites, self.N), scal=mk(self.n_sites, 2))
-                       for _ in range(2)]
-        self._k = 0
-        b = ch.batch
-        b.lb_zero, b.multi_session = 1, 0
-        b.warm_shift = 1
-        b.warm_had = p(d["had"])
-        b.warm_mu = p(d["warm_mu"])
+        self._state = [ch.new_warm_state(), ch.new_warm_state()]
+        ch.lb_zero = True  # the synthetic EVs have no minimum rate
         o = ch.objective
         o.prev_peak = p(d["prev_peak"])
         o.prices_stride = 0  # one price vector for the whole fleet, read from the current period on
@@ -346,26 +330,22 @@ class DeviceFleetReplay(FleetReplay):
     def step(self, t: int, want_first: bool = True):
         C, L, ch, d, p = self._C, _cabi.lib(), self._ch, self._d, engine._ptr
         st = C.c_void_p(torch.cuda.current_stream(self._bac.device).cuda_stream)
-        b, o = ch.batch, ch.objective
-        cur, prev = self._state[self._k], self._state[1 - self._k]
-        if self.warm_start and self._started:
-            b.warm_v1, b.warm_vc, b.warm_scal, b.warm_mu = p(prev["v1"]), p(prev["vc"]), p(prev["scal"]), p(d["warm_mu"])
-        else:
-            b.warm_v1 = b.warm_vc = b.warm_scal = b.warm_mu = None
-        b.out_v1, b.out_vc, b.out_mu, b.out_scal = p(cur["v1"]), p(cur["vc"]), p(cur["mu"]), p(cur["scal"])
+        o = ch.objective
+        prev, out = self._state
+        ch.set_warm(dict(prev, mu=d["warm_mu"]) if self.warm_start and self._started else None, out, shift=1, had=d["had"])
         o.prices = C.c_void_p(d["prices"].data_ptr() + 8 * t) if self._bac.need_prices else None
         _cabi.check(L.acb_fleet_sessions(self.site.handle, C.byref(self._fleet), t, C.byref(ch.sessions), p(d["sess_ev"]), p(d["warm_mu"]), st), "acb_fleet_sessions")
-        _cabi.check(L.acb_pack_sessions(self.site.handle, C.byref(ch.sessions), C.byref(o), C.byref(b), p(ch.flags), st), "acb_pack_sessions")
-        _cabi.check(L.acb_solve_batch(self.site.handle, C.byref(b), C.byref(self._bac.options), st), "acb_solve_batch")
+        _cabi.check(L.acb_pack_sessions(self.site.handle, C.byref(ch.sessions), C.byref(o), C.byref(ch.struct), p(ch.flags), st), "acb_pack_sessions")
+        ch.solve(self._bac.options, st)
         if self.pilot_mode:  # the solve skipped the continuous projection (batch.pilots NULL); acb_fleet_apply reads batch.pilots
-            _cabi.check(L.acb_quantize_pilots(self.site.handle, self.pilot_mode, C.byref(ch.sessions), float(self.period), C.byref(b), p(ch.pilots), st),
+            _cabi.check(L.acb_quantize_pilots(self.site.handle, self.pilot_mode, C.byref(ch.sessions), float(self.period), C.byref(ch.struct), p(ch.pilots), st),
                         "acb_quantize_pilots")
-            b.pilots = p(ch.pilots)
-        _cabi.check(L.acb_fleet_apply(self.site.handle, C.byref(self._fleet), t, float(self.period), C.byref(b), p(d["sess_ev"]),
+            ch.bind_pilots(True)
+        _cabi.check(L.acb_fleet_apply(self.site.handle, C.byref(self._fleet), t, float(self.period), C.byref(ch.struct), p(d["sess_ev"]),
                                       p(d["first"]) if want_first else None, p(d["stats"]), st), "acb_fleet_apply")
         if self.pilot_mode:
-            b.pilots = None
-        self._k = 1 - self._k
+            ch.bind_pilots(False)
+        self._state.reverse()
         self._started = True
         return d["first"].cpu().numpy() if want_first else None
 

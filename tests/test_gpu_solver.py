@@ -203,29 +203,6 @@ def test_infrastructure_infeasibility_is_certified_early(require_gpu, path):
     assert aco.last_info["status"] == 2 and aco.last_info["iters"] <= 3000, aco.last_info
 
 
-def test_host_pipeline_equals_one_batch(require_gpu):
-    """engine.HostPipeline (chunks on their own streams, pinned host results) returns exactly what one PackedBatch does."""
-    import torch
-
-    obj = [ab.ObjectiveComponent(ab.tou_energy_cost), ab.ObjectiveComponent(ab.total_energy, 0.3), ab.ObjectiveComponent(ab.demand_charge, 1 / 30)]
-    insts = []
-    for seed in range(10):
-        iface = ab.TestingInterface(config_c2(seed + 70))
-        S, I = iface.active_sessions(), iface.infrastructure_info()
-        aco = ab.AdaptiveChargingOptimization(obj, iface)
-        insts.append(aco.build_instance(S, I, None, iface.get_prev_peak()))
-    site = aco._site_for(I, insts[0])
-    pb = engine.PackedBatch(site, insts).upload().solve()
-    pipe = engine.HostPipeline(site, insts, chunks=3).run()
-    torch.cuda.synchronize()
-    np.testing.assert_array_equal(pipe.host_status.numpy(), pb.status.cpu().numpy())
-    np.testing.assert_array_equal(pipe.host_iters.numpy(), pb.iters.cpu().numpy())
-    np.testing.assert_array_equal(pipe.host_rates.numpy(), pb.rates.cpu().numpy())
-    pipe.run()  # reusable
-    torch.cuda.synchronize()
-    np.testing.assert_array_equal(pipe.host_rates.numpy(), pb.rates.cpu().numpy())
-
-
 def _cabi_opts(**kw):
     from adacharge_b200 import _cabi
 

@@ -1,7 +1,7 @@
 """Warm start of acb_solve_batch on both solve paths, at the C ABI (acb_batch.warm_* / out_*):
 
 - the state a solve writes (out_v1, out_vc, out_mu, out_scal), fed to the next control step with warm_shift = 1, gives
-  bit for bit what the same state shifted one column on the host gives with warm_shift = 0 (FleetReplay._shifted_warm);
+  bit for bit what the same state shifted one column on the host gives with warm_shift = 0;
 - warm_had = 0 is a cold solve, bit for bit, whatever the warm arrays hold, also with positive minimum rates (v then
   starts at clamp(0, lb, ub), not at 0) and with the second stagnation rescue allowed (it is for warm-started solves);
 - the device fleet replay equals the host fleet replay, and warm-started replay steps match a cold oracle solve, on the
@@ -80,7 +80,7 @@ def test_warm_shift_equals_host_shifted_state(require_gpu, case):
         assert prev["status"][0] == 0
         dev = {k: torch.from_numpy(prev["out_" + k]).cuda() for k in ("v1", "vc", "mu", "scal")}
 
-        def shift(x):  # column t of the new problem is column t + 1 of the old one (FleetReplay._shifted_warm)
+        def shift(x):  # column t of the new problem is column t + 1 of the old one
             y = torch.zeros_like(x)
             y[:, :, :-1] = x[:, :, 1:]
             return y

@@ -6,7 +6,7 @@ import common
 from adacharge_b200 import _cabi, engine
 site, insts, _ = common.build_instances(148, 0)
 pb = engine.PackedBatch(site, insts, want_warm_out=True).upload()
-pb.warm_out["mu"] = torch.zeros((148, 256), dtype=torch.float32, device=pb.rates.device)
+pb.warm_out = dict(pb.warm_out, mu=torch.zeros((148, 256), dtype=torch.float32, device=pb.rates.device))
 opt = _cabi.default_options(max_iter=300)
 pb.solve(opt); torch.cuda.synchronize()
 m = pb.warm_out["mu"][0, :160].cpu().numpy().reshape(32, 5)
