@@ -18,7 +18,7 @@ ACB_PILOTS_DISCRETE, ACB_PILOTS_REALLOCATE = 1, 2  # acb_quantize_pilots modes
 EXPORTS = [
     "acb_site_create", "acb_site_destroy", "acb_site_dims", "acb_site_max_horizon", "acb_default_options",
     "acb_solve_batch", "acb_charging_rate_bounds", "acb_project_continuous", "acb_project_discrete",
-    "acb_reallocate", "acb_quantize_pilots", "acb_constraints_feasible", "acb_min_rate_admission", "acb_pack_sessions", "acb_preprocess_sessions", "acb_fleet_sessions", "acb_fleet_apply", "acb_last_error", "acb_version",
+    "acb_reallocate", "acb_quantize_pilots", "acb_constraints_feasible", "acb_min_rate_admission", "acb_admit_sessions", "acb_pack_sessions", "acb_preprocess_sessions", "acb_fleet_sessions", "acb_fleet_apply", "acb_last_error", "acb_version",
 ]
 ACB_MAX_COMPONENTS = 16
 # acb_objective.kind values (include/adacharge_b200.h)
@@ -52,12 +52,14 @@ class Batch(C.Structure):
         ("warm_v1", _P), ("warm_vc", _P), ("warm_mu", _P), ("warm_scal", _P), ("warm_shift", C.c_int32), ("warm_had", _P),
         ("out_v1", _P), ("out_vc", _P), ("out_mu", _P), ("out_scal", _P),
         ("rates", _P), ("pilots", _P), ("rate_est", _P), ("status", _P), ("iters", _P), ("stats", _P),
+        ("sess_min0", _P), ("sess_max0", _P),
     ]
 
 
 class Sessions(C.Structure):
     _fields_ = [("B", C.c_int32), ("S_max", C.c_int32), ("station", _P), ("arrival_offset", _P), ("remaining_time", _P),
-                ("remaining_demand", _P), ("min_rate", _P), ("max_rate", _P)]
+                ("remaining_demand", _P), ("min_rate", _P), ("max_rate", _P), ("arrival", _P), ("min_rate0", _P),
+                ("max_rate0", _P)]
 
 
 class Objective(C.Structure):
@@ -101,6 +103,7 @@ def lib():
     L.acb_quantize_pilots.argtypes = [_P, C.c_int, C.POINTER(Sessions), C.c_double, C.POINTER(Batch), _P, _P]
     L.acb_constraints_feasible.argtypes = [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P]
     L.acb_min_rate_admission.argtypes = [_P, C.c_int, C.c_int, _P, _P, _P, _P, _P]
+    L.acb_admit_sessions.argtypes = [_P, C.POINTER(Sessions), _P, C.c_double, C.c_double, C.c_int32, _P]
     L.acb_preprocess_sessions.argtypes = [_P, C.POINTER(Sessions), C.c_int, _P, _P]
     L.acb_fleet_sessions.argtypes = [_P, C.POINTER(Fleet), C.c_int, C.POINTER(Sessions), _P, _P, _P]
     L.acb_fleet_apply.argtypes = [_P, C.POINTER(Fleet), C.c_int, C.c_double, C.POINTER(Batch), _P, _P, _P, _P]

@@ -103,6 +103,8 @@ class _Chunk(engine.DeviceBatch):
             raw["peak_limit"] = ((B, Tp), np.float64)
         if owner.estimate_max_rate:
             raw["upper_bound"] = ((B, S), np.float64)
+        if owner.uninterrupted_charging:
+            raw["arrival"] = ((B, S), np.int32)
         self.host = {k: torch.empty(shape, dtype=torch.from_numpy(np.empty(0, dt)).dtype).pin_memory() for k, (shape, dt) in raw.items()}
         self.dev_raw = {k: torch.empty_like(v, device=dev) for k, v in self.host.items()}
         self.h2d_bytes = sum(v.numel() * v.element_size() for v in self.host.values())
@@ -117,6 +119,9 @@ class _Chunk(engine.DeviceBatch):
             d["peak_limit"] = mk((B, Tp), f32)
         if owner.need_sess_quad:
             d["sess_quad"] = mk((B, S), f32)
+        if owner.uninterrupted_charging:  # first-period limits: acb_admit_sessions -> the packer -> the solve
+            d["sess_min0"], d["sess_max0"] = mk((B, S), f32), mk((B, S), f32)
+            self.limits0 = {k: mk((B, S), torch.float64) for k in ("min_rate0", "max_rate0")}
         # pilots: continuous from the solve's epilogue; quantised from acb_quantize_pilots, without that projection first
         super().__init__(owner.site, d, Tp, S, multi_session=owner.multi_session, pilots=True)
         self.bind_pilots(not owner.pilot_mode)
@@ -127,6 +132,8 @@ class _Chunk(engine.DeviceBatch):
         s.B, s.S_max = B, S
         for n, _ in SESSION_FIELDS:
             setattr(s, n, p(self.dev_raw[n]))
+        if owner.uninterrupted_charging:
+            s.arrival, s.min_rate0, s.max_rate0 = p(self.dev_raw["arrival"]), p(self.limits0["min_rate0"]), p(self.limits0["max_rate0"])
         self.sessions = s
         o = _cabi.Objective()
         o.n = len(owner.components)
@@ -162,12 +169,20 @@ class BatchedAdaptiveCharging:
         quantize, reallocate: as AdaptiveSchedulingAlgorithm's (ada.py:101-113, 177-190): pilots rounded down into each
             EVSE's allowable set (every EVSE needs one), and with ``reallocate`` the first period's rounding loss given
             back greedily.  Bit-identical to the drop-in class with the same flags.
+        uninterrupted_charging: as AdaptiveSchedulingAlgorithm's (ada.py:149-150, acnportal's apply_minimum_charging_rate
+            with override = period): the sessions of each instance are put in arrival order and, while the network stays
+            feasible, each is given min(min_pilot, period) as its first-period minimum; a refused session gets 0 A in the
+            first period.  ``schedule`` then needs the sessions' absolute ``arrival``.  Bit-identical to the drop-in class.
+        skip_unabsorbable: with uninterrupted_charging, a session whose remaining energy is less than one period at its
+            try rate is not offered the minimum (it keeps its own limits) instead of making the instance infeasible, as
+            the drop-in class does.  For closed-loop use; off by default.
     """
 
     def __init__(self, objective: List[aco.ObjectiveComponent], infrastructure, period, batch: int, max_sessions: int, horizon: int,
                  constraint_type="SOC", enforce_energy_equality=False, peak_limit=False, multi_session=False, demand_charge=0.0,
                  per_instance_demand_charge=False, solver_options: Optional[dict] = None, device=None, chunks: int = 4,
-                 enforce_pilot_limit=True, estimate_max_rate=False, quantize=False, reallocate=False):
+                 enforce_pilot_limit=True, estimate_max_rate=False, quantize=False, reallocate=False, uninterrupted_charging=False,
+                 skip_unabsorbable=False):
         if isinstance(infrastructure, dict):
             infrastructure = infrastructure_from_dict(infrastructure)
         self.pilot_mode = pilot_mode(quantize, reallocate, infrastructure)
@@ -188,6 +203,12 @@ class BatchedAdaptiveCharging:
         # estimate_max_rate, the estimator's per-session upper bounds (passed to schedule() as `upper_bound`)
         self.enforce_pilot_limit, self.estimate_max_rate = bool(enforce_pilot_limit), bool(estimate_max_rate)
         self.demand_charge_scalar = float(demand_charge)
+        self.uninterrupted_charging, self.skip_unabsorbable = bool(uninterrupted_charging), bool(skip_unabsorbable)
+        if self.uninterrupted_charging:
+            mp = np.asarray(infrastructure.min_pilot, dtype=np.float64)
+            # try rate of each EVSE, min(min_pilot, override) as the reference writes it; any try > 0 rules out lb_zero
+            self.try_rate = np.array([min(infrastructure.min_pilot[i], period) for i in range(len(mp))], dtype=np.float64)
+            self.min_pilot = torch.from_numpy(mp).to(self.device)
         opts = dict(solver_options or {})
         if K["equal_share"] not in kinds:
             opts.setdefault("rate_tol", 0.0)  # no strictly convex term: nothing for the rate polish to do
@@ -205,16 +226,18 @@ class BatchedAdaptiveCharging:
         self.h2d_bytes = sum(c.h2d_bytes for c in self.chunks)
         self.d2h_bytes = sum(t.numel() * t.element_size() for t in (self.host_pilots, self.host_status, self.host_iters, self.host_T, self.host_stats))
         # own kernels per call and chunk: the packer + the solve (three launches when phased: solve, relaunch list, solve;
-        # the general path launches per phase and is not counted here) + the preprocessing + the quantised pilots
+        # the general path launches per phase and is not counted here) + the preprocessing + the admission + the quantised pilots
         phased = self.options.phase_iters > 0 and self.options.phase_iters < self.options.max_iter
         self.kernel_launches_per_call = len(self.chunks) * (1 + (3 if phased else 1) + int(self.enforce_pilot_limit or self.estimate_max_rate)
-                                                            + int(self.pilot_mode != 0))
+                                                            + int(self.uninterrupted_charging) + int(self.pilot_mode != 0))
 
     # ------------------------------------------------------------------------------------------------
     def _stage(self, ch: _Chunk, arrays: Dict[str, np.ndarray]):
         """host arrays -> the chunk's pinned staging (a plain memcpy per field)."""
-        # every minimum rate 0 (the usual case) is declared to the library: fastest on-chip variant
-        ch.lb_zero = not np.any(np.asarray(arrays["min_rate"])[ch.lo:ch.hi] != 0)
+        # every minimum rate 0 (the usual case) is declared to the library: fastest on-chip variant.  With uninterrupted
+        # charging an admitted session's first-period minimum is its EVSE's try rate: only try rates of 0 keep the promise
+        ch.lb_zero = not np.any(np.asarray(arrays["min_rate"])[ch.lo:ch.hi] != 0) and not (
+            self.uninterrupted_charging and np.any(self.try_rate > 0))
         for k, dst in ch.host.items():
             src = arrays.get(k)
             if src is None:
@@ -247,6 +270,8 @@ class BatchedAdaptiveCharging:
             if self.enforce_pilot_limit or self.estimate_max_rate:
                 _cabi.check(L.acb_preprocess_sessions(self.site.handle, C.byref(ch.sessions), int(self.enforce_pilot_limit),
                                                       engine._ptr(ch.dev_raw.get("upper_bound")), st), "acb_preprocess_sessions")
+            if self.uninterrupted_charging:
+                self.admit(ch, st)
             _cabi.check(L.acb_pack_sessions(self.site.handle, C.byref(ch.sessions), C.byref(ch.objective), C.byref(ch.struct), engine._ptr(ch.flags), st), "acb_pack_sessions")
             if events is not None:
                 ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
@@ -266,6 +291,15 @@ class BatchedAdaptiveCharging:
                 self.host_stats[ch.lo:ch.hi].copy_(ch.stats, non_blocking=True)
                 ch.flags_host.copy_(ch.flags, non_blocking=True)
 
+    def admit(self, ch: _Chunk, stream):
+        """Enqueue acb_admit_sessions on the chunk's raw tables (in place: arrival order, first-period limits)."""
+        _cabi.check(_cabi.lib().acb_admit_sessions(self.site.handle, C.byref(ch.sessions), engine._ptr(self.min_pilot), float(self.period),
+                                                   float(self.period), int(self.skip_unabsorbable), stream), "acb_admit_sessions")
+
+    def _check_arrays(self, sessions):
+        if self.uninterrupted_charging and sessions.get("arrival") is None:
+            raise ValueError("uninterrupted_charging needs the sessions' absolute `arrival` (the admission takes them in arrival order)")
+
     def schedule_async(self, sessions: Dict[str, np.ndarray], prices=None, prev_peak=None, demand_charge=None, external_signal=None, peak_limit=None,
                        upper_bound=None, independent=False, start_event=None):
         """Stage, copy, pack, solve and copy back, chunk by chunk; returns after everything is enqueued.  By default the
@@ -273,6 +307,7 @@ class BatchedAdaptiveCharging:
         synchronize of the current stream makes ``result()`` valid.  ``independent=True`` leaves the current stream out
         (the chunks start after ``start_event`` if given): calls on different objects then overlap on the device
         (double buffering); use ``wait()`` / ``join()`` before reading the result."""
+        self._check_arrays(sessions)
         self.wait()  # the pinned staging and the result buffers of the previous call on this object are reused
         arrays = dict(sessions)
         arrays.update(prices=prices, prev_peak=prev_peak, demand_charge=demand_charge, external_signal=external_signal, peak_limit=peak_limit,
@@ -329,6 +364,7 @@ class BatchedAdaptiveCharging:
 
     # resident form (bench `value`): raw arrays already on the device, results stay there
     def upload_raw(self, sessions: Dict[str, np.ndarray], **kw):
+        self._check_arrays(sessions)
         arrays = dict(sessions)
         arrays.update(kw)
         for ch in self.chunks:
@@ -351,11 +387,12 @@ class BatchedAdaptiveCharging:
 
 
 def sessions_to_arrays(session_lists, infrastructure, S_max: Optional[int] = None) -> Dict[str, np.ndarray]:
-    """Lists of SessionInfo (one list per instance) -> the [B, S_max] tables ``schedule`` takes.  Convenience for
-    callers that hold reference-style objects; sessions must carry constant min/max rates."""
+    """Lists of SessionInfo (one list per instance) -> the [B, S_max] tables ``schedule`` takes, with ``arrival``
+    (absolute, for uninterrupted_charging).  Convenience for callers that hold reference-style objects; sessions must
+    carry constant min/max rates."""
     B = len(session_lists)
     S = S_max or max(1, max(len(s) for s in session_lists))
-    out = {n: np.zeros((B, S), dtype=dt) for n, dt in SESSION_FIELDS}
+    out = {n: np.zeros((B, S), dtype=dt) for n, dt in SESSION_FIELDS + (("arrival", np.int32),)}
     out["station"][...] = -1
     for b, ss in enumerate(session_lists):
         for j, s in enumerate(ss):
@@ -364,6 +401,7 @@ def sessions_to_arrays(session_lists, infrastructure, S_max: Optional[int] = Non
                 raise ValueError("sessions_to_arrays: time-varying rate limits need the per-instance packer (AdaptiveChargingOptimization)")
             out["station"][b, j] = infrastructure.get_station_index(s.station_id)
             out["arrival_offset"][b, j] = s.arrival_offset
+            out["arrival"][b, j] = s.arrival
             out["remaining_time"][b, j] = s.remaining_time
             out["remaining_demand"][b, j] = s.remaining_demand
             out["min_rate"][b, j] = mn.flat[0] if mn.size else 0.0

@@ -42,6 +42,8 @@ __global__ void acb_pack_kernel(SiteDev S, acb_sessions X, acb_objective O, acb_
     float* o_min = const_cast<float*>(B.min_rates) + base;
     float* o_max = const_cast<float*>(B.max_rates) + base;
     float* o_sq = B.sess_quad ? const_cast<float*>(B.sess_quad) + base : nullptr;
+    float* o_min0 = B.sess_min0 ? const_cast<float*>(B.sess_min0) + base : nullptr;
+    float* o_max0 = B.sess_max0 ? const_cast<float*>(B.sess_max0) + base : nullptr;
     for (int s = tid; s < Sm; s += nt) {
         const int k = key[s];
         if (k == 0x7fffffff) continue;
@@ -58,6 +60,10 @@ __global__ void acb_pack_kernel(SiteDev S, acb_sessions X, acb_objective O, acb_
         o_off[rank] = -(int)(base + rank + 1);
         o_min[rank] = (float)X.min_rate[base + s];
         o_max[rank] = (float)fmin(X.max_rate[base + s], 3.0e38);
+        if (o_min0) {  // first-period limits (uninterrupted charging), rounded like min_rates / max_rates
+            o_min0[rank] = (float)(X.min_rate0 ? X.min_rate0[base + s] : X.min_rate[base + s]);
+            o_max0[rank] = (float)fmin(X.max_rate0 ? X.max_rate0[base + s] : X.max_rate[base + s], 3.0e38);
+        }
         if (o_sq) {  // non_completion_penalty, norm 2: coefficient * (kWh per A*period)^2 per session
             double c2 = 0.0;
             for (int c = 0; c < O.n; ++c)
@@ -65,7 +71,7 @@ __global__ void acb_pack_kernel(SiteDev S, acb_sessions X, acb_objective O, acb_
             o_sq[rank] = (float)(c2 * w * w);
         }
     }
-    for (int s = n + tid; s < Sm; s += nt) { o_row[s] = 0; o_start[s] = 0; o_len[s] = 0; o_en[s] = 0.f; o_off[s] = -(int)(base + s + 1); o_min[s] = 0.f; o_max[s] = 0.f; if (o_sq) o_sq[s] = 0.f; }
+    for (int s = n + tid; s < Sm; s += nt) { o_row[s] = 0; o_start[s] = 0; o_len[s] = 0; o_en[s] = 0.f; o_off[s] = -(int)(base + s + 1); o_min[s] = 0.f; o_max[s] = 0.f; if (o_sq) o_sq[s] = 0.f; if (o_min0) { o_min0[s] = 0.f; o_max0[s] = 0.f; } }
     __syncthreads();
     if (tid == 0) {
         const_cast<int32_t*>(B.T)[b] = T;

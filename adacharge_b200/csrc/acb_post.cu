@@ -348,7 +348,7 @@ __global__ void __launch_bounds__(ACB_QP_THREADS) k_quantize_pilots(SiteDev S, i
             s_start[j] = X.arrival_offset[base + s];
             // interface.remaining_amp_periods: remaining_demand * 1000 / voltage * (60 / period), in this order
             s_ramp[j] = __dmul_rn(__ddiv_rn(__dmul_rn(X.remaining_demand[base + s], 1000.0), S.volt[row]), per_period);
-            s_max0[j] = X.max_rate[base + s];
+            s_max0[j] = X.max_rate0 ? X.max_rate0[base + s] : X.max_rate[base + s];  // max_rates[0]
         }
         n += __popc(m);
     }
@@ -382,28 +382,117 @@ __global__ void k_feasible(SiteDev S, const double* rates, int B, int T, int col
     if (lane == 0) feasible[b] = ok ? 1 : 0;
 }
 
-// Preprocessing greedy of apply_minimum_charging_rate (acnportal, called at adacharge.py:149-150): sessions are
-// offered in the caller's order; a session keeps its minimum rate if the network stays feasible with everything
-// admitted before it.  One warp per instance.
-__global__ void k_min_rate_admission(SiteDev S, int B, int S_max, const int32_t* n_sessions, const int32_t* sess_row,
-                                     const double* try_rate, int32_t* admitted) {
-    extern __shared__ __align__(16) unsigned char smraw[];
-    double* col = reinterpret_cast<double*>(smraw);
-    const int b = blockIdx.x, lane = threadIdx.x;
+// Preprocessing greedy of apply_minimum_charging_rate (acnportal, called at adacharge.py:149-150): the n sessions are
+// offered in list order; a session keeps its minimum rate if the network stays feasible with everything admitted
+// before it.  Run by one full warp; col [N] is the first column being built (zeroed here).
+__device__ void min_rate_greedy(const SiteDev& S, double* col, int n, const int32_t* row, const double* try_rate, int32_t* admitted,
+                                int lane) {
     for (int i = lane; i < S.N; i += 32) col[i] = 0.0;
     __syncwarp();
-    const int nS = n_sessions[b];
-    for (int s = 0; s < nS; ++s) {
-        const size_t k = (size_t)b * S_max + s;
-        const int i = sess_row[k];
-        if (lane == 0) col[i] = try_rate[k];
+    for (int s = 0; s < n; ++s) {
+        const int i = row[s];
+        if (lane == 0) col[i] = try_rate[s];
         __syncwarp();
         const bool ok = warp_feasible(S, col, lane);
         if (lane == 0) {
             if (!ok) col[i] = 0.0;
-            admitted[k] = ok ? 1 : 0;
+            admitted[s] = ok ? 1 : 0;
         }
         __syncwarp();
+    }
+}
+
+// One warp per instance, sessions in the caller's order.
+__global__ void k_min_rate_admission(SiteDev S, int B, int S_max, const int32_t* n_sessions, const int32_t* sess_row,
+                                     const double* try_rate, int32_t* admitted) {
+    extern __shared__ __align__(16) unsigned char smraw[];
+    const size_t k = (size_t)blockIdx.x * S_max;
+    min_rate_greedy(S, reinterpret_cast<double*>(smraw), n_sessions[blockIdx.x], sess_row + k, try_rate + k, admitted + k, threadIdx.x);
+}
+
+// acb_admit_sessions: one warp per instance.  Shared memory: the instance's raw tables (staged for the in-place
+// permutation), the candidates of the greedy and its first column.
+#define ACB_ADMIT_DBL 3  // remaining_demand, min_rate, max_rate
+#define ACB_ADMIT_INT 4  // station, arrival_offset, remaining_time, arrival
+static size_t admit_smem_bytes(int N, int S_max) {
+    return (size_t)S_max * (ACB_ADMIT_DBL + 1) * sizeof(double) + (size_t)N * sizeof(double) +
+           (size_t)S_max * (ACB_ADMIT_INT + 3) * sizeof(int32_t);
+}
+
+__global__ void k_admit_sessions(SiteDev S, acb_sessions X, const double* min_pilot, double override, double period, int skip) {
+    extern __shared__ __align__(16) unsigned char smraw[];
+    const int b = blockIdx.x, lane = threadIdx.x, Sm = X.S_max, N = S.N;
+    double* d_dem = reinterpret_cast<double*>(smraw);
+    double* d_min = d_dem + Sm;
+    double* d_max = d_min + Sm;
+    double* c_try = d_max + Sm;      // [Sm] try rate of each candidate
+    double* col = c_try + Sm;        // [N]
+    int32_t* i_st = reinterpret_cast<int32_t*>(col + N);
+    int32_t* i_off = i_st + Sm;
+    int32_t* i_rem = i_off + Sm;
+    int32_t* i_arr = i_rem + Sm;
+    int32_t* c_row = i_arr + Sm;     // [Sm] EVSE of each candidate
+    int32_t* c_pos = c_row + Sm;     // [Sm] its position in the sorted table
+    int32_t* c_adm = c_pos + Sm;     // [Sm] admitted flag
+    const size_t base = (size_t)b * Sm;
+    int32_t* station = const_cast<int32_t*>(X.station) + base;
+    int32_t* aoff = const_cast<int32_t*>(X.arrival_offset) + base;
+    int32_t* rem_t = const_cast<int32_t*>(X.remaining_time) + base;
+    int32_t* arr = const_cast<int32_t*>(X.arrival) + base;
+    double* dem = const_cast<double*>(X.remaining_demand) + base;
+    double* mn = const_cast<double*>(X.min_rate) + base;
+    double* mx = const_cast<double*>(X.max_rate) + base;
+    double* mn0 = const_cast<double*>(X.min_rate0) + base;
+    double* mx0 = const_cast<double*>(X.max_rate0) + base;
+    for (int s = lane; s < Sm; s += 32) {
+        i_st[s] = station[s]; i_off[s] = aoff[s]; i_rem[s] = rem_t[s]; i_arr[s] = arr[s];
+        d_dem[s] = dem[s]; d_min[s] = mn[s]; d_max[s] = mx[s];
+    }
+    __syncwarp();
+    // stable sort by (arrival, slot), empty slots (station outside [0, N)) last in slot order: a rank sort
+    for (int s = lane; s < Sm; s += 32) {
+        const bool ok = i_st[s] >= 0 && i_st[s] < N;
+        const int a = i_arr[s];
+        int r = 0;
+        for (int j = 0; j < Sm; ++j) {
+            const bool oj = i_st[j] >= 0 && i_st[j] < N;
+            r += ok ? (oj && (i_arr[j] < a || (i_arr[j] == a && j < s))) : (oj || j < s);
+        }
+        station[r] = i_st[s]; aoff[r] = i_off[s]; rem_t[r] = i_rem[s]; arr[r] = a;
+        dem[r] = d_dem[s]; mn[r] = d_min[s]; mx[r] = d_max[s];
+        mn0[r] = d_min[s]; mx0[r] = d_max[s];  // empty slots and sessions left out of the greedy keep their own limits
+    }
+    __syncwarp();
+    // candidates in sorted order (lane 0: S_max is small next to the greedy, which costs one network check per candidate)
+    int nC = 0;
+    if (lane == 0) {
+        const double per_period = __ddiv_rn(60.0, period);
+        for (int s = 0; s < Sm; ++s) {
+            const int i = station[s];
+            if (i < 0 || i >= N) break;
+            const double mp = min_pilot[i];
+            const double tr = (override < mp) ? override : mp;  // Python's min(min_pilot, override)
+            if (skip) {  // interface.remaining_amp_periods, in the order acb_quantize_pilots computes it
+                const double ramp = __dmul_rn(__ddiv_rn(__dmul_rn(dem[s], 1000.0), S.volt[i]), per_period);
+                if (ramp < tr) continue;
+            }
+            c_row[nC] = i; c_try[nC] = tr; c_pos[nC] = s;
+            ++nC;
+        }
+    }
+    nC = __shfl_sync(0xffffffffu, nC, 0);
+    __syncwarp();
+    min_rate_greedy(S, col, nC, c_row, c_try, c_adm, lane);
+    for (int c = lane; c < nC; c += 32) {
+        const int s = c_pos[c];
+        if (c_adm[c]) {
+            const double lo = (mn[s] < c_try[c]) ? c_try[c] : mn[s];  // max(try, min_rates[0])
+            mn0[s] = lo;
+            mx0[s] = (mx[s] < lo) ? lo : mx[s];  // reconcile: max_rates[0] = max(max_rates[0], min_rates[0])
+        } else {
+            mn0[s] = 0.0;
+            mx0[s] = 0.0;
+        }
     }
 }
 
@@ -493,6 +582,23 @@ extern "C" int acb_min_rate_admission(acb_site* site, int B, int S_max, const in
     }
     ACB_CUDA(cudaSetDevice(site->device));
     k_min_rate_admission<<<B, 32, site->d.N * sizeof(double), (cudaStream_t)stream>>>(site->d, B, S_max, n_sessions, sess_row, try_rate, admitted);
+    ACB_CUDA(cudaGetLastError());
+    return ACB_OK;
+}
+
+extern "C" int acb_admit_sessions(acb_site* site, const acb_sessions* sessions, const double* min_pilot, double override, double period,
+                                  int32_t skip_unabsorbable, void* stream) {
+    if (!site || !sessions || !min_pilot || sessions->B <= 0 || sessions->S_max <= 0 || !sessions->station || !sessions->arrival_offset ||
+        !sessions->remaining_time || !sessions->remaining_demand || !sessions->min_rate || !sessions->max_rate || !sessions->arrival ||
+        !sessions->min_rate0 || !sessions->max_rate0 || (skip_unabsorbable && !(period > 0))) {
+        acb_set_error("acb_admit_sessions: bad arguments (the session tables need arrival, min_rate0 and max_rate0; skip_unabsorbable needs period > 0)");
+        return ACB_E_INVALID;
+    }
+    const size_t smem = admit_smem_bytes(site->d.N, sessions->S_max);
+    if (smem > ACB_MAX_SMEM) { acb_set_error("acb_admit_sessions: site and S_max need more shared memory than a block has"); return ACB_E_TOO_LARGE; }
+    ACB_CUDA(cudaSetDevice(site->device));
+    if (smem > 48 * 1024) ACB_CUDA(cudaFuncSetAttribute(k_admit_sessions, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k_admit_sessions<<<sessions->B, 32, smem, (cudaStream_t)stream>>>(site->d, *sessions, min_pilot, override, period, skip_unabsorbable);
     ACB_CUDA(cudaGetLastError());
     return ACB_OK;
 }

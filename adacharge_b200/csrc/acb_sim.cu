@@ -22,6 +22,7 @@ __global__ void acb_fleet_sessions_kernel(acb_fleet F, int t, acb_sessions X, in
     double* dem = const_cast<double*>(X.remaining_demand) + base;
     double* mn = const_cast<double*>(X.min_rate) + base;
     double* mx = const_cast<double*>(X.max_rate) + base;
+    int32_t* ev_arr = X.arrival ? const_cast<int32_t*>(X.arrival) + base : nullptr;  // (uninterrupted charging)
     const bool had = F.had[b] != 0;
     int n = 0;
     for (int e0 = lo; e0 < hi; e0 += 32) {
@@ -41,6 +42,7 @@ __global__ void acb_fleet_sessions_kernel(acb_fleet F, int t, acb_sessions X, in
             dem[j] = owed;
             mn[j] = 0.0;
             mx[j] = F.ev_max[e];
+            if (ev_arr) ev_arr[j] = F.ev_arr[e];
             sess_ev[base + j] = e;
             warm_mu[base + j] = had ? F.ev_mu[e] : 0.f;
         }
@@ -49,6 +51,7 @@ __global__ void acb_fleet_sessions_kernel(acb_fleet F, int t, acb_sessions X, in
     n = min(n, X.S_max);
     for (int j = n + lane; j < X.S_max; j += 32) {
         station[j] = -1; arr[j] = 0; rem_t[j] = 0; dem[j] = 0.0; mn[j] = 0.0; mx[j] = 0.0;
+        if (ev_arr) ev_arr[j] = 0;
         sess_ev[base + j] = -1;
         warm_mu[base + j] = 0.f;
     }

@@ -22,7 +22,8 @@ __global__ void acb_bounds_kernel(SiteDev S, acb_batch B, float* lb, float* ub) 
         int row = B.sess_row[k], a = B.sess_start[k], len = B.sess_len[k], off = B.sess_rate_off[k];
         for (int j = lane; j < len; j += 32) {
             const int ri = off >= 0 ? off + j : -(off + 1);  // off < 0: one (min, max) pair for the whole session
-            float lo = B.min_rates[ri], hi = B.max_rates[ri];
+            const bool f0 = j == 0 && B.sess_min0;  // first-period limits (uninterrupted charging)
+            float lo = f0 ? B.sess_min0[k] : B.min_rates[ri], hi = f0 ? B.sess_max0[k] : B.max_rates[ri];
             if (a + j < Tp) { lbb[row * Tp + a + j] = lo; ubb[row * Tp + a + j] = fmaxf(hi, lo); }
         }
     }

@@ -312,6 +312,13 @@ __global__ void __launch_bounds__(Q > 0 ? 128 : 256, Q > 0 ? 5 : 1) k_rows(SiteD
                 const bool in = (unsigned)(lane + 32 * q - s_a) < (unsigned)s_len;
                 rs.LB(q) = in ? s_lo : 0.f; rs.UB(q) = in ? s_hi : 0.f;
             }
+            if (B.sess_min0 && s_len > 0) {  // first-period limits (uninterrupted charging): the second pair, column s_a only
+                const size_t k0 = (size_t)b * B.S_max + sf;
+                const float lo0 = B.sess_min0[k0], hi0 = fmaxf(B.sess_max0[k0], lo0);
+#pragma unroll
+                for (int q = 0; q < nq; ++q)
+                    if (lane + 32 * q == s_a) { rs.LB(q) = lo0; rs.UB(q) = hi0; }
+            }
         } else {
 #pragma unroll
             for (int q = 0; q < nq; ++q) { rs.LB(q) = 0.f; rs.UB(q) = 0.f; }
@@ -322,8 +329,10 @@ __global__ void __launch_bounds__(Q > 0 ? 128 : 256, Q > 0 ? 5 : 1) k_rows(SiteD
                     const int j = lane + 32 * q - a;
                     if (j >= 0 && j < len) {
                         const int ri = off >= 0 ? off + j : -(off + 1);
-                        const float lo = B.min_rates[ri];
-                        rs.LB(q) = lo; rs.UB(q) = fmaxf(B.max_rates[ri], lo);
+                        const bool f0 = j == 0 && B.sess_min0;  // first-period limits (uninterrupted charging)
+                        const size_t k0 = (size_t)b * B.S_max + s;
+                        const float lo = f0 ? B.sess_min0[k0] : B.min_rates[ri];
+                        rs.LB(q) = lo; rs.UB(q) = fmaxf(f0 ? B.sess_max0[k0] : B.max_rates[ri], lo);
                     }
                 }
             }

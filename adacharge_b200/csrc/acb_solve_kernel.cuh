@@ -276,7 +276,8 @@ __global__ void __launch_bounds__(TPW == 2 ? 1024 : (FAST ? ACB_FAST_THREADS : 7
         int row = B.sess_row[k], a = SESS_A[s], len = SESS_B[s] - a, off = B.sess_rate_off[k];
         for (int j = lane; j < len; j += 32) {
             const int ri = off >= 0 ? off + j : -(off + 1);  // off < 0: one (min, max) pair for the whole session
-            float lo = B.min_rates[ri], hi = B.max_rates[ri];
+            const bool f0 = j == 0 && B.sess_min0;  // first-period limits (uninterrupted charging)
+            float lo = f0 ? B.sess_min0[k] : B.min_rates[ri], hi = f0 ? B.sess_max0[k] : B.max_rates[ri];
             if (a + j < Tp) {
                 if constexpr (FAST) { if (lo != 0.f) SCAL[SC_LBPOS] = 1.f; }  // the caller's lb_zero promise is broken: flagged below
                 else LB[row * Tp + a + j] = lo;

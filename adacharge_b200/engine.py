@@ -254,7 +254,7 @@ class DeviceBatch:
     ``C.byref(self.struct)``.
 
     `packed` holds the input tensors by acb_batch field name (`T`, `n_sessions`, `sess_*`, `min_rates`, `max_rates`,
-    `alpha`, `beta`, `qd`, `gamma`, `peak_w`, `peak_p0`; `ext`, `peak_limit`, `sess_quad` optional).  `pilots`
+    `alpha`, `beta`, `qd`, `gamma`, `peak_w`, `peak_p0`; `ext`, `peak_limit`, `sess_quad`, `sess_min0` / `sess_max0` optional).  `pilots`
     allocates the float64 [B, N, Tp] pilots the solve's epilogue writes; `rate_est` the rate polish's estimate."""
 
     def __init__(self, site: Site, packed: Dict[str, torch.Tensor], Tp: int, S_max: int, multi_session=False, lb_zero=False,

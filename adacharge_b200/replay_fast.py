@@ -40,12 +40,17 @@ class FleetStats:
 class FleetReplay:
     """`n_sites` copies of one site, `days` seeded days of EVs each (day d of site s is
     `synthetic_day(seed0 + s * days + d)` shifted by d * steps_per_day periods).  `quantize` / `reallocate` are
-    AdaptiveSchedulingAlgorithm's flags: the EVs are charged with pilots from each EVSE's allowable set."""
+    AdaptiveSchedulingAlgorithm's flags: the EVs are charged with pilots from each EVSE's allowable set.
+    `uninterrupted_charging` is its flag too (acnportal's apply_minimum_charging_rate with override = period): each step
+    the EVs of a site are offered min(min_pilot, period) as their first-period minimum in arrival order while the network
+    stays feasible.  An EV whose remaining energy is less than one period at that rate is not offered it (the
+    reference would make the whole site's problem infeasible until that EV leaves)."""
 
     def __init__(self, infra: Dict, objective: List[ObjectiveComponent], n_sites: int, steps_per_day: int = 288, days: int = 1,
                  period: float = 5, prices: Optional[np.ndarray] = None, demand_charge: float = 15.51, seed0: int = 0,
                  warm_start: bool = True, solver_options: Optional[dict] = None, device=None, mean_sessions: int = 40,
-                 Tp: int = 288, site_offset: int = 0, quantize: bool = False, reallocate: bool = False):
+                 Tp: int = 288, site_offset: int = 0, quantize: bool = False, reallocate: bool = False,
+                 uninterrupted_charging: bool = False):
         self.infra, self.objective, self.n_sites, self.period = infra, objective, n_sites, period
         self.steps_per_day, self.days, self.steps = steps_per_day, days, steps_per_day * days
         self.warm_start, self.device, self.Tp = warm_start, device, Tp
@@ -63,6 +68,10 @@ class FleetReplay:
         from .batched import pilot_mode
 
         self.pilot_mode = pilot_mode(quantize, reallocate, self.info)
+        self.uninterrupted_charging = bool(uninterrupted_charging)
+        self.try_rate = np.array([min(self.info.min_pilot[i], period) for i in range(self.N)], dtype=np.float64)
+        # an admitted EV's first-period minimum is its EVSE's try rate: the lb_zero promise holds only if every try is 0
+        self.lb_zero = not (self.uninterrupted_charging and bool(np.any(self.try_rate > 0)))
         cols = {k: [] for k in ("site", "station", "arr", "dep", "req", "maxrate")}
         for s in range(n_sites):
             for d in range(days):
@@ -175,6 +184,36 @@ class FleetReplay:
         h.update(self._objective_arrays(t, T))
         return h, idx, s, pos, n_sess
 
+    def _admit(self, h, idx, s, pos):
+        """apply_minimum_charging_rate of every site (what acb_admit_sessions does on the device): the greedy over the
+        sessions in (arrival, slot) order, minus those that cannot absorb one period at their try rate, and the
+        resulting first-period limits in the packed tables (sess_min0 / sess_max0)."""
+        B, S_ = self.n_sites, self.N
+        order = np.lexsort((pos, self.ev_arr[idx], s))  # by site, then arrival, then slot
+        st, rem, flat = self.ev_station[idx], self.ev_req[idx] - self.ev_dlv[idx], s * S_ + pos
+        tr = self.try_rate[st]
+        ramp = rem * 1000 / self.volt[st] * (60 / self.period)  # interface.remaining_amp_periods
+        cand = order[ramp[order] >= tr[order]]
+        n_c = np.bincount(s[cand], minlength=B)
+        c_pos = np.arange(len(cand)) - np.concatenate(([0], np.cumsum(n_c)[:-1]))[s[cand]]
+        rows, tries = np.zeros((B, S_), dtype=np.int32), np.zeros((B, S_))
+        rows[s[cand], c_pos], tries[s[cand], c_pos] = st[cand], tr[cand]
+        adm = engine.min_rate_admission(self.site, n_c, rows, tries)[s[cand], c_pos]
+        mn0, mx0 = np.zeros(len(idx)), self.ev_max[idx].copy()  # sessions left out keep their own limits (0, max rate)
+        lo = np.where(0.0 < tr[cand], tr[cand], 0.0)  # max(try, min_rates[0])
+        mn0[cand] = np.where(adm, lo, 0.0)
+        mx0[cand] = np.where(adm, np.where(mx0[cand] < lo, lo, mx0[cand]), 0.0)
+        for name, v in (("sess_min0", mn0), ("sess_max0", np.minimum(mx0, 3.0e38))):
+            a = np.zeros(B * S_, dtype=np.float32)
+            a[flat] = v
+            h[name] = a.reshape(B, S_)
+        # position of each session in its site's arrival-ordered list, as the device admission leaves the raw tables
+        # (the reallocation's tie order), and its max_rates[0]
+        n_s = np.bincount(s, minlength=B)
+        self._arr_order = np.empty_like(pos)
+        self._arr_order[order] = np.arange(len(order)) - np.concatenate(([0], np.cumsum(n_s)[:-1]))[s[order]]
+        self._max0, self._limits0 = mx0, (mn0, mx0)
+
     # ------------------------------------------------------------------ one control step
     def step(self, t: int):
         t0 = time.perf_counter()
@@ -182,12 +221,16 @@ class FleetReplay:
         if self.site is None:
             use_u = bool((h["gamma"] > 0).any() or (h["peak_w"] > 0).any())
             self.site = engine.get_site(self.info, "SOC", False, use_u, self.device)
+        self._arr_order = None
+        if self.uninterrupted_charging:
+            self._admit(h, idx, s, pos)
         if self._pb is None:
             self._pb = engine.PackedBatch.from_arrays(self.site, h, self.Tp, self.N, multi_session=False)
             self._state = [self._pb.new_warm_state(), self._pb.new_warm_state()]
         else:
             self._pb.refill(h)  # same shapes every step: reuse the pinned staging and the device buffers
         pb = self._pb
+        pb.lb_zero = pb.lb_zero and self.lb_zero
         prev, out = self._state
         dev = pb.device
         t1 = time.perf_counter()
@@ -238,9 +281,16 @@ class FleetReplay:
             B, S_ = h["sess_row"].shape
             ramp, max0 = np.zeros((B, S_)), np.zeros((B, S_))
             rem = self.ev_req[idx] - self.ev_dlv[idx]
+            rows = h["sess_row"]
+            if self._arr_order is not None:  # uninterrupted charging: arrival order and max_rates[0] from the admission
+                pos, mx = self._arr_order, self._max0
+                rows = np.zeros((B, S_), dtype=np.int32)
+                rows[s, pos] = self.ev_station[idx]
+            else:
+                mx = self.ev_max[idx]
             ramp[s, pos] = rem * 1000 / self.volt[self.ev_station[idx]] * (60 / self.period)
-            max0[s, pos] = self.ev_max[idx]
-            return engine.reallocate(self.site, 1, rates, h["n_sessions"], h["sess_row"], h["sess_start"], ramp, max0)
+            max0[s, pos] = mx
+            return engine.reallocate(self.site, 1, rates, h["n_sessions"], rows, h["sess_start"], ramp, max0)
         return engine.project_discrete(self.site, rates)
 
     def _warm(self, prev, idx_d, s_d, pos_d):
@@ -277,8 +327,13 @@ class DeviceFleetReplay(FleetReplay):
     launches on one stream -- active sessions (acb_fleet_sessions), packing (acb_pack_sessions), the warm-started solve
     whose prologue reads the previous state one column ahead (acb_batch.warm_shift) and whose epilogue projects the
     pilots, and the simulator update (acb_fleet_apply) -- with no host synchronisation between steps.  Quantised pilots
-    take a fifth launch (acb_quantize_pilots) between the solve and the update.  Same schedules,
-    bit for bit, as FleetReplay (tests/test_gpu_replay.py)."""
+    take a fifth launch (acb_quantize_pilots) between the solve and the update, uninterrupted charging one more
+    (acb_admit_sessions) between the active sessions and the packing.  Same schedules, bit for bit, as FleetReplay
+    (tests/test_gpu_replay.py, tests/test_gpu_uninterrupted.py).
+
+    The admission puts the raw tables in arrival order but leaves `sess_ev` / `warm_mu` in the EV table's (station)
+    order: they are indexed like the packed batch (warm_mu, out_mu), whose (EVSE, slot) order of a single-session site
+    is the station order whatever the slot order."""
 
     def __init__(self, *a, **kw):
         super().__init__(*a, **kw)
@@ -291,7 +346,8 @@ class DeviceFleetReplay(FleetReplay):
         self._bac = BatchedAdaptiveCharging(self.objective, self.info, self.period, batch=self.n_sites, max_sessions=self.N, horizon=self.Tp,
                                             demand_charge=self.demand_charge, solver_options=opts, device=self.device, chunks=1,
                                             enforce_pilot_limit=False, quantize=self.pilot_mode != 0,
-                                            reallocate=self.pilot_mode == _cabi.ACB_PILOTS_REALLOCATE)
+                                            reallocate=self.pilot_mode == _cabi.ACB_PILOTS_REALLOCATE,
+                                            uninterrupted_charging=self.uninterrupted_charging, skip_unabsorbable=True)
         if self._bac.Tp != self.Tp:
             raise ValueError(f"Tp = {self.Tp} is not a padded horizon of the solve path")
         self.site = self._bac.site
@@ -320,7 +376,7 @@ class DeviceFleetReplay(FleetReplay):
         f.ev_dlv, f.ev_mu, f.day_site_off, f.prev_peak, f.had = p(d["dlv"]), p(d["mu"]), p(d["off"]), p(d["prev_peak"]), p(d["had"])
         self._fleet = f
         self._state = [ch.new_warm_state(), ch.new_warm_state()]
-        ch.lb_zero = True  # the synthetic EVs have no minimum rate
+        ch.lb_zero = self.lb_zero  # the synthetic EVs have no minimum rate of their own
         o = ch.objective
         o.prev_peak = p(d["prev_peak"])
         o.prices_stride = 0  # one price vector for the whole fleet, read from the current period on
@@ -335,6 +391,8 @@ class DeviceFleetReplay(FleetReplay):
         ch.set_warm(dict(prev, mu=d["warm_mu"]) if self.warm_start and self._started else None, out, shift=1, had=d["had"])
         o.prices = C.c_void_p(d["prices"].data_ptr() + 8 * t) if self._bac.need_prices else None
         _cabi.check(L.acb_fleet_sessions(self.site.handle, C.byref(self._fleet), t, C.byref(ch.sessions), p(d["sess_ev"]), p(d["warm_mu"]), st), "acb_fleet_sessions")
+        if self.uninterrupted_charging:
+            self._bac.admit(ch, st)
         _cabi.check(L.acb_pack_sessions(self.site.handle, C.byref(ch.sessions), C.byref(o), C.byref(ch.struct), p(ch.flags), st), "acb_pack_sessions")
         ch.solve(self._bac.options, st)
         if self.pilot_mode:  # the solve skipped the continuous projection (batch.pilots NULL); acb_fleet_apply reads batch.pilots

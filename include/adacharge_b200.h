@@ -171,6 +171,10 @@ typedef struct acb_batch {
     int32_t* status;             /* [B] */
     int32_t* iters;              /* [B] */
     float* stats;                /* [B][ACB_NSTATS] */
+    /* first-period limits (uninterrupted charging, acb_admit_sessions), NULL = none: the pair replaces min_rates /
+     * max_rates of session k at its first column sess_start[k] only (the bound there is max(sess_max0, sess_min0)) */
+    const float* sess_min0;      /* [B*S_max] */
+    const float* sess_max0;      /* [B*S_max] */
 } acb_batch;
 
 int acb_solve_batch(acb_site* site, const acb_batch* batch, const acb_options* opt, void* stream);
@@ -199,6 +203,9 @@ typedef struct acb_sessions {      /* [B][S_max] tables, any order within an ins
     const double* remaining_demand; /* SessionInfo.remaining_demand, kWh */
     const double* min_rate;         /* constant per session (time-varying limits go through the host packer) */
     const double* max_rate;
+    const int32_t* arrival;         /* absolute arrival period (SessionInfo.arrival); read by acb_admit_sessions only */
+    const double* min_rate0;        /* first-period limits (written by acb_admit_sessions); NULL = min_rate / max_rate */
+    const double* max_rate0;
 } acb_sessions;
 
 typedef struct acb_objective {     /* the ObjectiveComponent list, in order: sum_c coef[c] * f_kind[c](rates) is maximised */
@@ -249,7 +256,8 @@ int acb_reallocate(acb_site* site, int mode, const double* rates_in, double* rat
  * batch->T, batch->n_sessions (an instance without sessions gets all-zero pilots) and, for ACB_PILOTS_REALLOCATE, the raw session tables (after acb_preprocess_sessions, if used); writes
  * pilots [B][N][Tp] float64, bit-identical to the reference applied to rates[:, :T] in float64 and then np.maximum(., 0).
  * Columns >= T[b] are 0.  The reallocation takes the sessions in slot order (empty slots, station < 0, skipped) and their
- * ramp as interface.remaining_amp_periods: remaining_demand * 1000 / voltage * (60 / period).  The site needs
+ * ramp as interface.remaining_amp_periods: remaining_demand * 1000 / voltage * (60 / period), and max_rates[0] from
+ * sessions->max_rate0 when given (acb_admit_sessions), else max_rate.  The site needs
  * allowable_pilots; sessions->B must equal batch->B. */
 #define ACB_PILOTS_DISCRETE 1   /* project_into_discrete_feasible_pilots   postprocessing.py:97-118 */
 #define ACB_PILOTS_REALLOCATE 2 /* diff_based_reallocation                 postprocessing.py:189-258 */
@@ -273,6 +281,20 @@ int acb_min_rate_admission(acb_site* site, int B, int S_max, const int32_t* n_se
  * it fell below the minimum rate. */
 int acb_preprocess_sessions(acb_site* site, const acb_sessions* sessions, int enforce_pilot_limit, const double* upper_bound, void* stream);
 
+/* Uninterrupted charging (reference adacharge/adacharge.py:149-150 -> acnportal's apply_minimum_charging_rate with
+ * override), batched, in place, one block per instance:
+ *  1. the raw tables (station, arrival_offset, remaining_time, remaining_demand, min_rate, max_rate, arrival) are
+ *     permuted into the stable (arrival, slot) order, empty slots last: the order of the reference's sorted(sessions,
+ *     key=arrival), which every later step (the packer's (EVSE, slot) sort, acb_quantize_pilots' tie order) then sees;
+ *  2. the sessions are offered try = min(min_pilot[EVSE], override) in that order (acb_min_rate_admission's greedy);
+ *  3. min_rate0 / max_rate0 receive the first-period limits: admitted max(try, min_rate) and max(max_rate, that);
+ *     refused 0 and 0.
+ * skip_unabsorbable = 1 (closed-loop replays): a session whose remaining_amp_periods (remaining_demand * 1000 / voltage
+ * * (60 / period)) is below its try rate is not offered the minimum and keeps min_rate / max_rate (the reference would
+ * declare the instance infeasible).  min_pilot: [N] device.  sessions needs arrival, min_rate0 and max_rate0. */
+int acb_admit_sessions(acb_site* site, const acb_sessions* sessions, const double* min_pilot, double override, double period,
+                       int32_t skip_unabsorbable, void* stream);
+
 /* ---- closed-loop replay on the device (the simulator side of a control step for a fleet of sites) ----
  * The loop acnportal's Simulator drives around AdaptiveSchedulingAlgorithm.schedule (adacharge/adacharge.py:18-39 active
  * sessions in, :135-193 pilots out; tests/test_integration.py:115-118), as two kernels around acb_pack_sessions +
@@ -293,8 +315,10 @@ typedef struct acb_fleet {
 } acb_fleet;
 
 /* Step t: the active sessions of every site (plugged in, energy still owed) into the raw tables acb_pack_sessions takes
- * (arrival_offset 0, remaining_time = departure - t, remaining_demand = requested - delivered), plus the EV behind each
- * slot (sess_ev [n_sites][S_max], -1 = empty) and its warm-start multiplier (warm_mu [n_sites][S_max]). */
+ * (arrival_offset 0, remaining_time = departure - t, remaining_demand = requested - delivered, arrival = ev_arr if
+ * sessions->arrival is given), plus the EV behind each slot (sess_ev [n_sites][S_max], -1 = empty) and its warm-start
+ * multiplier (warm_mu [n_sites][S_max]).  Slots are in station order; sess_ev and warm_mu keep that order after
+ * acb_admit_sessions, which is the packed order of a single-session site. */
 int acb_fleet_sessions(acb_site* site, const acb_fleet* fleet, int t, const acb_sessions* sessions, int32_t* sess_ev, float* warm_mu,
                        void* stream);
 /* After the solve of step t: the first-period pilots (batch->pilots) charge every plugged-in EV (delivered energy capped at
