@@ -17,8 +17,8 @@ ACB_NSTATS = 8
 ACB_PILOTS_DISCRETE, ACB_PILOTS_REALLOCATE = 1, 2  # acb_quantize_pilots modes
 EXPORTS = [
     "acb_site_create", "acb_site_destroy", "acb_site_dims", "acb_site_max_horizon", "acb_default_options",
-    "acb_solve_batch", "acb_charging_rate_bounds", "acb_project_continuous", "acb_project_discrete",
-    "acb_reallocate", "acb_quantize_pilots", "acb_constraints_feasible", "acb_min_rate_admission", "acb_admit_sessions", "acb_pack_sessions", "acb_preprocess_sessions", "acb_fleet_sessions", "acb_fleet_apply", "acb_last_error", "acb_version",
+    "acb_solve_batch", "acb_solve_batch_masked", "acb_charging_rate_bounds", "acb_project_continuous", "acb_project_discrete",
+    "acb_reallocate", "acb_quantize_pilots", "acb_quantize_pilots_masked", "acb_constraints_feasible", "acb_min_rate_admission", "acb_admit_sessions", "acb_pack_sessions", "acb_preprocess_sessions", "acb_fleet_sessions", "acb_fleet_apply", "acb_last_error", "acb_version",
 ]
 ACB_MAX_COMPONENTS = 16
 # acb_objective.kind values (include/adacharge_b200.h)
@@ -71,7 +71,8 @@ class Objective(C.Structure):
 
 class Fleet(C.Structure):
     _fields_ = [("n_sites", C.c_int32), ("n_ev", C.c_int32), ("days", C.c_int32), ("steps_per_day", C.c_int32), ("ev_station", _P), ("ev_arr", _P),
-                ("ev_dep", _P), ("ev_req", _P), ("ev_max", _P), ("ev_dlv", _P), ("ev_mu", _P), ("day_site_off", _P), ("prev_peak", _P), ("had", _P)]
+                ("ev_dep", _P), ("ev_req", _P), ("ev_max", _P), ("ev_dlv", _P), ("ev_mu", _P), ("day_site_off", _P), ("prev_peak", _P), ("had", _P),
+                ("max_recompute", C.c_int32), ("last_solve", _P), ("recompute", _P), ("shift", _P)]
 
 
 _lib = None
@@ -96,11 +97,13 @@ def lib():
     L.acb_default_options.argtypes = [C.POINTER(Options)]
     L.acb_default_options.restype = None
     L.acb_solve_batch.argtypes = [_P, C.POINTER(Batch), C.POINTER(Options), _P]
+    L.acb_solve_batch_masked.argtypes = [_P, C.POINTER(Batch), _P, _P, C.POINTER(Options), _P]
     L.acb_charging_rate_bounds.argtypes = [_P, C.POINTER(Batch), _P, _P, _P]
     L.acb_project_continuous.argtypes = [_P, _P, _P, C.c_int, C.c_int, _P]
     L.acb_project_discrete.argtypes = [_P, _P, _P, C.c_int, C.c_int, _P]
     L.acb_reallocate.argtypes = [_P, C.c_int, _P, _P, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P]
     L.acb_quantize_pilots.argtypes = [_P, C.c_int, C.POINTER(Sessions), C.c_double, C.POINTER(Batch), _P, _P]
+    L.acb_quantize_pilots_masked.argtypes = [_P, C.c_int, C.POINTER(Sessions), C.c_double, C.POINTER(Batch), _P, _P, _P]
     L.acb_constraints_feasible.argtypes = [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P]
     L.acb_min_rate_admission.argtypes = [_P, C.c_int, C.c_int, _P, _P, _P, _P, _P]
     L.acb_admit_sessions.argtypes = [_P, C.POINTER(Sessions), _P, C.c_double, C.c_double, C.c_int32, _P]

@@ -26,6 +26,16 @@ def get_active_sessions(active_evs, current_time):
     ]
 
 
+def quantized_max_recompute(max_recompute, quantize, default=None):
+    """The re-solve period that goes with `quantize` (ada.py:106-113): quantised pilots are recomputed every period, so
+    with `quantize` it is 1, with the reference's warning when the caller asked for anything but `default`."""
+    if not quantize:
+        return max_recompute
+    if max_recompute != default:
+        warnings.warn("Overriding max_recompute to 1 since quantization is on.")
+    return 1
+
+
 class AdaptiveSchedulingAlgorithm(BaseAlgorithm):
     """MPC based adaptive scheduling algorithm (ada.py:42-193); same kwargs.
     ``solver`` is accepted and ignored; ``solver_options`` goes to the device solver."""
@@ -48,12 +58,7 @@ class AdaptiveSchedulingAlgorithm(BaseAlgorithm):
         self.solver_options = solver_options
         if not self.quantize and self.reallocate:  # ada.py:101-105
             raise ValueError("reallocate cannot be true without quantize. Otherwise there is nothing to reallocate :).")
-        if self.quantize:  # ada.py:106-113
-            if max_recompute is not None:
-                warnings.warn("Overriding max_recompute to 1 since quantization is on.")
-            self.max_recompute = 1
-        else:
-            self.max_recompute = max_recompute
+        self.max_recompute = quantized_max_recompute(max_recompute, self.quantize)
         self.allow_overcharging = allow_overcharging
 
     def register_interface(self, interface):

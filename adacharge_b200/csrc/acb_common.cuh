@@ -97,5 +97,20 @@ inline void acb_keep_pool(int device) {
         cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep);
     }
 }
+// event-driven recompute (acb_solve_batch_masked's solve_mask / warm_shifts, NULL = none)
+__device__ __forceinline__ bool acb_masked_out(const int32_t* mask, int b) { return mask && mask[b] == 0; }
+__device__ __forceinline__ int acb_warm_shift(const acb_batch& B, const int32_t* shifts, int b) { return shifts ? shifts[b] : B.warm_shift; }
+// a skipped instance's state for the next step: out_* <- warm_* unshifted (one block, any number of threads)
+__device__ inline void acb_keep_warm(const acb_batch& B, int b, int N, int R, int Tp) {
+    const int tid = threadIdx.x, nt = blockDim.x;
+    if (B.warm_v1 && B.out_v1)
+        for (size_t i = tid, n = (size_t)N * Tp; i < n; i += nt) B.out_v1[(size_t)b * n + i] = B.warm_v1[(size_t)b * n + i];
+    if (B.warm_vc && B.out_vc)
+        for (size_t i = tid, n = (size_t)R * Tp; i < n; i += nt) B.out_vc[(size_t)b * n + i] = B.warm_vc[(size_t)b * n + i];
+    if (B.warm_mu && B.out_mu)
+        for (int i = tid; i < B.S_max; i += nt) B.out_mu[(size_t)b * B.S_max + i] = B.warm_mu[(size_t)b * B.S_max + i];
+    if (B.warm_scal && B.out_scal && tid < 2) B.out_scal[b * 2 + tid] = B.warm_scal[b * 2 + tid];
+}
 size_t acb_solve_smem_bytes(const SiteDev& s, int Tp, int S_max, int nwarps);
-int acb_solve_general(acb_site* site, const acb_batch* batch, const acb_options& opt, cudaStream_t st);
+int acb_solve_general(acb_site* site, const acb_batch* batch, const int32_t* solve_mask, const int32_t* warm_shifts, const acb_options& opt,
+                      cudaStream_t st);

@@ -305,8 +305,10 @@ __global__ void k_reallocate(SiteDev S, int mode, const double* rates_in, double
 // column, while the other warps project the rest.
 #define ACB_QP_THREADS 256
 __global__ void __launch_bounds__(ACB_QP_THREADS) k_quantize_pilots(SiteDev S, int mode, acb_sessions X, double period, const float* rates,
-                                                                    const int32_t* Tv, const int32_t* n_sessions, int Tp, double* pilots) {
+                                                                    const int32_t* Tv, const int32_t* n_sessions, int Tp, const int32_t* mask,
+                                                                    double* pilots) {
     extern __shared__ __align__(16) unsigned char smraw[];
+    if (mask && mask[blockIdx.x] == 0) return;  // not solved this step: keeps its pilots
     const int b = blockIdx.x, tid = threadIdx.x, N = S.N, T = (n_sessions[b] > 0) ? Tv[b] : 0;
     const float* Rb = rates + (size_t)b * N * Tp;
     double* Pb = pilots + (size_t)b * N * Tp;
@@ -545,6 +547,11 @@ extern "C" int acb_reallocate(acb_site* site, int mode, const double* rates_in, 
 
 extern "C" int acb_quantize_pilots(acb_site* site, int mode, const acb_sessions* sessions, double period, const acb_batch* batch,
                                    double* pilots, void* stream) {
+    return acb_quantize_pilots_masked(site, mode, sessions, period, batch, nullptr, pilots, stream);
+}
+
+extern "C" int acb_quantize_pilots_masked(acb_site* site, int mode, const acb_sessions* sessions, double period, const acb_batch* batch,
+                                          const int32_t* solve_mask, double* pilots, void* stream) {
     if (!site || !sessions || !batch || !pilots || !batch->rates || !batch->T || !batch->n_sessions || batch->B <= 0 || batch->Tp <= 0 ||
         (mode != ACB_PILOTS_DISCRETE && mode != ACB_PILOTS_REALLOCATE) || sessions->B != batch->B) {
         acb_set_error("acb_quantize_pilots: bad arguments");
@@ -561,7 +568,7 @@ extern "C" int acb_quantize_pilots(acb_site* site, int mode, const acb_sessions*
     ACB_CUDA(cudaSetDevice(site->device));
     if (smem > 48 * 1024) ACB_CUDA(cudaFuncSetAttribute(k_quantize_pilots, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     k_quantize_pilots<<<batch->B, ACB_QP_THREADS, smem, (cudaStream_t)stream>>>(site->d, mode, *sessions, period, batch->rates, batch->T,
-                                                                                batch->n_sessions, batch->Tp, pilots);
+                                                                                batch->n_sessions, batch->Tp, solve_mask, pilots);
     ACB_CUDA(cudaGetLastError());
     return ACB_OK;
 }

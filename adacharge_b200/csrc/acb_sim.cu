@@ -9,6 +9,10 @@
 //                        slot and its warm-start multiplier)
 //   acb_fleet_apply      first-period pilots -> energy delivered, previous peak, per-EV multipliers, step statistics
 // The EV table is sorted by (day, site, station), so a site's active sessions come out ordered by EVSE row.
+// With acb_fleet.last_solve the step is event-driven, as acnportal's Simulator loop is (this library's reading of it:
+// DESIGN.md §8): acb_fleet_sessions decides which sites re-solve (a plug-in or unplug there, max_recompute steps since the
+// last solve, or no solve yet) and that decision is acb_solve_batch_masked's solve_mask; every other site keeps its last schedule and
+// acb_fleet_apply charges its EVs with the schedule's next column.
 #include "acb_common.cuh"
 
 __global__ void acb_fleet_sessions_kernel(acb_fleet F, int t, acb_sessions X, int32_t* sess_ev, float* warm_mu) {
@@ -25,13 +29,16 @@ __global__ void acb_fleet_sessions_kernel(acb_fleet F, int t, acb_sessions X, in
     int32_t* ev_arr = X.arrival ? const_cast<int32_t*>(X.arrival) + base : nullptr;  // (uninterrupted charging)
     const bool had = F.had[b] != 0;
     int n = 0;
+    bool event = false;  // an EV plugs in or unplugs at this site now
     for (int e0 = lo; e0 < hi; e0 += 32) {
         const int e = e0 + lane;
         bool act = false;
         double owed = 0.0;
         if (e < hi) {
             owed = F.ev_req[e] - F.ev_dlv[e];
-            act = F.ev_arr[e] <= t && t < F.ev_dep[e] && owed > 1e-6;  // plugged in and energy still owed
+            const int a = F.ev_arr[e], d = F.ev_dep[e];
+            act = a <= t && t < d && owed > 1e-6;  // plugged in and energy still owed
+            event |= a == t || d == t;
         }
         const unsigned m = __ballot_sync(0xffffffffu, act);
         const int j = n + __popc(m & ((1u << lane) - 1u));
@@ -55,6 +62,20 @@ __global__ void acb_fleet_sessions_kernel(acb_fleet F, int t, acb_sessions X, in
         sess_ev[base + j] = -1;
         warm_mu[base + j] = 0.f;
     }
+    if (F.last_solve) {
+        // the unplug of a previous-day EV at a day boundary (t = d * steps_per_day) is in day d - 1's slice
+        const int d = t / F.steps_per_day;
+        if (t % F.steps_per_day == 0 && d >= 1 && d <= F.days) {
+            const int lo1 = F.day_site_off[(size_t)(d - 1) * F.n_sites + b], hi1 = F.day_site_off[(size_t)(d - 1) * F.n_sites + b + 1];
+            for (int e = lo1 + lane; e < hi1; e += 32) event |= F.ev_dep[e] == t;
+        }
+        event = __any_sync(0xffffffffu, event);
+        if (lane == 0) {
+            const int last = F.last_solve[b];
+            F.recompute[b] = (last < 0 || event || (F.max_recompute > 0 && t - last >= F.max_recompute)) ? 1 : 0;
+            F.shift[b] = t - last;
+        }
+    }
 }
 
 __global__ void acb_fleet_apply_kernel(SiteDev S, acb_fleet F, int t, double period, const double* pilots, int Tp, const int32_t* n_sessions,
@@ -64,46 +85,59 @@ __global__ void acb_fleet_apply_kernel(SiteDev S, acb_fleet F, int t, double per
     const int N = S.N;
     const int day = min(t / F.steps_per_day, F.days - 1);
     const int lo = F.day_site_off[(size_t)day * F.n_sites + b], hi = F.day_site_off[(size_t)day * F.n_sites + b + 1];
-    const double* p0 = pilots + (size_t)b * N * Tp;  // pilots[b][i][0] = p0[i * Tp]
-    // the simulator side: the first-period pilots charge every EV that is plugged in (also those that owe nothing)
+    // a site that solved now applies column 0 of its schedule, any other site column c = t - last_solve of the schedule its
+    // last solve left in `pilots`.  Columns from that solve's horizon to Tp hold 0 (the rate bounds are 0 outside every
+    // session window); c >= Tp (a site idle overnight without max_recompute) is 0 and never loaded.  (The horizon is not
+    // batch->T: the packer rewrites T and the session tables of every site at every step.)
+    const bool solved = !F.last_solve || F.recompute[b] != 0;
+    const int c = solved ? 0 : t - F.last_solve[b];
+    const bool live = c < Tp;
+    const double* p0 = pilots + (size_t)b * N * Tp + (live ? c : 0);  // pilots[b][i][c] = p0[i * Tp]
+    auto pil = [&](int i) -> double { return live ? p0[(size_t)i * Tp] : 0.0; };
+    // the simulator side: the applied pilots charge every EV that is plugged in (also those that owe nothing)
     for (int e = lo + lane; e < hi; e += 32) {
         if (F.ev_arr[e] <= t && t < F.ev_dep[e]) {
             const int i = F.ev_station[e];
             const double w = S.volt[i] * period / 1e3 / 60;  // kWh per A*period
             const double owed = F.ev_req[e] - F.ev_dlv[e];
-            double de = p0[(size_t)i * Tp] * w;
+            double de = pil(i) * w;
             de = (owed < de) ? owed : de;
             F.ev_dlv[e] += (de > 0.0) ? de : 0.0;
         }
     }
-    const int n = n_sessions[b];
-    for (int j = lane; j < n; j += 32) {
-        const int e = sess_ev[(size_t)b * S_max + j];
-        if (e >= 0) F.ev_mu[e] = out_mu[(size_t)b * S_max + j];
-    }
+    const int n = n_sessions[b];  // (this step's sessions: those of the solve when the site solved)
+    if (solved)
+        for (int j = lane; j < n; j += 32) {
+            const int e = sess_ev[(size_t)b * S_max + j];
+            if (e >= 0) F.ev_mu[e] = out_mu[(size_t)b * S_max + j];
+        }
     if (first_out)
-        for (int i = lane; i < N; i += 32) first_out[(size_t)b * N + i] = p0[(size_t)i * Tp];
+        for (int i = lane; i < N; i += 32) first_out[(size_t)b * N + i] = pil(i);
+    __syncwarp();  // every lane has read last_solve[b]
     if (lane == 0) {
-        // aggregate first-period current, summed in numpy's pairwise order (the host replay takes first.sum(axis=1))
+        // aggregate applied current, summed in numpy's pairwise order (the host replay takes first.sum(axis=1))
         double tot;
         if (N < 8) {
             tot = 0.0;
-            for (int i = 0; i < N; ++i) tot = __dadd_rn(tot, p0[(size_t)i * Tp]);
+            for (int i = 0; i < N; ++i) tot = __dadd_rn(tot, pil(i));
         } else {
             double r[8];
-            for (int j = 0; j < 8; ++j) r[j] = p0[(size_t)j * Tp];
+            for (int j = 0; j < 8; ++j) r[j] = pil(j);
             int i;
             for (i = 8; i < N - (N % 8); i += 8)
-                for (int j = 0; j < 8; ++j) r[j] = __dadd_rn(r[j], p0[(size_t)(i + j) * Tp]);
+                for (int j = 0; j < 8; ++j) r[j] = __dadd_rn(r[j], pil(i + j));
             tot = __dadd_rn(__dadd_rn(__dadd_rn(r[0], r[1]), __dadd_rn(r[2], r[3])), __dadd_rn(__dadd_rn(r[4], r[5]), __dadd_rn(r[6], r[7])));
-            for (; i < N; ++i) tot = __dadd_rn(tot, p0[(size_t)i * Tp]);
+            for (; i < N; ++i) tot = __dadd_rn(tot, pil(i));
         }
         if (tot > F.prev_peak[b]) F.prev_peak[b] = tot;
-        F.had[b] = n > 0 ? 1 : 0;
-        if (stats && n > 0) {
-            atomicAdd(stats + 0, 1.0);                                  // site-steps solved
-            atomicAdd(stats + 1, (double)iters[b]);                     // iterations
-            if (status[b] != ACB_SOLVED) atomicAdd(stats + 2, 1.0);     // not certified
+        if (solved) {
+            F.had[b] = n > 0 ? 1 : 0;
+            if (F.last_solve) F.last_solve[b] = t;
+            if (stats && n > 0) {
+                atomicAdd(stats + 0, 1.0);                                  // site-steps solved
+                atomicAdd(stats + 1, (double)iters[b]);                     // iterations
+                if (status[b] != ACB_SOLVED) atomicAdd(stats + 2, 1.0);     // not certified
+            }
         }
     }
 }
@@ -112,6 +146,10 @@ extern "C" int acb_fleet_sessions(acb_site* site, const acb_fleet* fleet, int t,
                                   void* stream) {
     if (!site || !fleet || !sessions || !sess_ev || !warm_mu || sessions->B != fleet->n_sites || t < 0) {
         acb_set_error("acb_fleet_sessions: bad arguments (one instance per site)");
+        return ACB_E_INVALID;
+    }
+    if (fleet->last_solve && (!fleet->recompute || !fleet->shift || fleet->max_recompute < 0)) {
+        acb_set_error("acb_fleet_sessions: last_solve needs recompute, shift and max_recompute >= 0");
         return ACB_E_INVALID;
     }
     ACB_CUDA(cudaSetDevice(site->device));
@@ -124,6 +162,10 @@ extern "C" int acb_fleet_apply(acb_site* site, const acb_fleet* fleet, int t, do
                                double* first_pilots, double* stats, void* stream) {
     if (!site || !fleet || !batch || !batch->pilots || !batch->out_mu || !sess_ev || batch->B != fleet->n_sites) {
         acb_set_error("acb_fleet_apply: bad arguments (the batch needs pilots and out_mu)");
+        return ACB_E_INVALID;
+    }
+    if (fleet->last_solve && !fleet->recompute) {
+        acb_set_error("acb_fleet_apply: last_solve needs recompute");
         return ACB_E_INVALID;
     }
     ACB_CUDA(cudaSetDevice(site->device));

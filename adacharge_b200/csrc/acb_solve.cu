@@ -37,8 +37,9 @@ int acb_launch_solve_q9(const acb_site*, const acb_batch*, const acb_options*, c
 // Between the launches of a phased solve: the parked (still running) instances, ordered by the relative gap of their
 // last convergence check, largest first (a counting sort over 256 logarithmic buckets; one block).  The gap after the
 // first phase is the best available predictor of the iterations an instance still needs, so the relaunch approximates
-// longest-processing-time-first scheduling and the longest instances no longer start last.
-__global__ void acb_phase_list_kernel(const int32_t* status, const float* stats, int B, int* list, int* count) {
+// longest-processing-time-first scheduling and the longest instances no longer start last.  An instance the solve skips
+// (mask) is never listed: its status is still the previous solve's.
+__global__ void acb_phase_list_kernel(const int32_t* status, const float* stats, const int32_t* mask, int B, int* list, int* count) {
     __shared__ int hist[256], base[256];
     const int tid = threadIdx.x;
     for (int i = tid; i < 256; i += blockDim.x) hist[i] = 0;
@@ -50,7 +51,7 @@ __global__ void acb_phase_list_kernel(const int32_t* status, const float* stats,
         return 255 - key;
     };
     for (int b = tid; b < B; b += blockDim.x)
-        if (status[b] == ACB_RUNNING) atomicAdd(&hist[bucket(b)], 1);
+        if (status[b] == ACB_RUNNING && (!mask || mask[b])) atomicAdd(&hist[bucket(b)], 1);
     __syncthreads();
     if (tid == 0) {
         int acc = 0;
@@ -59,10 +60,15 @@ __global__ void acb_phase_list_kernel(const int32_t* status, const float* stats,
     }
     __syncthreads();
     for (int b = tid; b < B; b += blockDim.x)
-        if (status[b] == ACB_RUNNING) list[atomicAdd(&base[bucket(b)], 1)] = b;
+        if (status[b] == ACB_RUNNING && (!mask || mask[b])) list[atomicAdd(&base[bucket(b)], 1)] = b;
 }
 
-extern "C" int acb_solve_batch(acb_site* site, const acb_batch* batch, const acb_options* opt_in, void* stream) {
+extern "C" int acb_solve_batch(acb_site* site, const acb_batch* batch, const acb_options* opt, void* stream) {
+    return acb_solve_batch_masked(site, batch, nullptr, nullptr, opt, stream);
+}
+
+extern "C" int acb_solve_batch_masked(acb_site* site, const acb_batch* batch, const int32_t* solve_mask, const int32_t* warm_shifts,
+                                      const acb_options* opt_in, void* stream) {
     if (!site || !batch || batch->B <= 0 || batch->Tp <= 0 || batch->Tp % 32 != 0) {
         acb_set_error("acb_solve_batch: bad arguments (Tp must be a positive multiple of 32)");
         return ACB_E_INVALID;
@@ -88,7 +94,7 @@ extern "C" int acb_solve_batch(acb_site* site, const acb_batch* batch, const acb
     int nthreads = std::min(768, ((want + 127) / 128) * 128);
     size_t smem = acb_solve_smem_bytes(d, batch->Tp, batch->S_max, nthreads / 32);
     const bool fits = chipQ && d.TPW == 3 && NIN <= 2 * ACB_OHT && nthreads <= 768 && d.nRowWarps * 32 <= nthreads && smem <= 232448;
-    if (opt.path == 2 || (!fits && opt.path == 0)) return acb_solve_general(site, batch, opt, st);
+    if (opt.path == 2 || (!fits && opt.path == 0)) return acb_solve_general(site, batch, solve_mask, warm_shifts, opt, st);
     if (!fits) {
         acb_set_error("acb_solve_batch: instance does not fit the on-chip path (Tp in {64, 128, 160, 288}, N <= ~66 EVSEs, <= 32 coupling tasks, " +
                       std::to_string(smem) + " B of shared memory needed, 232448 available)");
@@ -132,6 +138,8 @@ extern "C" int acb_solve_batch(acb_site* site, const acb_batch* batch, const acb
     char* base = nullptr;
     SolvePhase ph{};
     ph.it_stop = opt.max_iter;
+    ph.solve_mask = solve_mask;
+    ph.warm_shifts = warm_shifts;
     if (wantZ || phased) {
         acb_keep_pool(site->device);
         ACB_CUDA(cudaMallocAsync((void**)&base, bytes, st));
@@ -153,7 +161,7 @@ extern "C" int acb_solve_batch(acb_site* site, const acb_batch* batch, const acb
         ph.it_stop = opt.phase_iters;
         rc = launch(ph);
         if (rc == ACB_OK) {
-            acb_phase_list_kernel<<<1, 1024, 0, st>>>(batch->status, batch->stats, B, list, count);
+            acb_phase_list_kernel<<<1, 1024, 0, st>>>(batch->status, batch->stats, solve_mask, B, list, count);
             ph.it_stop = opt.max_iter; ph.resume = 1; ph.list = list; ph.count = count;
             rc = launch(ph);
         }

@@ -61,17 +61,30 @@ struct GenWork {
     int* iters;      // [B]
 };
 
+// acb_solve_batch_masked's solve_mask / warm_shifts (NULL = none); only the kernels that read them take them
+struct GenSel {
+    const int32_t* mask;
+    const int32_t* shifts;
+};
+
 struct GenDims {
     int N, R, NG, Tp, Tt /*tiles*/, S_max, nDisc, nLin, has_pl, has_u, rPL, rU, lin_two_sided;
 };
 
 // ---------------------------------------------------------------------------- setup
-__global__ void k_setup(SiteDev S, acb_batch B, acb_options opt, GenWork W, GenDims D) {
+__global__ void k_setup(SiteDev S, acb_batch B, acb_options opt, GenWork W, GenDims D, GenSel Sel) {
     const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = blockDim.x >> 5;
     const int nS = B.n_sessions[b], Tb = B.T[b], Tp = D.Tp;
     __shared__ float red[32];
+    if (acb_masked_out(Sel.mask, b)) {
+        // not solved this step: finished from the start, so the host loop does not wait for it; no later kernel touches
+        // its outputs (k_rows setup and write modes, k_setup_agg and k_finish skip it, the others see the status)
+        acb_keep_warm(B, b, D.N, D.R, Tp);
+        if (tid == 0) { W.status[b] = ACB_SOLVED; W.iters[b] = 0; atomicAdd(W.ndone, 1); }
+        return;
+    }
     // (warm_shift / warm_had: see the on-chip kernel)
-    const int wsh = B.warm_shift;
+    const int wsh = acb_warm_shift(B, Sel.shifts, b);
     const bool hadW = !B.warm_had || B.warm_had[b] != 0;
     for (int i = tid; i < D.N; i += blockDim.x) { W.row_first[(size_t)b * D.N + i] = 0; W.row_cnt[(size_t)b * D.N + i] = 0; }
     __syncthreads();
@@ -157,8 +170,9 @@ __global__ void k_setup(SiteDev S, acb_batch B, acb_options opt, GenWork W, GenD
 
 // per instance, after k_rows<Q, 6 / 7>: the aggregate-power terms of the box maximum of the objective from the group sums
 // of the bounds (SG: upper, SGZ: lower or absent)
-__global__ void k_setup_agg(SiteDev S, acb_batch B, GenWork W, GenDims D, int have_lb) {
+__global__ void k_setup_agg(SiteDev S, acb_batch B, GenWork W, GenDims D, int have_lb, GenSel Sel) {
     const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = blockDim.x >> 5;
+    if (acb_masked_out(Sel.mask, b)) return;
     const float* sc = W.scal + (size_t)b * GS_N;
     const float gam_s = sc[GS_GAMMA], pkw_s = sc[GS_PKW];
     if (!D.has_u || !(gam_s > 0.f || pkw_s > 0.f)) return;
@@ -225,10 +239,11 @@ struct RowStore<0> {
 };
 
 template <int Q, int MODE>
-__global__ void __launch_bounds__(Q > 0 ? 128 : 256, Q > 0 ? 5 : 1) k_rows(SiteDev S, acb_batch B, acb_options opt, GenWork W, GenDims D, const int* grp_off) {
+__global__ void __launch_bounds__(Q > 0 ? 128 : 256, Q > 0 ? 5 : 1) k_rows(SiteDev S, acb_batch B, acb_options opt, GenWork W, GenDims D, const int* grp_off, GenSel Sel) {
     constexpr bool SETUP = (MODE == 6 || MODE == 7), ITER = (MODE == 0 || MODE == 8), TRACK = (MODE == 0);
     const int g = blockIdx.x, b = blockIdx.y;
     if (W.status[b] >= 0 && MODE != 4 && !SETUP) return;
+    if ((MODE == 4 || SETUP) && acb_masked_out(Sel.mask, b)) return;  // (the other modes see its status)
     constexpr bool DYN = (Q == 0);
     const int Tp = DYN ? D.Tp : 32 * Q, nq = DYN ? D.Tp / 32 : Q;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = blockDim.x >> 5;
@@ -340,7 +355,7 @@ __global__ void __launch_bounds__(Q > 0 ? 128 : 256, Q > 0 ? 5 : 1) k_rows(SiteD
         if (SETUP) {
             if (MODE == 6) {
                 // (warm_shift / warm_had: see the on-chip kernel)
-                const int wsh = B.warm_shift;
+                const int wsh = acb_warm_shift(B, Sel.shifts, b);
                 const bool hadW = !B.warm_had || B.warm_had[b] != 0;
 #pragma unroll
                 for (int q = 0; q < nq; ++q) {
@@ -1052,9 +1067,17 @@ __global__ void k_clear_check(GenWork W, int B_) {
     sc[GS_E1] = sc[GS_E2] = sc[GS_XMAX] = sc[GS_YMAX] = 0.f;
 }
 
-__global__ void k_finish(acb_batch B, GenWork W, GenDims D) {
+// coupling-row state of the solved instances (a skipped one got its copy of warm_vc, or nothing, in k_setup)
+__global__ void k_out_vc(acb_batch B, GenWork W, GenDims D, GenSel Sel) {
+    const int b = blockIdx.x;
+    if (acb_masked_out(Sel.mask, b)) return;
+    const size_t n = (size_t)D.R * D.Tp;
+    for (size_t i = threadIdx.x; i < n; i += blockDim.x) B.out_vc[(size_t)b * n + i] = W.VC[(size_t)b * n + i];
+}
+
+__global__ void k_finish(acb_batch B, GenWork W, GenDims D, GenSel Sel) {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= B.B) return;
+    if (b >= B.B || acb_masked_out(Sel.mask, b)) return;
     const float* sc = W.scal + (size_t)b * GS_N;
     int st = W.status[b];
     B.status[b] = st < 0 ? ACB_MAX_ITER : st;
@@ -1067,7 +1090,8 @@ __global__ void k_finish(acb_batch B, GenWork W, GenDims D) {
 }
 
 template <int Q>
-int run_general(acb_site* site, const acb_batch* batch, const acb_options& opt, cudaStream_t st) {
+int run_general(acb_site* site, const acb_batch* batch, const int32_t* solve_mask, const int32_t* warm_shifts, const acb_options& opt,
+                cudaStream_t st) {
     const SiteDev& d = site->d;
     const int B = batch->B, Tp = batch->Tp, N = d.N, R = d.R, NG = d.NG;
     GenDims D{N, R, NG, Tp, Tp / 32, batch->S_max, d.nDisc, d.nLin, d.has_pl, d.has_u, 2 * d.nDisc + d.nLin, 2 * d.nDisc + d.nLin + d.has_pl, d.lin_two_sided};
@@ -1098,6 +1122,7 @@ int run_general(acb_site* site, const acb_batch* batch, const acb_options& opt, 
     W.status = (int*)take(B, 4); W.iters = (int*)take(B, 4);
     W.row_first = (int*)take((size_t)B * N, 4); W.row_cnt = (int*)take((size_t)B * N, 4);
     W.ndone = (int*)take(1, 4);
+    const GenSel Sel{solve_mask, warm_shifts};
     ACB_CUDA(cudaMemsetAsync(W.ndone, 0, sizeof(int), st));
     ACB_CUDA(cudaMemsetAsync(W.HG, 0, nGT * sizeof(float), st));
     // row kernels: registers (Q > 0: 8 warps, Tp floats of partial sums each) or shared-memory staging (Q = 0: as many
@@ -1123,12 +1148,12 @@ int run_general(acb_site* site, const acb_batch* batch, const acb_options& opt, 
         ACB_CUDA(cudaFuncSetAttribute(k_rows<Q, 7>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)row_smem));
         ACB_CUDA(cudaFuncSetAttribute(k_rows<Q, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)row_smem));
     }
-#define ROWS(MODE) k_rows<Q, MODE><<<grow, row_threads, row_smem, st>>>(d, *batch, opt, W, D, site->grp_off_dev)
+#define ROWS(MODE) k_rows<Q, MODE><<<grow, row_threads, row_smem, st>>>(d, *batch, opt, W, D, site->grp_off_dev, Sel)
     const dim3 grow(NG, B), gcol((Tp + 32 * ACB_CPL - 1) / (32 * ACB_CPL), B);
-    k_setup<<<B, 256, 0, st>>>(d, *batch, opt, W, D);
+    k_setup<<<B, 256, 0, st>>>(d, *batch, opt, W, D, Sel);
     ROWS(6);
     if (!batch->lb_zero) ROWS(7);
-    k_setup_agg<<<B, 256, 0, st>>>(d, *batch, W, D, batch->lb_zero ? 0 : 1);
+    k_setup_agg<<<B, 256, 0, st>>>(d, *batch, W, D, batch->lb_zero ? 0 : 1, Sel);
     const size_t smem_cols = ((size_t)(NG + std::max(R, 1) + std::max(d.Rp, 4)) * 32 * ACB_CPL + (size_t)MM_KC * 128) * sizeof(float);
     const size_t smem_it = ((size_t)MM_KC * 128 + (size_t)(std::max(NG, std::max(d.nEigp, 4)) + std::max(R, 1) + std::max(d.Rp, 4)) * 32) * sizeof(float);
     if (smem_it > 48 * 1024) ACB_CUDA(cudaFuncSetAttribute(k_cols_it, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_it));
@@ -1175,8 +1200,9 @@ int run_general(acb_site* site, const acb_batch* batch, const acb_options& opt, 
         if (h_done >= B) break;
     }
     ROWS(4);
-    k_finish<<<(B + 127) / 128, 128, 0, st>>>(*batch, W, D);
-    if (batch->out_vc) ACB_CUDA(cudaMemcpyAsync(batch->out_vc, W.VC, nRT * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    k_finish<<<(B + 127) / 128, 128, 0, st>>>(*batch, W, D, Sel);
+    if (batch->out_vc && solve_mask) k_out_vc<<<B, 256, 0, st>>>(*batch, W, D, Sel);
+    else if (batch->out_vc) ACB_CUDA(cudaMemcpyAsync(batch->out_vc, W.VC, nRT * sizeof(float), cudaMemcpyDeviceToDevice, st));
     ACB_CUDA(cudaGetLastError());
     ACB_CUDA(cudaFreeAsync(base, st));
     return ACB_OK;
@@ -1185,11 +1211,12 @@ int run_general(acb_site* site, const acb_batch* batch, const acb_options& opt, 
 
 }  // namespace
 
-int acb_solve_general(acb_site* site, const acb_batch* batch, const acb_options& opt, cudaStream_t st) {
+int acb_solve_general(acb_site* site, const acb_batch* batch, const int32_t* solve_mask, const int32_t* warm_shifts, const acb_options& opt,
+                      cudaStream_t st) {
     const int Q = batch->Tp / 32;
-    if (Q == 2) return run_general<2>(site, batch, opt, st);
-    if (Q == 4) return run_general<4>(site, batch, opt, st);
-    if (Q == 5) return run_general<5>(site, batch, opt, st);
-    if (Q == 9) return run_general<9>(site, batch, opt, st);
-    return run_general<0>(site, batch, opt, st);  // any other multiple of 32: rows staged in shared memory
+    if (Q == 2) return run_general<2>(site, batch, solve_mask, warm_shifts, opt, st);
+    if (Q == 4) return run_general<4>(site, batch, solve_mask, warm_shifts, opt, st);
+    if (Q == 5) return run_general<5>(site, batch, solve_mask, warm_shifts, opt, st);
+    if (Q == 9) return run_general<9>(site, batch, solve_mask, warm_shifts, opt, st);
+    return run_general<0>(site, batch, solve_mask, warm_shifts, opt, st);  // any other multiple of 32: rows staged in shared memory
 }

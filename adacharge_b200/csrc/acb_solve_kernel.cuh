@@ -138,6 +138,8 @@ struct SolvePhase {
     float* st_mu;
     float* st_scal;
     float* zprev;      // [B][N][Tp] schedule at the previous check (rate polish) or NULL
+    const int32_t* solve_mask;   // acb_solve_batch_masked: [B] 0 = not solved, or NULL
+    const int32_t* warm_shifts;  // [B] per-instance warm shift, or NULL (acb_batch.warm_shift)
 };
 
 #ifdef ACB_TRACE
@@ -187,6 +189,7 @@ __global__ void __launch_bounds__(TPW == 2 ? 1024 : (FAST ? ACB_FAST_THREADS : 7
 
     if (P.count && (int)blockIdx.x >= *P.count) return;
     const int b = P.list ? P.list[blockIdx.x] : blockIdx.x;
+    if (acb_masked_out(P.solve_mask, b)) { acb_keep_warm(B, b, N, R, Tp); return; }  // not solved this step (a relaunch never lists it)
     const int Tb = B.T[b];
     const int nS = B.n_sessions[b];
     const int nDisc = S.nDisc, nLin = S.nLin;
@@ -230,9 +233,9 @@ __global__ void __launch_bounds__(TPW == 2 ? 1024 : (FAST ? ACB_FAST_THREADS : 7
     // ------------------------------------------------------------------ prologue
     for (int i = tid; i < 2 * N * Tp; i += nthreads) LB[i] = 0.f;  // LB (FAST: v) and UB are contiguous
     // warm start of a closed-loop replay: the previous step's state is read `warm_shift` columns ahead (column t of this
-    // problem was column t + 1 of the previous one), and instances whose site was idle before start cold (warm_had = 0:
-    // no warm array is read, the same start as a solve without warm arrays)
-    const int wsh = B.warm_shift;
+    // problem was column t + 1 of the previous one; per instance with P.warm_shifts), and instances whose site was idle
+    // before start cold (warm_had = 0: no warm array is read, the same start as a solve without warm arrays)
+    const int wsh = acb_warm_shift(B, P.warm_shifts, b);
     const bool hadW = !B.warm_had || B.warm_had[b] != 0;
     const float* warm_v1 = hadW ? B.warm_v1 : nullptr;
     for (int i = tid; i < R * Tp; i += nthreads) {

@@ -304,13 +304,17 @@ class DeviceBatch:
         return dict(v1=mk(B, self.site.N, Tp), vc=mk(B, max(self.site.R, 1), Tp), mu=mk(B, self.S_max), scal=mk(B, 2))
 
     def set_warm(self, warm: Optional[Dict[str, torch.Tensor]] = None, out: Optional[Dict[str, torch.Tensor]] = None, shift: int = 0,
-                 had: Optional[torch.Tensor] = None):
+                 had: Optional[torch.Tensor] = None, shifts: Optional[torch.Tensor] = None, mask: Optional[torch.Tensor] = None):
         """Where the following solves start from and where they leave their final state (see `warm`, `warm_out`).
-        `warm` is read `shift` columns ahead (1: the previous control step's state), and an instance whose `had` [B]
-        int32 entry is 0 starts cold (its site was idle before)."""
+        `warm` is read `shift` columns ahead (1: the previous control step's state), or `shifts[b]` columns ahead for
+        instance b when the [B] int32 `shifts` is given, and an instance whose `had` [B] int32 entry is 0 starts cold (its
+        site was idle before).  An instance whose `mask` [B] int32 entry is 0 is not solved: its results keep their
+        values and `out` receives an unshifted copy of its `warm` state.  With `shifts` or `mask`, solve() calls
+        acb_solve_batch_masked."""
         self.warm, self.warm_out = warm, out
         self.struct.warm_shift, self.struct.warm_had = shift, _ptr(had)
         self._had = had  # the struct holds a raw pointer: keep the tensor alive
+        self.warm_shifts, self.solve_mask = shifts, mask
 
     @property
     def warm(self) -> Optional[Dict[str, torch.Tensor]]:
@@ -340,9 +344,14 @@ class DeviceBatch:
         self.struct.pilots = _ptr(self.pilots) if on else None
 
     def solve(self, options: Options, stream=None):
-        """Enqueue acb_solve_batch on `stream` (a cudaStream_t; default: the current stream)."""
+        """Enqueue acb_solve_batch (acb_solve_batch_masked with set_warm's `mask` / `shifts`) on `stream` (a cudaStream_t;
+        default: the current stream)."""
         st = _stream_ptr(self.site.device) if stream is None else stream
-        _cabi.check(_cabi.lib().acb_solve_batch(self.site.handle, C.byref(self.struct), C.byref(options), st), "acb_solve_batch")
+        if self.solve_mask is None and self.warm_shifts is None:
+            _cabi.check(_cabi.lib().acb_solve_batch(self.site.handle, C.byref(self.struct), C.byref(options), st), "acb_solve_batch")
+        else:
+            _cabi.check(_cabi.lib().acb_solve_batch_masked(self.site.handle, C.byref(self.struct), _ptr(self.solve_mask), _ptr(self.warm_shifts),
+                                                           C.byref(options), st), "acb_solve_batch_masked")
         return self
 
 

@@ -4,8 +4,14 @@ AdaptiveSchedulingAlgorithm.schedule (reference adacharge/adacharge.py:135-193) 
 site at once — but the EVs of all sites live in flat numpy arrays and the acb_batch is
 packed with array operations, so the host cost per step is O(milliseconds) for a thousand
 sites instead of one Python object per session.  The batch always holds every site (idle
-sites carry zero sessions), so the warm-start state of step t lines up with step t+1 by
+sites carry zero sessions), so the warm-start state of a site lines up with its next solve by
 construction; session multipliers follow their EV through a per-EV table on the device.
+
+`max_recompute` is the Simulator's re-solve rule (DESIGN.md §8): a site re-solves at a plug-in or
+unplug there and after `max_recompute` steps without one (None: at events only; 1, the default:
+every step); in between each EVSE gets the next column of the site's last schedule.  The solve
+(acb_solve_batch_masked) skips the other sites (solve_mask) and warm-starts each site from its own
+last solve (warm_shifts).
 
 Sharding: sites are independent, so a rank replays `sharding.shard_range(n_sites, ...)`
 of them with no data-path collective; `summary()` returns what `gather_summaries` reduces.
@@ -20,6 +26,7 @@ import numpy as np
 import torch
 
 from . import _cabi, engine
+from .adacharge import quantized_max_recompute
 from .adaptive_charging_optimization import ObjectiveComponent, pack_objective
 from .interface import TestingInterface, infrastructure_from_dict
 from .replay import REPLAY_SOLVER_DEFAULTS, synthetic_day
@@ -29,8 +36,9 @@ from .replay import REPLAY_SOLVER_DEFAULTS, synthetic_day
 class FleetStats:
     iters_mean: List[float] = field(default_factory=list)
     iters_max: List[int] = field(default_factory=list)
-    unsolved: List[int] = field(default_factory=list)      # instances per step whose status != ACB_SOLVED
-    active_sites: List[int] = field(default_factory=list)
+    unsolved: List[int] = field(default_factory=list)      # solves per step whose status != ACB_SOLVED
+    active_sites: List[int] = field(default_factory=list)  # sites per step with sessions
+    solved_sites: List[int] = field(default_factory=list)  # ... of which re-solved this step (the others applied their last schedule)
     host_ms: List[float] = field(default_factory=list)     # packing + bookkeeping on the host
     device_ms: List[float] = field(default_factory=list)   # upload + solve + projection + read-back of the pilots
     delivered_frac: Optional[np.ndarray] = None
@@ -44,13 +52,23 @@ class FleetReplay:
     `uninterrupted_charging` is its flag too (acnportal's apply_minimum_charging_rate with override = period): each step
     the EVs of a site are offered min(min_pilot, period) as their first-period minimum in arrival order while the network
     stays feasible.  An EV whose remaining energy is less than one period at that rate is not offered it (the
-    reference would make the whole site's problem infeasible until that EV leaves)."""
+    reference would make the whole site's problem infeasible until that EV leaves).
+    `max_recompute` is AdaptiveSchedulingAlgorithm's kwarg as acnportal's Simulator reads it: a site re-solves when an EV
+    plugs in or unplugs there or `max_recompute` steps after its last solve (None: at events only); in between its EVSEs
+    get the next column of its last schedule.  The default 1 re-solves every site every step (the reference's default is
+    None); with `quantize` it is 1, with the reference's warning if anything else was asked for."""
 
     def __init__(self, infra: Dict, objective: List[ObjectiveComponent], n_sites: int, steps_per_day: int = 288, days: int = 1,
                  period: float = 5, prices: Optional[np.ndarray] = None, demand_charge: float = 15.51, seed0: int = 0,
                  warm_start: bool = True, solver_options: Optional[dict] = None, device=None, mean_sessions: int = 40,
                  Tp: int = 288, site_offset: int = 0, quantize: bool = False, reallocate: bool = False,
-                 uninterrupted_charging: bool = False):
+                 uninterrupted_charging: bool = False, max_recompute: Optional[int] = 1):
+        if max_recompute is not None and not (isinstance(max_recompute, (int, np.integer)) and not isinstance(max_recompute, bool)
+                                              and max_recompute >= 1):
+            raise ValueError(f"max_recompute must be None or an integer >= 1, not {max_recompute!r}")
+        self.max_recompute = quantized_max_recompute(max_recompute, quantize, default=1)
+        # at 1 every site re-solves every step: the solve then needs neither the mask nor per-site warm shifts
+        self._event_driven = self.max_recompute != 1
         self.infra, self.objective, self.n_sites, self.period = infra, objective, n_sites, period
         self.steps_per_day, self.days, self.steps = steps_per_day, days, steps_per_day * days
         self.warm_start, self.device, self.Tp = warm_start, device, Tp
@@ -99,8 +117,12 @@ class FleetReplay:
         self._day_slice = [slice(int(edges[d]), int(edges[d + 1])) for d in range(days)]
         self._w_ev = self.volt[self.ev_station] * period / 1e3 / 60  # kWh per A-period of each EV's EVSE
         self.prev_peak = np.zeros(n_sites)  # A
+        self.last_solve = np.full(n_sites, -1, dtype=np.int64)  # step of each site's last solve
+        self.had = np.zeros(n_sites, dtype=np.int32)  # 1 if the site had sessions at its last solve
+        self.recompute: Optional[np.ndarray] = None  # the last step's re-solve decision per site
         self.site: Optional[engine.Site] = None
-        self._prev = None  # (EV index / site / position of the previous step's sessions, had-sessions mask)
+        self._prev = None  # EV index / site / position of the previous step's sessions
+        self._sched: Optional[torch.Tensor] = None  # each site's pilots from its last solve [B, N, Tp]
         self._pb: Optional[engine.PackedBatch] = None  # one batch object for the whole replay (refilled every step)
         self._state = None  # two sets of warm-state tensors: a step reads the previous step's set and writes the other
         self.stats = FleetStats()
@@ -214,9 +236,24 @@ class FleetReplay:
         self._arr_order[order] = np.arange(len(order)) - np.concatenate(([0], np.cumsum(n_s)[:-1]))[s[order]]
         self._max0, self._limits0 = mx0, (mn0, mx0)
 
+    def _recompute(self, t: int):
+        """Which sites re-solve at step t (what acb_fleet_sessions decides on the device), and each site's t - last_solve:
+        no solve yet, an EV plugs in or unplugs there now, or max_recompute steps since the last solve."""
+        spd, ev = self.steps_per_day, np.zeros(self.n_sites, dtype=bool)
+        d = t // spd
+        slices = [self._day_slice[min(d, self.days - 1)]]
+        if t % spd == 0 and 1 <= d <= self.days:
+            slices.append(self._day_slice[d - 1])  # a previous-day EV unplugging at midnight
+        for sl in slices:
+            ev[self.ev_site[sl][(self.ev_arr[sl] == t) | (self.ev_dep[sl] == t)]] = True
+        since = t - self.last_solve
+        mr = self.max_recompute or 0
+        return (self.last_solve < 0) | ev | ((mr > 0) & (since >= mr)), since
+
     # ------------------------------------------------------------------ one control step
     def step(self, t: int):
         t0 = time.perf_counter()
+        rec, since = self._recompute(t)
         h, idx, s, pos, n_sess = self._pack(t)
         if self.site is None:
             use_u = bool((h["gamma"] > 0).any() or (h["peak_w"] > 0).any())
@@ -238,13 +275,29 @@ class FleetReplay:
         ev0.record()
         idx_d = torch.from_numpy(idx).to(dev)
         s_d, pos_d = torch.from_numpy(s).to(dev), torch.from_numpy(pos).to(dev)
+        i32 = lambda a: torch.from_numpy(np.ascontiguousarray(a, dtype=np.int32)).to(dev)  # noqa: E731
+        rec_d, shift_d = i32(rec), i32(since)
+        ev = self._event_driven
         if self.warm_start and self._prev is not None:
-            pb.set_warm(self._warm(prev, idx_d, s_d, pos_d), out, shift=1, had=self._prev[-1])
+            pb.set_warm(self._warm(prev, idx_d, s_d, pos_d), out, shift=1, had=i32(self.had), shifts=shift_d if ev else None,
+                        mask=rec_d if ev else None)
         else:
-            pb.set_warm(None, out)
+            pb.set_warm(None, out, mask=rec_d if ev else None)
         pb.upload().solve(self.options)
         pilots = self._project(pb.rates.to(torch.float64), h, idx, s, pos)
-        first = pilots[:, :, 0].contiguous().cpu().numpy()
+        # the sites that re-solved take their new schedule's column 0, the others column t - last_solve of their last one
+        # (0 from Tp on)
+        if self._sched is None:
+            self._sched = pilots.clone()
+        else:
+            self._sched[rec_d.bool()] = pilots[rec_d.bool()]
+        self.last_solve[rec] = t
+        self.had[rec] = n_sess[rec] > 0
+        col = t - self.last_solve
+        B = self.n_sites
+        first_d = self._sched.gather(2, i32(np.minimum(col, self.Tp - 1)).long().view(B, 1, 1).expand(B, self.N, 1)).squeeze(2)
+        first_d[torch.from_numpy(col >= self.Tp).to(dev)] = 0.0
+        first = first_d.cpu().numpy()
         it, stt = pb.iters.cpu().numpy(), pb.status.cpu().numpy()
         ev1.record()
         ev1.synchronize()
@@ -255,14 +308,17 @@ class FleetReplay:
         e = np.minimum(first[self.ev_site[present], self.ev_station[present]] * self._w_ev[present], self.ev_req[present] - self.ev_dlv[present])
         self.ev_dlv[present] += np.maximum(e, 0.0)
         self.prev_peak = np.maximum(self.prev_peak, first.sum(axis=1))
-        self._prev = (idx_d, s_d, pos_d, torch.from_numpy((n_sess > 0).astype(np.int32)).to(dev))
+        self._prev = (idx_d, s_d, pos_d)
         self._state.reverse()
+        self.recompute = rec
         act = n_sess > 0
+        sol = act & rec
         st_ = self.stats
-        st_.iters_mean.append(float(it[act].mean()) if act.any() else 0.0)
-        st_.iters_max.append(int(it[act].max()) if act.any() else 0)
-        st_.unsolved.append(int((stt[act] != _cabi.ACB_SOLVED).sum()))
+        st_.iters_mean.append(float(it[sol].mean()) if sol.any() else 0.0)
+        st_.iters_max.append(int(it[sol].max()) if sol.any() else 0)
+        st_.unsolved.append(int((stt[sol] != _cabi.ACB_SOLVED).sum()))
         st_.active_sites.append(int(act.sum()))
+        st_.solved_sites.append(int(sol.sum()))
         st_.device_ms.append(ev0.elapsed_time(ev1))
         st_.host_ms.append((t1 - t0 + time.perf_counter() - t2) * 1e3)
         return first
@@ -294,9 +350,10 @@ class FleetReplay:
         return engine.project_discrete(self.site, rates)
 
     def _warm(self, prev, idx_d, s_d, pos_d):
-        """The previous step's state for this step's solve, which reads it one period ahead (sites idle before start
-        cold through warm_had); the session multipliers follow their EV."""
-        pidx, ps, ppos, _ = self._prev
+        """The state each site's last solve left (a step that skips a site copies it forward) for this step's solve,
+        which reads it t - last_solve periods ahead (sites idle at their last solve start cold through warm_had); the
+        session multipliers follow their EV."""
+        pidx, ps, ppos = self._prev
         mu_ev = torch.zeros(len(self.ev_req), dtype=torch.float32, device=prev["mu"].device)
         mu_ev[pidx] = prev["mu"][ps, ppos]
         mu = torch.zeros_like(prev["mu"])
@@ -315,9 +372,9 @@ class FleetReplay:
     def summary(self) -> Dict[str, float]:
         s = self.stats
         n = max(len(s.device_ms), 1)
-        return dict(site_steps=float(sum(s.active_sites)), steps=float(len(s.device_ms)), unsolved=float(sum(s.unsolved)),
-                    device_ms=float(sum(s.device_ms)), host_ms=float(sum(s.host_ms)),
-                    iters_mean=float(np.average(s.iters_mean, weights=np.maximum(s.active_sites, 1e-9))) if n else 0.0,
+        return dict(site_steps=float(sum(s.active_sites)), solves=float(sum(s.solved_sites)), steps=float(len(s.device_ms)),
+                    unsolved=float(sum(s.unsolved)), device_ms=float(sum(s.device_ms)), host_ms=float(sum(s.host_ms)),
+                    iters_mean=float(np.average(s.iters_mean, weights=np.maximum(s.solved_sites, 1e-9))) if n else 0.0,
                     iters_max=float(max(s.iters_max, default=0)))
 
 
@@ -325,8 +382,9 @@ class DeviceFleetReplay(FleetReplay):
     """FleetReplay with the simulator side of the control step on the device as well (SURVEY.md §8(f) N1): the EV table,
     the energy delivered, the previous peaks and the per-EV warm-start multipliers stay in device arrays; a step is four
     launches on one stream -- active sessions (acb_fleet_sessions), packing (acb_pack_sessions), the warm-started solve
-    whose prologue reads the previous state one column ahead (acb_batch.warm_shift) and whose epilogue projects the
-    pilots, and the simulator update (acb_fleet_apply) -- with no host synchronisation between steps.  Quantised pilots
+    whose prologue reads each site's last state t - last_solve columns ahead (acb_solve_batch_masked's warm_shifts) and whose epilogue
+    projects the pilots, and the simulator update (acb_fleet_apply) -- with no host synchronisation between steps.  The
+    re-solve decision (max_recompute) is made by acb_fleet_sessions and is the solve's solve_mask.  Quantised pilots
     take a fifth launch (acb_quantize_pilots) between the solve and the update, uninterrupted charging one more
     (acb_admit_sessions) between the active sessions and the packing.  Same schedules, bit for bit, as FleetReplay
     (tests/test_gpu_replay.py, tests/test_gpu_uninterrupted.py).
@@ -363,6 +421,8 @@ class DeviceFleetReplay(FleetReplay):
             sess_ev=torch.full((self.n_sites, self.N), -1, dtype=torch.int32, device=dev),
             warm_mu=torch.zeros((self.n_sites, self.N), dtype=torch.float32, device=dev),
             first=torch.zeros((self.n_sites, self.N), dtype=torch.float64, device=dev), stats=torch.zeros(3, dtype=torch.float64, device=dev),
+            last_solve=torch.full((self.n_sites,), -1, dtype=torch.int32, device=dev),
+            recompute=torch.zeros(self.n_sites, dtype=torch.int32, device=dev), shift=torch.zeros(self.n_sites, dtype=torch.int32, device=dev),
         )
         # first EV of every (day, site): the table is sorted by (day, site, station)
         key = (self.ev_arr // self.steps_per_day) * self.n_sites + self.ev_site
@@ -374,6 +434,9 @@ class DeviceFleetReplay(FleetReplay):
         d = self._d
         f.ev_station, f.ev_arr, f.ev_dep, f.ev_req, f.ev_max = p(d["station"]), p(d["arr"]), p(d["dep"]), p(d["req"]), p(d["mx"])
         f.ev_dlv, f.ev_mu, f.day_site_off, f.prev_peak, f.had = p(d["dlv"]), p(d["mu"]), p(d["off"]), p(d["prev_peak"]), p(d["had"])
+        f.max_recompute = self.max_recompute or 0
+        if self._event_driven:  # (NULL last_solve: every site solves every step, column 0 applies)
+            f.last_solve, f.recompute, f.shift = p(d["last_solve"]), p(d["recompute"]), p(d["shift"])
         self._fleet = f
         self._state = [ch.new_warm_state(), ch.new_warm_state()]
         ch.lb_zero = self.lb_zero  # the synthetic EVs have no minimum rate of their own
@@ -388,7 +451,9 @@ class DeviceFleetReplay(FleetReplay):
         st = C.c_void_p(torch.cuda.current_stream(self._bac.device).cuda_stream)
         o = ch.objective
         prev, out = self._state
-        ch.set_warm(dict(prev, mu=d["warm_mu"]) if self.warm_start and self._started else None, out, shift=1, had=d["had"])
+        ev = self._event_driven
+        ch.set_warm(dict(prev, mu=d["warm_mu"]) if self.warm_start and self._started else None, out, shift=1, had=d["had"],
+                    shifts=d["shift"] if ev else None, mask=d["recompute"] if ev else None)
         o.prices = C.c_void_p(d["prices"].data_ptr() + 8 * t) if self._bac.need_prices else None
         _cabi.check(L.acb_fleet_sessions(self.site.handle, C.byref(self._fleet), t, C.byref(ch.sessions), p(d["sess_ev"]), p(d["warm_mu"]), st), "acb_fleet_sessions")
         if self.uninterrupted_charging:
@@ -423,4 +488,5 @@ class DeviceFleetReplay(FleetReplay):
 
     def summary(self) -> Dict[str, float]:
         s = self._d["stats"].cpu().numpy()
-        return dict(site_steps=float(s[0]), unsolved=float(s[2]), iters_mean=float(s[1] / max(s[0], 1.0)))
+        # (site_steps counts the solves of sites with sessions: with max_recompute != 1 the steps in between are not in it)
+        return dict(site_steps=float(s[0]), solves=float(s[0]), unsolved=float(s[2]), iters_mean=float(s[1] / max(s[0], 1.0)))

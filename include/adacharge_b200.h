@@ -12,7 +12,7 @@
  *       max_pilot / allowable_pilots            adacharge/postprocessing.py:92,114,176
  *   acb_charging_rate_bounds
  *       AdaptiveChargingOptimization.charging_rate_bounds        ...optimization.py:45-79
- *   acb_solve_batch
+ *   acb_solve_batch / acb_solve_batch_masked
  *       build_problem + solve (cvxpy canonicalisation + ECOS)    ...optimization.py:220-321
  *       objective library quick_charge ... load_flattening        ...optimization.py:363-408
  *   acb_project_continuous      project_into_continuous_feasible_pilots   postprocessing.py:77-94
@@ -178,6 +178,16 @@ typedef struct acb_batch {
 } acb_batch;
 
 int acb_solve_batch(acb_site* site, const acb_batch* batch, const acb_options* opt, void* stream);
+/* Event-driven recompute (closed-loop replays that re-solve a site only at events or every max_recompute steps):
+ * acb_solve_batch with two optional [B] device arrays (acb_solve_batch = both NULL; acb_batch keeps its layout).
+ *  solve_mask   NULL = solve every instance.  An instance with solve_mask[b] == 0 is not solved and none of its outputs is
+ *               written (rates, pilots, rate_est, status, iters, stats), except that with both warm_* and out_* given its
+ *               out_v1 / out_vc / out_mu / out_scal receive an unshifted copy of its warm_v1 / warm_vc / warm_mu / warm_scal
+ *               (a replay that alternates two state sets keeps the state of a site it skips).
+ *  warm_shifts  NULL = batch->warm_shift for every instance; else instance b reads its warm arrays warm_shifts[b] columns
+ *               ahead (zero beyond the horizon). */
+int acb_solve_batch_masked(acb_site* site, const acb_batch* batch, const int32_t* solve_mask, const int32_t* warm_shifts,
+                           const acb_options* opt, void* stream);
 
 /* ---- packing on the device: raw session tables + interface quantities -> the acb_batch input fields ----
  * What the reference does on the host before every solve (T = max(arrival_offset + remaining_time) aco.py:243-245,
@@ -258,11 +268,14 @@ int acb_reallocate(acb_site* site, int mode, const double* rates_in, double* rat
  * Columns >= T[b] are 0.  The reallocation takes the sessions in slot order (empty slots, station < 0, skipped) and their
  * ramp as interface.remaining_amp_periods: remaining_demand * 1000 / voltage * (60 / period), and max_rates[0] from
  * sessions->max_rate0 when given (acb_admit_sessions), else max_rate.  The site needs
- * allowable_pilots; sessions->B must equal batch->B. */
+ * allowable_pilots; sessions->B must equal batch->B.  acb_quantize_pilots_masked: an instance with solve_mask[b] == 0 (the
+ * mask of acb_solve_batch_masked; NULL = none) keeps its pilots. */
 #define ACB_PILOTS_DISCRETE 1   /* project_into_discrete_feasible_pilots   postprocessing.py:97-118 */
 #define ACB_PILOTS_REALLOCATE 2 /* diff_based_reallocation                 postprocessing.py:189-258 */
 int acb_quantize_pilots(acb_site* site, int mode, const acb_sessions* sessions, double period, const acb_batch* batch,
                         double* pilots, void* stream);
+int acb_quantize_pilots_masked(acb_site* site, int mode, const acb_sessions* sessions, double period, const acb_batch* batch,
+                               const int32_t* solve_mask, double* pilots, void* stream);
 
 /* feasible[b] = 1 iff every SOC line current of column `col` is <= limit + 1e-7. */
 int acb_constraints_feasible(acb_site* site, const double* rates, int B, int T, int col, int32_t* feasible, void* stream);
@@ -311,20 +324,30 @@ typedef struct acb_fleet {
     float* ev_mu;                /* [n_ev] state: energy-row multiplier of the EV's last solve (warm start) */
     const int32_t* day_site_off; /* [days * n_sites + 1] */
     double* prev_peak;           /* [n_sites] state: largest aggregate first-period current so far, A (interface.get_prev_peak) */
-    int32_t* had;                /* [n_sites] state: 1 if the site had sessions in the previous step */
+    int32_t* had;                /* [n_sites] state: 1 if the site had sessions at its last solve */
+    /* event-driven recompute (acnportal's Simulator re-solves a site only at a plug-in or unplug there, or when max_recompute
+     * periods have passed since its last solve; in between each EVSE gets the next column of the last schedule) */
+    int32_t max_recompute;       /* 0 = at events only (max_recompute None); k >= 1 = also at least every k steps */
+    int32_t* last_solve;         /* [n_sites] state: step of the site's last solve, -1 = none yet; NULL = every site solves every step */
+    int32_t* recompute;          /* [n_sites] written by acb_fleet_sessions (with last_solve): 1 = solve this step (acb_solve_batch_masked's solve_mask) */
+    int32_t* shift;              /* [n_sites] written by acb_fleet_sessions (with last_solve): t - last_solve (its warm_shifts) */
 } acb_fleet;
 
 /* Step t: the active sessions of every site (plugged in, energy still owed) into the raw tables acb_pack_sessions takes
  * (arrival_offset 0, remaining_time = departure - t, remaining_demand = requested - delivered, arrival = ev_arr if
  * sessions->arrival is given), plus the EV behind each slot (sess_ev [n_sites][S_max], -1 = empty) and its warm-start
  * multiplier (warm_mu [n_sites][S_max]).  Slots are in station order; sess_ev and warm_mu keep that order after
- * acb_admit_sessions, which is the packed order of a single-session site. */
+ * acb_admit_sessions, which is the packed order of a single-session site.  With last_solve: recompute[b] = 1 if the site has
+ * never solved, an EV plugs in or unplugs there at t (ev_arr == t or ev_dep == t; an EV that has its energy but is still
+ * plugged in is no event), or max_recompute > 0 and t - last_solve[b] >= max_recompute; shift[b] = t - last_solve[b]. */
 int acb_fleet_sessions(acb_site* site, const acb_fleet* fleet, int t, const acb_sessions* sessions, int32_t* sess_ev, float* warm_mu,
                        void* stream);
 /* After the solve of step t: the first-period pilots (batch->pilots) charge every plugged-in EV (delivered energy capped at
  * the request), prev_peak and had are updated, the session multipliers (batch->out_mu) go back to their EVs.  first_pilots
  * (optional [n_sites][N]) receives the applied pilots; stats (optional, 3 doubles) accumulates site-steps solved, iterations,
- * uncertified solves. */
+ * uncertified solves.  With last_solve: a site that solved (recompute[b]) applies column 0 and sets last_solve[b] = t; any
+ * other site applies column c = t - last_solve[b] of the pilots its last solve left in batch->pilots (0 for c >= Tp), and
+ * only sites that solved update had, their EVs' multipliers and stats. */
 int acb_fleet_apply(acb_site* site, const acb_fleet* fleet, int t, double period, const acb_batch* batch, const int32_t* sess_ev,
                     double* first_pilots, double* stats, void* stream);
 
