@@ -18,7 +18,7 @@ ACB_PILOTS_DISCRETE, ACB_PILOTS_REALLOCATE = 1, 2  # acb_quantize_pilots modes
 EXPORTS = [
     "acb_site_create", "acb_site_destroy", "acb_site_dims", "acb_site_max_horizon", "acb_default_options",
     "acb_solve_batch", "acb_solve_batch_masked", "acb_charging_rate_bounds", "acb_project_continuous", "acb_project_discrete",
-    "acb_reallocate", "acb_quantize_pilots", "acb_quantize_pilots_masked", "acb_constraints_feasible", "acb_min_rate_admission", "acb_admit_sessions", "acb_pack_sessions", "acb_preprocess_sessions", "acb_fleet_sessions", "acb_fleet_apply", "acb_last_error", "acb_version",
+    "acb_reallocate", "acb_quantize_pilots", "acb_quantize_pilots_masked", "acb_constraints_feasible", "acb_min_rate_admission", "acb_admit_sessions", "acb_pack_sessions", "acb_preprocess_sessions", "acb_fleet_sessions", "acb_fleet_apply", "acb_fleet_sessions_ev", "acb_fleet_apply_ev", "acb_last_error", "acb_version",
 ]
 ACB_MAX_COMPONENTS = 16
 # acb_objective.kind values (include/adacharge_b200.h)
@@ -75,6 +75,11 @@ class Fleet(C.Structure):
                 ("max_recompute", C.c_int32), ("last_solve", _P), ("recompute", _P), ("shift", _P)]
 
 
+class FleetEV(C.Structure):
+    _fields_ = [("ev_cap", _P), ("ev_charge", _P), ("transition_soc", C.c_double), ("ev_ub", _P), ("up_increment", C.c_double),
+                ("down_threshold", C.c_double), ("upper_bound", _P), ("rates", _P)]
+
+
 _lib = None
 
 
@@ -110,6 +115,8 @@ def lib():
     L.acb_preprocess_sessions.argtypes = [_P, C.POINTER(Sessions), C.c_int, _P, _P]
     L.acb_fleet_sessions.argtypes = [_P, C.POINTER(Fleet), C.c_int, C.POINTER(Sessions), _P, _P, _P]
     L.acb_fleet_apply.argtypes = [_P, C.POINTER(Fleet), C.c_int, C.c_double, C.POINTER(Batch), _P, _P, _P, _P]
+    L.acb_fleet_sessions_ev.argtypes = [_P, C.POINTER(Fleet), C.POINTER(FleetEV), C.c_int, C.POINTER(Sessions), _P, _P, _P]
+    L.acb_fleet_apply_ev.argtypes = [_P, C.POINTER(Fleet), C.POINTER(FleetEV), C.c_int, C.c_double, C.POINTER(Batch), _P, _P, _P, _P]
     L.acb_pack_sessions.argtypes = [_P, C.POINTER(Sessions), C.POINTER(Objective), C.POINTER(Batch), _P, _P]
     _lib = L
     return L

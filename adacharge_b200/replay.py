@@ -46,6 +46,18 @@ def synthetic_day(infra: Dict, seed: int, steps: int = 288, period: float = 5, m
     return [EV(int(s), f"s{seed}-{j}", int(a), int(d), float(r)) for j, (s, a, d, r) in enumerate(zip(stations, arr, dep, req))]
 
 
+def synthetic_batteries(seed: int, requested) -> tuple:
+    """Seeded batteries for the EVs of one site-day (requested: their requests in kWh, in synthetic_day's order):
+    (capacity, initial charge), kWh.  The request would bring each battery to a state of charge soc_f ~ U(0.75, 1); the
+    capacity is U(30, 80) kWh, raised to requested / soc_f where that is larger, and the initial charge soc_f * capacity -
+    requested.  Its own generator ((seed, 1)), so the EVs of synthetic_day(seed) do not change."""
+    rng = np.random.default_rng((seed, 1))
+    req = np.asarray(requested, dtype=np.float64)
+    soc_f = rng.uniform(0.75, 1.0, len(req))
+    cap = np.maximum(rng.uniform(30.0, 80.0, len(req)), req / soc_f)
+    return cap, soc_f * cap - req
+
+
 class _SiteIface(TestingInterface):
     """TestingInterface whose price vector is indexed by absolute time."""
 

@@ -13,6 +13,11 @@ every step); in between each EVSE gets the next column of the site's last schedu
 (acb_solve_batch_masked) skips the other sites (solve_mask) and warm-starts each site from its own
 last solve (warm_shifts).
 
+`battery` gives every EV a two-stage battery (`battery_current`: acnportal's Linear2StageBattery without noise, in
+amperes) that takes less than its pilot near full charge; `estimate_max_rate` is AdaptiveSchedulingAlgorithm's flag with
+acnportal's SimpleRampdown estimator (`rampdown_update`), whose per-EV bound caps the session's maximum rate at every
+solve (DESIGN.md §8 states both rules).
+
 Sharding: sites are independent, so a rank replays `sharding.shard_range(n_sites, ...)`
 of them with no data-path collective; `summary()` returns what `gather_summaries` reduces.
 """
@@ -29,7 +34,31 @@ from . import _cabi, engine
 from .adacharge import quantized_max_recompute
 from .adaptive_charging_optimization import ObjectiveComponent, pack_objective
 from .interface import TestingInterface, infrastructure_from_dict
-from .replay import REPLAY_SOLVER_DEFAULTS, synthetic_day
+from .replay import REPLAY_SOLVER_DEFAULTS, synthetic_batteries, synthetic_day
+
+
+def battery_current(p, w, amax, cap, charge, owed, transition_soc):
+    """One step of two-stage batteries, element-wise (what acb_fleet_apply_ev computes, bit for bit): the current a (A)
+    each battery takes under pilot p on an EVSE of w kWh per A-period, and the energy de (kWh) it receives.
+      a = 0 if p == 0; else min(p, amax) below transition_soc and min(p, (1 - soc) / (1 - transition_soc) * amax) from it
+      on (soc = charge / cap), cut to (cap - charge) / w where charge + a * w would pass cap, and at least 0;
+      de = max(min(a * w, owed), 0)."""
+    with np.errstate(divide="ignore", invalid="ignore"):
+        soc = charge / cap
+        lim = np.where(soc < transition_soc, amax, ((1.0 - soc) / (1.0 - transition_soc)) * amax)
+        a = np.where(lim < p, lim, p)
+        a = np.where(charge + a * w > cap, (cap - charge) / w, a)
+    a = np.where(p == 0.0, 0.0, np.where(a > 0.0, a, 0.0))
+    de = a * w
+    de = np.where(owed < de, owed, de)
+    return a, np.where(de > 0.0, de, 0.0)
+
+
+def rampdown_update(ub, p, a, up_increment, down_threshold):
+    """acnportal's SimpleRampdown after one applied step, element-wise: where the EV took more than down_threshold below
+    its pilot its bound becomes a + up_increment, elsewhere it stays.  Returns (new bounds, where it fired)."""
+    fire = (p - a) > down_threshold
+    return np.where(fire, a + up_increment, ub), fire
 
 
 @dataclass
@@ -56,13 +85,28 @@ class FleetReplay:
     `max_recompute` is AdaptiveSchedulingAlgorithm's kwarg as acnportal's Simulator reads it: a site re-solves when an EV
     plugs in or unplugs there or `max_recompute` steps after its last solve (None: at events only); in between its EVSEs
     get the next column of its last schedule.  The default 1 re-solves every site every step (the reference's default is
-    None); with `quantize` it is 1, with the reference's warning if anything else was asked for."""
+    None); with `quantize` it is 1, with the reference's warning if anything else was asked for.
+    `battery`: every EV has a two-stage battery (`synthetic_batteries` of its site-day: `ev_cap`, `ev_charge`) that takes
+    the current `battery_current` gives under its pilot, tapering from `transition_soc` on; the site's peak is the sum of
+    those currents.  `rates` holds each EVSE's current of the last step.  `estimate_max_rate`: each EV keeps acnportal's
+    SimpleRampdown estimate `ev_ub` (from its EVSE's max_pilot; `rampdown_update` with `up_increment` and
+    `down_threshold`), and every solve caps the session's maximum rate at it (apply_upper_bound_estimate).  Without
+    `battery` every EV takes its pilot and the estimate never moves."""
 
     def __init__(self, infra: Dict, objective: List[ObjectiveComponent], n_sites: int, steps_per_day: int = 288, days: int = 1,
                  period: float = 5, prices: Optional[np.ndarray] = None, demand_charge: float = 15.51, seed0: int = 0,
                  warm_start: bool = True, solver_options: Optional[dict] = None, device=None, mean_sessions: int = 40,
                  Tp: int = 288, site_offset: int = 0, quantize: bool = False, reallocate: bool = False,
-                 uninterrupted_charging: bool = False, max_recompute: Optional[int] = 1):
+                 uninterrupted_charging: bool = False, max_recompute: Optional[int] = 1, battery: bool = False,
+                 transition_soc: float = 0.8, estimate_max_rate: bool = False, up_increment: float = 1.0, down_threshold: float = 1.0):
+        if not 0.0 < transition_soc < 1.0:
+            raise ValueError(f"transition_soc must be in (0, 1), not {transition_soc!r}")
+        if not up_increment > 0.0:
+            raise ValueError(f"up_increment must be > 0, not {up_increment!r}")
+        if not down_threshold >= 0.0:
+            raise ValueError(f"down_threshold must be >= 0, not {down_threshold!r}")
+        self.battery, self.transition_soc = bool(battery), float(transition_soc)
+        self.estimate_max_rate, self.up_increment, self.down_threshold = bool(estimate_max_rate), float(up_increment), float(down_threshold)
         if max_recompute is not None and not (isinstance(max_recompute, (int, np.integer)) and not isinstance(max_recompute, bool)
                                               and max_recompute >= 1):
             raise ValueError(f"max_recompute must be None or an integer >= 1, not {max_recompute!r}")
@@ -90,17 +134,22 @@ class FleetReplay:
         self.try_rate = np.array([min(self.info.min_pilot[i], period) for i in range(self.N)], dtype=np.float64)
         # an admitted EV's first-period minimum is its EVSE's try rate: the lb_zero promise holds only if every try is 0
         self.lb_zero = not (self.uninterrupted_charging and bool(np.any(self.try_rate > 0)))
-        cols = {k: [] for k in ("site", "station", "arr", "dep", "req", "maxrate")}
+        cols = {k: [] for k in ("site", "station", "arr", "dep", "req", "maxrate", "cap", "charge")}
         for s in range(n_sites):
             for d in range(days):
                 seed = seed0 + (site_offset + s) * days + d if days > 1 else seed0 + site_offset + s
-                for ev in synthetic_day(infra, seed, steps_per_day, period, mean_sessions):
+                evs = synthetic_day(infra, seed, steps_per_day, period, mean_sessions)
+                for ev in evs:
                     cols["site"].append(s)
                     cols["station"].append(ev.station)
                     cols["arr"].append(ev.arrival + d * steps_per_day)
                     cols["dep"].append(ev.departure + d * steps_per_day)
                     cols["req"].append(ev.requested)
                     cols["maxrate"].append(ev.max_rate)
+                if self.battery:
+                    cap, charge = synthetic_batteries(seed, [ev.requested for ev in evs])
+                    cols["cap"] += list(cap)
+                    cols["charge"] += list(charge)
         # EV table sorted by (day, site, station): a day is a contiguous slice (sessions never span midnight, so step t
         # only looks at its own day) and any active subset of it is grouped by site and ordered by EVSE row
         arr_all = np.array(cols["arr"], dtype=np.int64)
@@ -112,6 +161,11 @@ class FleetReplay:
         self.ev_req = np.array(cols["req"], dtype=np.float64)[order]
         self.ev_max = np.array(cols["maxrate"], dtype=np.float64)[order]
         self.ev_dlv = np.zeros_like(self.ev_req)
+        # batteries (kWh) and the rampdown estimate (A) per EV, None without
+        self.ev_cap = np.array(cols["cap"], dtype=np.float64)[order] if self.battery else None
+        self.ev_charge = np.array(cols["charge"], dtype=np.float64)[order] if self.battery else None
+        self.ev_ub = np.asarray(self.info.max_pilot, dtype=np.float64)[self.ev_station] if self.estimate_max_rate else None
+        self.rates: Optional[np.ndarray] = None  # each EVSE's current at the last step [n_sites, N]
         day = self.ev_arr // steps_per_day
         edges = np.searchsorted(day, np.arange(days + 1))
         self._day_slice = [slice(int(edges[d]), int(edges[d + 1])) for d in range(days)]
@@ -202,9 +256,18 @@ class FleetReplay:
         h["sess_start"] = np.zeros((B, S_), dtype=i32)
         h["min_rates"] = np.zeros(B * S_, dtype=f32)  # fixed length (one slot per possible session): the staging buffers are reused
         h["max_rates"] = np.zeros(B * S_, dtype=f32)
-        h["max_rates"][: len(idx)] = self.ev_max[idx]
+        h["max_rates"][: len(idx)] = self._max_rate(idx)
         h.update(self._objective_arrays(t, T))
         return h, idx, s, pos, n_sess
+
+    def _max_rate(self, idx):
+        """The maximum rate of the EVs idx as the solve sees it: their own, with estimate_max_rate cut to the estimate and
+        then raised to the minimum rate 0 where it fell below (what acb_preprocess_sessions does with the upper bounds)."""
+        if self.ev_ub is None:
+            return self.ev_max[idx]
+        ub, mx = self.ev_ub[idx], self.ev_max[idx]
+        m = np.where(ub < mx, ub, mx)
+        return np.where(m < 0.0, 0.0, m)
 
     def _admit(self, h, idx, s, pos):
         """apply_minimum_charging_rate of every site (what acb_admit_sessions does on the device): the greedy over the
@@ -221,7 +284,7 @@ class FleetReplay:
         rows, tries = np.zeros((B, S_), dtype=np.int32), np.zeros((B, S_))
         rows[s[cand], c_pos], tries[s[cand], c_pos] = st[cand], tr[cand]
         adm = engine.min_rate_admission(self.site, n_c, rows, tries)[s[cand], c_pos]
-        mn0, mx0 = np.zeros(len(idx)), self.ev_max[idx].copy()  # sessions left out keep their own limits (0, max rate)
+        mn0, mx0 = np.zeros(len(idx)), self._max_rate(idx).copy()  # sessions left out keep their own limits (0, max rate)
         lo = np.where(0.0 < tr[cand], tr[cand], 0.0)  # max(try, min_rates[0])
         mn0[cand] = np.where(adm, lo, 0.0)
         mx0[cand] = np.where(adm, np.where(mx0[cand] < lo, lo, mx0[cand]), 0.0)
@@ -305,9 +368,25 @@ class FleetReplay:
         # the simulator side: first-period pilots charge the EVs that are plugged in
         sl = self._day_slice[min(t // self.steps_per_day, self.days - 1)]
         present = np.nonzero((self.ev_arr[sl] <= t) & (t < self.ev_dep[sl]))[0] + sl.start
-        e = np.minimum(first[self.ev_site[present], self.ev_station[present]] * self._w_ev[present], self.ev_req[present] - self.ev_dlv[present])
-        self.ev_dlv[present] += np.maximum(e, 0.0)
-        self.prev_peak = np.maximum(self.prev_peak, first.sum(axis=1))
+        if self.battery or self.estimate_max_rate:
+            at = (self.ev_site[present], self.ev_station[present])
+            p, w, owed = first[at], self._w_ev[present], self.ev_req[present] - self.ev_dlv[present]
+            if self.battery:
+                a, e = battery_current(p, w, self.ev_max[present], self.ev_cap[present], self.ev_charge[present], owed, self.transition_soc)
+                self.ev_charge[present] += e
+            else:
+                a, e = p, np.maximum(np.minimum(p * w, owed), 0.0)
+            self.ev_dlv[present] += e
+            if self.estimate_max_rate:
+                self.ev_ub[present] = rampdown_update(self.ev_ub[present], p, a, self.up_increment, self.down_threshold)[0]
+            self.rates = np.zeros_like(first)
+            self.rates[at] = a
+        else:
+            e = np.minimum(first[self.ev_site[present], self.ev_station[present]] * self._w_ev[present], self.ev_req[present] - self.ev_dlv[present])
+            self.ev_dlv[present] += np.maximum(e, 0.0)
+            self.rates = first
+        # the site's peak: of the currents the batteries took (acb_fleet_apply_ev sums `rates` with ev_cap), else of the pilots
+        self.prev_peak = np.maximum(self.prev_peak, (self.rates if self.battery else first).sum(axis=1))
         self._prev = (idx_d, s_d, pos_d)
         self._state.reverse()
         self.recompute = rec
@@ -343,7 +422,7 @@ class FleetReplay:
                 rows = np.zeros((B, S_), dtype=np.int32)
                 rows[s, pos] = self.ev_station[idx]
             else:
-                mx = self.ev_max[idx]
+                mx = self._max_rate(idx)
             ramp[s, pos] = rem * 1000 / self.volt[self.ev_station[idx]] * (60 / self.period)
             max0[s, pos] = mx
             return engine.reallocate(self.site, 1, rates, h["n_sessions"], rows, h["sess_start"], ramp, max0)
@@ -391,7 +470,11 @@ class DeviceFleetReplay(FleetReplay):
 
     The admission puts the raw tables in arrival order but leaves `sess_ev` / `warm_mu` in the EV table's (station)
     order: they are indexed like the packed batch (warm_mu, out_mu), whose (EVSE, slot) order of a single-session site
-    is the station order whatever the slot order."""
+    is the station order whatever the slot order.
+
+    With `battery` or `estimate_max_rate` the fleet kernels are the _ev entry points (acb_fleet_ev: batteries, estimates,
+    the per-EVSE currents in `rates`), and with the estimate acb_preprocess_sessions caps each session's maximum rate
+    at its EV's bound between the active sessions and the admission."""
 
     def __init__(self, *a, **kw):
         super().__init__(*a, **kw)
@@ -405,7 +488,8 @@ class DeviceFleetReplay(FleetReplay):
                                             demand_charge=self.demand_charge, solver_options=opts, device=self.device, chunks=1,
                                             enforce_pilot_limit=False, quantize=self.pilot_mode != 0,
                                             reallocate=self.pilot_mode == _cabi.ACB_PILOTS_REALLOCATE,
-                                            uninterrupted_charging=self.uninterrupted_charging, skip_unabsorbable=True)
+                                            uninterrupted_charging=self.uninterrupted_charging, skip_unabsorbable=True,
+                                            estimate_max_rate=self.estimate_max_rate)
         if self._bac.Tp != self.Tp:
             raise ValueError(f"Tp = {self.Tp} is not a padded horizon of the solve path")
         self.site = self._bac.site
@@ -438,6 +522,19 @@ class DeviceFleetReplay(FleetReplay):
         if self._event_driven:  # (NULL last_solve: every site solves every step, column 0 applies)
             f.last_solve, f.recompute, f.shift = p(d["last_solve"]), p(d["recompute"]), p(d["shift"])
         self._fleet = f
+        self._fev = None  # batteries / estimates (acb_fleet_ev); None = the plain fleet kernels
+        if self.battery or self.estimate_max_rate:
+            e = _cabi.FleetEV()
+            d["rates"] = torch.zeros((self.n_sites, self.N), dtype=torch.float64, device=dev)
+            e.rates = p(d["rates"])
+            if self.battery:
+                d["cap"], d["charge"] = up(self.ev_cap, np.float64), up(self.ev_charge, np.float64)
+                e.ev_cap, e.ev_charge, e.transition_soc = p(d["cap"]), p(d["charge"]), self.transition_soc
+            if self.estimate_max_rate:
+                d["ub"] = up(self.ev_ub, np.float64)
+                e.ev_ub, e.up_increment, e.down_threshold = p(d["ub"]), self.up_increment, self.down_threshold
+                e.upper_bound = p(ch.dev_raw["upper_bound"])
+            self._fev = e
         self._state = [ch.new_warm_state(), ch.new_warm_state()]
         ch.lb_zero = self.lb_zero  # the synthetic EVs have no minimum rate of their own
         o = ch.objective
@@ -455,7 +552,11 @@ class DeviceFleetReplay(FleetReplay):
         ch.set_warm(dict(prev, mu=d["warm_mu"]) if self.warm_start and self._started else None, out, shift=1, had=d["had"],
                     shifts=d["shift"] if ev else None, mask=d["recompute"] if ev else None)
         o.prices = C.c_void_p(d["prices"].data_ptr() + 8 * t) if self._bac.need_prices else None
-        _cabi.check(L.acb_fleet_sessions(self.site.handle, C.byref(self._fleet), t, C.byref(ch.sessions), p(d["sess_ev"]), p(d["warm_mu"]), st), "acb_fleet_sessions")
+        fev = C.byref(self._fev) if self._fev is not None else None
+        _cabi.check(L.acb_fleet_sessions_ev(self.site.handle, C.byref(self._fleet), fev, t, C.byref(ch.sessions), p(d["sess_ev"]), p(d["warm_mu"]), st),
+                    "acb_fleet_sessions_ev")
+        if self.estimate_max_rate:  # max_rate <- min(max_rate, the EV's estimate), then the minimum rate wins
+            _cabi.check(L.acb_preprocess_sessions(self.site.handle, C.byref(ch.sessions), 0, p(ch.dev_raw["upper_bound"]), st), "acb_preprocess_sessions")
         if self.uninterrupted_charging:
             self._bac.admit(ch, st)
         _cabi.check(L.acb_pack_sessions(self.site.handle, C.byref(ch.sessions), C.byref(o), C.byref(ch.struct), p(ch.flags), st), "acb_pack_sessions")
@@ -464,13 +565,17 @@ class DeviceFleetReplay(FleetReplay):
             _cabi.check(L.acb_quantize_pilots(self.site.handle, self.pilot_mode, C.byref(ch.sessions), float(self.period), C.byref(ch.struct), p(ch.pilots), st),
                         "acb_quantize_pilots")
             ch.bind_pilots(True)
-        _cabi.check(L.acb_fleet_apply(self.site.handle, C.byref(self._fleet), t, float(self.period), C.byref(ch.struct), p(d["sess_ev"]),
-                                      p(d["first"]) if want_first else None, p(d["stats"]), st), "acb_fleet_apply")
+        _cabi.check(L.acb_fleet_apply_ev(self.site.handle, C.byref(self._fleet), fev, t, float(self.period), C.byref(ch.struct), p(d["sess_ev"]),
+                                         p(d["first"]) if want_first else None, p(d["stats"]), st), "acb_fleet_apply_ev")
         if self.pilot_mode:
             ch.bind_pilots(False)
         self._state.reverse()
         self._started = True
-        return d["first"].cpu().numpy() if want_first else None
+        if not want_first:
+            return None
+        first = d["first"].cpu().numpy()
+        self.rates = d["rates"].cpu().numpy() if "rates" in d else first
+        return first
 
     def run(self, t0: int = 0, t1: Optional[int] = None) -> FleetStats:
         for t in range(t0, self.steps if t1 is None else t1):
@@ -480,6 +585,10 @@ class DeviceFleetReplay(FleetReplay):
             raise ValueError("the device packer flagged the fleet's sessions (two sessions on one EVSE, or a session beyond the padded horizon)")
         self.ev_dlv = self._d["dlv"].cpu().numpy()
         self.prev_peak = self._d["prev_peak"].cpu().numpy()
+        if self.battery:
+            self.ev_charge = self._d["charge"].cpu().numpy()
+        if self.estimate_max_rate:
+            self.ev_ub = self._d["ub"].cpu().numpy()
         req = np.bincount(self.ev_site, weights=self.ev_req, minlength=self.n_sites)
         dlv = np.bincount(self.ev_site, weights=self.ev_dlv, minlength=self.n_sites)
         self.stats.delivered_frac = dlv / np.maximum(req, 1e-9)

@@ -26,7 +26,7 @@
  *                                                                 ...optimization.py:114-122, 200-218, 243-245, 363-408
  *   acb_preprocess_sessions / acb_min_rate_admission
  *                               acnportal preprocessing called at      adacharge/adacharge.py:141-150
- *   acb_fleet_sessions / acb_fleet_apply
+ *   acb_fleet_sessions / acb_fleet_apply (_ev: with batteries and the rampdown estimate)
  *                               the simulator side of a closed-loop step  adacharge/adacharge.py:18-39, 135-193
  *
  * Conventions: plain C, no exceptions; every function returns 0 on success or a
@@ -350,6 +350,34 @@ int acb_fleet_sessions(acb_site* site, const acb_fleet* fleet, int t, const acb_
  * only sites that solved update had, their EVs' multipliers and stats. */
 int acb_fleet_apply(acb_site* site, const acb_fleet* fleet, int t, double period, const acb_batch* batch, const int32_t* sess_ev,
                     double* first_pilots, double* stats, void* stream);
+
+/* Per-EV batteries and the rampdown max-rate estimate of a fleet replay (acb_fleet keeps its layout: these are a struct of
+ * their own, passed to the _ev entry points).  All pointers device.
+ * Battery (acnportal's stepwise Linear2StageBattery without noise, in amperes; this library's statement: DESIGN.md §8): a
+ * plugged-in EV e under pilot p on an EVSE of w kWh per A*period takes the current
+ *   a = 0 if p == 0, else min(p, ev_max) below transition_soc and min(p, (1 - soc) / (1 - transition_soc) * ev_max) from it
+ *   on (soc = charge / cap), cut to (cap - charge) / w where charge + a * w would pass cap, and at least 0;
+ * it receives de = max(min(a * w, requested - delivered), 0), added to ev_dlv and ev_charge.  float64, no contraction.
+ * Rampdown estimate (acnportal's SimpleRampdown): after every applied step where e is plugged in, if p - a > down_threshold
+ * then ev_ub[e] = a + up_increment.  acb_fleet_sessions_ev writes each slot's ev_ub into upper_bound, the table
+ * acb_preprocess_sessions takes. */
+typedef struct acb_fleet_ev {
+    const double* ev_cap;        /* [n_ev] battery capacity, kWh; NULL = ideal batteries (a = p) */
+    double* ev_charge;           /* [n_ev] state: battery charge, kWh (required with ev_cap) */
+    double transition_soc;       /* state of charge where the taper starts, in (0, 1) */
+    double* ev_ub;               /* [n_ev] state: estimated maximum rate, A; NULL = no estimate */
+    double up_increment;         /* A, > 0 */
+    double down_threshold;       /* A, >= 0 */
+    double* upper_bound;         /* [n_sites][S_max] written by acb_fleet_sessions_ev (with ev_ub): the slot's ev_ub, 0 in empty slots */
+    double* rates;               /* [n_sites][N] written by acb_fleet_apply_ev: each EVSE's current a, 0 where no EV is plugged in;
+                                  * required with ev_cap (prev_peak is then the largest sum of these) */
+} acb_fleet_ev;
+
+/* acb_fleet_sessions / acb_fleet_apply with batteries and the rampdown estimate; ev NULL = the plain entry points. */
+int acb_fleet_sessions_ev(acb_site* site, const acb_fleet* fleet, const acb_fleet_ev* ev, int t, const acb_sessions* sessions,
+                          int32_t* sess_ev, float* warm_mu, void* stream);
+int acb_fleet_apply_ev(acb_site* site, const acb_fleet* fleet, const acb_fleet_ev* ev, int t, double period, const acb_batch* batch,
+                       const int32_t* sess_ev, double* first_pilots, double* stats, void* stream);
 
 const char* acb_last_error(void);
 int acb_version(void);
