@@ -258,31 +258,13 @@ class BatchedAdaptiveCharging:
                 d[...] = a[ch.lo:ch.hi]
 
     def enqueue(self, ch: _Chunk, from_device_raw=False, events=None):
-        """H2D of the raw arrays (unless they are already on the device), pack, solve, quantise (if asked), D2H — on the chunk's stream.
-        `events`: a list that receives a (start, end) pair of CUDA events around the solve launch(es)."""
-        L = _cabi.lib()
-        st = C.c_void_p(ch.stream.cuda_stream)
+        """H2D of the raw arrays (unless they are already on the device), `_launch`, D2H — on the chunk's stream."""
         with torch.cuda.stream(ch.stream):
             if not from_device_raw:
                 for k, t in ch.host.items():
                     ch.dev_raw[k].copy_(t, non_blocking=True)
             ch.flags.zero_()
-            if self.enforce_pilot_limit or self.estimate_max_rate:
-                _cabi.check(L.acb_preprocess_sessions(self.site.handle, C.byref(ch.sessions), int(self.enforce_pilot_limit),
-                                                      engine._ptr(ch.dev_raw.get("upper_bound")), st), "acb_preprocess_sessions")
-            if self.uninterrupted_charging:
-                self.admit(ch, st)
-            _cabi.check(L.acb_pack_sessions(self.site.handle, C.byref(ch.sessions), C.byref(ch.objective), C.byref(ch.struct), engine._ptr(ch.flags), st), "acb_pack_sessions")
-            if events is not None:
-                ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
-                ev[0].record(ch.stream)
-            ch.solve(self.options, st)
-            if events is not None:
-                ev[1].record(ch.stream)
-                events.append(ev)
-            if self.pilot_mode:
-                _cabi.check(L.acb_quantize_pilots(self.site.handle, self.pilot_mode, C.byref(ch.sessions), float(self.period), C.byref(ch.struct),
-                                                  engine._ptr(ch.pilots), st), "acb_quantize_pilots")
+            self._launch(ch, ch.stream, events)
             if not from_device_raw:
                 self.host_pilots[ch.lo:ch.hi].copy_(ch.pilots, non_blocking=True)
                 self.host_status[ch.lo:ch.hi].copy_(ch.status, non_blocking=True)
@@ -290,6 +272,30 @@ class BatchedAdaptiveCharging:
                 self.host_T[ch.lo:ch.hi].copy_(ch.packed["T"], non_blocking=True)
                 self.host_stats[ch.lo:ch.hi].copy_(ch.stats, non_blocking=True)
                 ch.flags_host.copy_(ch.flags, non_blocking=True)
+
+    def _launch(self, ch: _Chunk, stream: torch.cuda.Stream, events=None):
+        """Enqueue on `stream` what turns the chunk's raw device tables into pilots: preprocess (pilot limit, upper-bound
+        estimate), admit (uninterrupted charging), pack, solve, quantise (quantize).  The packer ORs its flags into
+        `ch.flags`, which this leaves as it finds them (the device fleet replay accumulates them over a run).
+        `events`: a list that receives a (start, end) pair of CUDA events around the solve launch(es)."""
+        L = _cabi.lib()
+        st = C.c_void_p(stream.cuda_stream)
+        if self.enforce_pilot_limit or self.estimate_max_rate:
+            _cabi.check(L.acb_preprocess_sessions(self.site.handle, C.byref(ch.sessions), int(self.enforce_pilot_limit),
+                                                  engine._ptr(ch.dev_raw.get("upper_bound")), st), "acb_preprocess_sessions")
+        if self.uninterrupted_charging:
+            self.admit(ch, st)
+        _cabi.check(L.acb_pack_sessions(self.site.handle, C.byref(ch.sessions), C.byref(ch.objective), C.byref(ch.struct), engine._ptr(ch.flags), st), "acb_pack_sessions")
+        if events is not None:
+            ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
+            ev[0].record(stream)
+        ch.solve(self.options, st)
+        if events is not None:
+            ev[1].record(stream)
+            events.append(ev)
+        if self.pilot_mode:
+            _cabi.check(L.acb_quantize_pilots(self.site.handle, self.pilot_mode, C.byref(ch.sessions), float(self.period), C.byref(ch.struct),
+                                              engine._ptr(ch.pilots), st), "acb_quantize_pilots")
 
     def admit(self, ch: _Chunk, stream):
         """Enqueue acb_admit_sessions on the chunk's raw tables (in place: arrival order, first-period limits)."""

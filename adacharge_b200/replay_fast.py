@@ -23,6 +23,7 @@ of them with no data-path collective; `summary()` returns what `gather_summaries
 """
 from __future__ import annotations
 
+import ctypes as C
 import time
 from dataclasses import dataclass, field
 from typing import Dict, List, Optional
@@ -74,7 +75,7 @@ class FleetStats:
     peak_kw: Optional[np.ndarray] = None
 
 
-class FleetReplay:
+class _FleetReplayBase:
     """`n_sites` copies of one site, `days` seeded days of EVs each (day d of site s is
     `synthetic_day(seed0 + s * days + d)` shifted by d * steps_per_day periods).  `quantize` / `reallocate` are
     AdaptiveSchedulingAlgorithm's flags: the EVs are charged with pilots from each EVSE's allowable set.
@@ -91,7 +92,9 @@ class FleetReplay:
     those currents.  `rates` holds each EVSE's current of the last step.  `estimate_max_rate`: each EV keeps acnportal's
     SimpleRampdown estimate `ev_ub` (from its EVSE's max_pilot; `rampdown_update` with `up_increment` and
     `down_threshold`), and every solve caps the session's maximum rate at it (apply_upper_bound_estimate).  Without
-    `battery` every EV takes its pilot and the estimate never moves."""
+    `battery` every EV takes its pilot and the estimate never moves.  Both replays take `step(t, want_first=True)` (it
+    returns the applied first-period pilots [n_sites, N]) and `state()`.  FleetReplay advances `ev_dlv`, `prev_peak`,
+    `ev_charge`, `ev_ub` and `rates` in place; DeviceFleetReplay copies them back at `state()` (`rates`: at want_first)."""
 
     def __init__(self, infra: Dict, objective: List[ObjectiveComponent], n_sites: int, steps_per_day: int = 288, days: int = 1,
                  period: float = 5, prices: Optional[np.ndarray] = None, demand_charge: float = 15.51, seed0: int = 0,
@@ -118,7 +121,7 @@ class FleetReplay:
         self.warm_start, self.device, self.Tp = warm_start, device, Tp
         # closed loop: the sunk demand charge w * prev_peak is a constant of every step's objective and can cancel the
         # energy term, so the gap is taken relative to the terms' magnitude; a stalled instance stops after 40 checks
-        self.options = _cabi.default_options(**{**REPLAY_SOLVER_DEFAULTS, **(solver_options or {})})
+        self.solver_options = {**REPLAY_SOLVER_DEFAULTS, **(solver_options or {})}
         from .generators import sce_tou_prices
 
         day_prices = sce_tou_prices(steps_per_day, period) if prices is None else np.asarray(prices, dtype=float)
@@ -160,26 +163,53 @@ class FleetReplay:
         self.ev_dep = np.array(cols["dep"], dtype=np.int64)[order]
         self.ev_req = np.array(cols["req"], dtype=np.float64)[order]
         self.ev_max = np.array(cols["maxrate"], dtype=np.float64)[order]
-        self.ev_dlv = np.zeros_like(self.ev_req)
         # batteries (kWh) and the rampdown estimate (A) per EV, None without
         self.ev_cap = np.array(cols["cap"], dtype=np.float64)[order] if self.battery else None
         self.ev_charge = np.array(cols["charge"], dtype=np.float64)[order] if self.battery else None
         self.ev_ub = np.asarray(self.info.max_pilot, dtype=np.float64)[self.ev_station] if self.estimate_max_rate else None
-        self.rates: Optional[np.ndarray] = None  # each EVSE's current at the last step [n_sites, N]
+        self.ev_dlv = np.zeros_like(self.ev_req)
+        self.prev_peak = np.zeros(n_sites)  # A
+        self.rates: Optional[np.ndarray] = None  # each EVSE's current at the last step [n_sites, N] (the pilots without batteries)
         day = self.ev_arr // steps_per_day
         edges = np.searchsorted(day, np.arange(days + 1))
         self._day_slice = [slice(int(edges[d]), int(edges[d + 1])) for d in range(days)]
         self._w_ev = self.volt[self.ev_station] * period / 1e3 / 60  # kWh per A-period of each EV's EVSE
-        self.prev_peak = np.zeros(n_sites)  # A
-        self.last_solve = np.full(n_sites, -1, dtype=np.int64)  # step of each site's last solve
-        self.had = np.zeros(n_sites, dtype=np.int32)  # 1 if the site had sessions at its last solve
-        self.recompute: Optional[np.ndarray] = None  # the last step's re-solve decision per site
+        self.stats = FleetStats()
+
+    def run(self, t0: int = 0, t1: Optional[int] = None) -> FleetStats:
+        for t in range(t0, self.steps if t1 is None else t1):
+            self.step(t, want_first=False)
+        s = self.state()
+        req = np.bincount(self.ev_site, weights=self.ev_req, minlength=self.n_sites)
+        dlv = np.bincount(self.ev_site, weights=s["ev_dlv"], minlength=self.n_sites)
+        self.stats.delivered_frac = dlv / np.maximum(req, 1e-9)
+        self.stats.peak_kw = s["prev_peak"] * self.volt[0] / 1000
+        return self.stats
+
+
+class FleetReplay(_FleetReplayBase):
+    """The simulator side of the step on the host, in numpy: the reference DeviceFleetReplay is checked against."""
+
+    def __init__(self, *a, **kw):
+        super().__init__(*a, **kw)
+        B = self.n_sites
+        self.options = _cabi.default_options(**self.solver_options)
+        self.last_solve = np.full(B, -1, dtype=np.int64)  # step of each site's last solve
+        self.had = np.zeros(B, dtype=np.int32)  # 1 if the site had sessions at its last solve
+        self.recompute = np.zeros(B, dtype=bool)  # the last step's re-solve decision per site
         self.site: Optional[engine.Site] = None
         self._prev = None  # EV index / site / position of the previous step's sessions
         self._sched: Optional[torch.Tensor] = None  # each site's pilots from its last solve [B, N, Tp]
         self._pb: Optional[engine.PackedBatch] = None  # one batch object for the whole replay (refilled every step)
         self._state = None  # two sets of warm-state tensors: a step reads the previous step's set and writes the other
-        self.stats = FleetStats()
+
+    def state(self) -> Dict[str, Optional[np.ndarray]]:
+        """The simulator state as numpy copies, the same keys on both replays: `ev_dlv` (kWh per EV), `prev_peak` (A per
+        site), `recompute` (bool per site: re-solved at the last step), `status` (per site, of its last solve; None
+        before the first step), `ev_charge` (with battery), `ev_ub` (with estimate_max_rate), `rates` (with either)."""
+        live = dict(ev_dlv=self.ev_dlv, prev_peak=self.prev_peak, recompute=self.recompute, ev_charge=self.ev_charge, ev_ub=self.ev_ub,
+                    rates=self.rates if self.battery or self.estimate_max_rate else None)
+        return dict({k: None if v is None else v.copy() for k, v in live.items()}, status=None if self._pb is None else self._pb.status.cpu().numpy())
 
     # ------------------------------------------------------------------ packing
     def _objective_arrays(self, t: int, T: np.ndarray) -> Dict[str, np.ndarray]:
@@ -314,7 +344,7 @@ class FleetReplay:
         return (self.last_solve < 0) | ev | ((mr > 0) & (since >= mr)), since
 
     # ------------------------------------------------------------------ one control step
-    def step(self, t: int):
+    def step(self, t: int, want_first: bool = True):
         t0 = time.perf_counter()
         rec, since = self._recompute(t)
         h, idx, s, pos, n_sess = self._pack(t)
@@ -400,7 +430,7 @@ class FleetReplay:
         st_.solved_sites.append(int(sol.sum()))
         st_.device_ms.append(ev0.elapsed_time(ev1))
         st_.host_ms.append((t1 - t0 + time.perf_counter() - t2) * 1e3)
-        return first
+        return first if want_first else None
 
     def _project(self, rates, h, idx, s, pos):
         """The pilots of the step's schedule (pp.py:77-118, 189-258 on the device)."""
@@ -439,15 +469,6 @@ class FleetReplay:
         mu[s_d, pos_d] = mu_ev[idx_d]
         return dict(prev, mu=mu)
 
-    def run(self, t0: int = 0, t1: Optional[int] = None) -> FleetStats:
-        for t in range(t0, self.steps if t1 is None else t1):
-            self.step(t)
-        req = np.bincount(self.ev_site, weights=self.ev_req, minlength=self.n_sites)
-        dlv = np.bincount(self.ev_site, weights=self.ev_dlv, minlength=self.n_sites)
-        self.stats.delivered_frac = dlv / np.maximum(req, 1e-9)
-        self.stats.peak_kw = self.prev_peak * self.volt[0] / 1000
-        return self.stats
-
     def summary(self) -> Dict[str, float]:
         s = self.stats
         n = max(len(s.device_ms), 1)
@@ -457,35 +478,27 @@ class FleetReplay:
                     iters_max=float(max(s.iters_max, default=0)))
 
 
-class DeviceFleetReplay(FleetReplay):
-    """FleetReplay with the simulator side of the control step on the device as well (SURVEY.md §8(f) N1): the EV table,
-    the energy delivered, the previous peaks and the per-EV warm-start multipliers stay in device arrays; a step is four
-    launches on one stream -- active sessions (acb_fleet_sessions), packing (acb_pack_sessions), the warm-started solve
-    whose prologue reads each site's last state t - last_solve columns ahead (acb_solve_batch_masked's warm_shifts) and whose epilogue
-    projects the pilots, and the simulator update (acb_fleet_apply) -- with no host synchronisation between steps.  The
-    re-solve decision (max_recompute) is made by acb_fleet_sessions and is the solve's solve_mask.  Quantised pilots
-    take a fifth launch (acb_quantize_pilots) between the solve and the update, uninterrupted charging one more
-    (acb_admit_sessions) between the active sessions and the packing.  Same schedules, bit for bit, as FleetReplay
-    (tests/test_gpu_replay.py, tests/test_gpu_uninterrupted.py).
+class DeviceFleetReplay(_FleetReplayBase):
+    """The simulator side of the control step on the device as well (SURVEY.md §8(f) N1): the EV table, the energy
+    delivered, the previous peaks and the per-EV warm-start multipliers stay in device arrays.  A step is, on the current
+    stream with no host synchronisation: the active sessions and the re-solve decision (acb_fleet_sessions), the launch
+    sequence of BatchedAdaptiveCharging (`_launch`: preprocessing, admission, packing, the solve -- masked by the
+    decision, each site warm-started from its own last state t - last_solve columns ahead -- and quantised pilots, as
+    configured), and the simulator update (acb_fleet_apply).  Same pilots and `state()`, bit for bit, as FleetReplay.
 
     The admission puts the raw tables in arrival order but leaves `sess_ev` / `warm_mu` in the EV table's (station)
     order: they are indexed like the packed batch (warm_mu, out_mu), whose (EVSE, slot) order of a single-session site
-    is the station order whatever the slot order.
-
-    With `battery` or `estimate_max_rate` the fleet kernels are the _ev entry points (acb_fleet_ev: batteries, estimates,
-    the per-EVSE currents in `rates`), and with the estimate acb_preprocess_sessions caps each session's maximum rate
-    at its EV's bound between the active sessions and the admission."""
+    is the station order whatever the slot order.  With `battery` or `estimate_max_rate` the fleet kernels are the _ev
+    entry points (acb_fleet_ev: batteries, estimates, the per-EVSE currents in `rates`); with the estimate the
+    preprocessing caps each session's maximum rate at its EV's bound."""
 
     def __init__(self, *a, **kw):
         super().__init__(*a, **kw)
-        import ctypes as C
-
         from .batched import BatchedAdaptiveCharging
 
         dev = torch.device("cuda", engine._dev_index(self.device))
-        opts = {**REPLAY_SOLVER_DEFAULTS, **(kw.get("solver_options") or {})}
         self._bac = BatchedAdaptiveCharging(self.objective, self.info, self.period, batch=self.n_sites, max_sessions=self.N, horizon=self.Tp,
-                                            demand_charge=self.demand_charge, solver_options=opts, device=self.device, chunks=1,
+                                            demand_charge=self.demand_charge, solver_options=self.solver_options, device=self.device, chunks=1,
                                             enforce_pilot_limit=False, quantize=self.pilot_mode != 0,
                                             reallocate=self.pilot_mode == _cabi.ACB_PILOTS_REALLOCATE,
                                             uninterrupted_charging=self.uninterrupted_charging, skip_unabsorbable=True,
@@ -493,8 +506,7 @@ class DeviceFleetReplay(FleetReplay):
         if self._bac.Tp != self.Tp:
             raise ValueError(f"Tp = {self.Tp} is not a padded horizon of the solve path")
         self.site = self._bac.site
-        ch = self._bac.chunks[0]
-        self._ch = ch
+        self._ch = ch = self._bac.chunks[0]
         up = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a.astype(dt))).to(dev)  # noqa: E731
         n_ev = len(self.ev_req)
         self._d = dict(
@@ -541,29 +553,21 @@ class DeviceFleetReplay(FleetReplay):
         o.prev_peak = p(d["prev_peak"])
         o.prices_stride = 0  # one price vector for the whole fleet, read from the current period on
         self._started = False
-        self._C = C
 
     def step(self, t: int, want_first: bool = True):
-        C, L, ch, d, p = self._C, _cabi.lib(), self._ch, self._d, engine._ptr
-        st = C.c_void_p(torch.cuda.current_stream(self._bac.device).cuda_stream)
-        o = ch.objective
+        L, ch, d, p = _cabi.lib(), self._ch, self._d, engine._ptr
+        stream = torch.cuda.current_stream(self._bac.device)
+        st = C.c_void_p(stream.cuda_stream)
         prev, out = self._state
         ev = self._event_driven
         ch.set_warm(dict(prev, mu=d["warm_mu"]) if self.warm_start and self._started else None, out, shift=1, had=d["had"],
                     shifts=d["shift"] if ev else None, mask=d["recompute"] if ev else None)
-        o.prices = C.c_void_p(d["prices"].data_ptr() + 8 * t) if self._bac.need_prices else None
+        ch.objective.prices = C.c_void_p(d["prices"].data_ptr() + 8 * t) if self._bac.need_prices else None
         fev = C.byref(self._fev) if self._fev is not None else None
         _cabi.check(L.acb_fleet_sessions_ev(self.site.handle, C.byref(self._fleet), fev, t, C.byref(ch.sessions), p(d["sess_ev"]), p(d["warm_mu"]), st),
                     "acb_fleet_sessions_ev")
-        if self.estimate_max_rate:  # max_rate <- min(max_rate, the EV's estimate), then the minimum rate wins
-            _cabi.check(L.acb_preprocess_sessions(self.site.handle, C.byref(ch.sessions), 0, p(ch.dev_raw["upper_bound"]), st), "acb_preprocess_sessions")
-        if self.uninterrupted_charging:
-            self._bac.admit(ch, st)
-        _cabi.check(L.acb_pack_sessions(self.site.handle, C.byref(ch.sessions), C.byref(o), C.byref(ch.struct), p(ch.flags), st), "acb_pack_sessions")
-        ch.solve(self._bac.options, st)
+        self._bac._launch(ch, stream)
         if self.pilot_mode:  # the solve skipped the continuous projection (batch.pilots NULL); acb_fleet_apply reads batch.pilots
-            _cabi.check(L.acb_quantize_pilots(self.site.handle, self.pilot_mode, C.byref(ch.sessions), float(self.period), C.byref(ch.struct), p(ch.pilots), st),
-                        "acb_quantize_pilots")
             ch.bind_pilots(True)
         _cabi.check(L.acb_fleet_apply_ev(self.site.handle, C.byref(self._fleet), fev, t, float(self.period), C.byref(ch.struct), p(d["sess_ev"]),
                                          p(d["first"]) if want_first else None, p(d["stats"]), st), "acb_fleet_apply_ev")
@@ -577,23 +581,18 @@ class DeviceFleetReplay(FleetReplay):
         self.rates = d["rates"].cpu().numpy() if "rates" in d else first
         return first
 
-    def run(self, t0: int = 0, t1: Optional[int] = None) -> FleetStats:
-        for t in range(t0, self.steps if t1 is None else t1):
-            self.step(t, want_first=False)
+    def state(self) -> Dict[str, Optional[np.ndarray]]:
+        """FleetReplay.state, copied back (into the attributes too) once the steps enqueued so far, on any stream, have
+        finished.  Raises if the device packer flagged a step's sessions (two on one EVSE, or one beyond the padded horizon)."""
         torch.cuda.synchronize(self._bac.device)
         if int(self._ch.flags.cpu()[0]) != 0:
             raise ValueError("the device packer flagged the fleet's sessions (two sessions on one EVSE, or a session beyond the padded horizon)")
-        self.ev_dlv = self._d["dlv"].cpu().numpy()
-        self.prev_peak = self._d["prev_peak"].cpu().numpy()
-        if self.battery:
-            self.ev_charge = self._d["charge"].cpu().numpy()
-        if self.estimate_max_rate:
-            self.ev_ub = self._d["ub"].cpu().numpy()
-        req = np.bincount(self.ev_site, weights=self.ev_req, minlength=self.n_sites)
-        dlv = np.bincount(self.ev_site, weights=self.ev_dlv, minlength=self.n_sites)
-        self.stats.delivered_frac = dlv / np.maximum(req, 1e-9)
-        self.stats.peak_kw = self.prev_peak * self.volt[0] / 1000
-        return self.stats
+        d = self._d
+        get = lambda k: d[k].cpu().numpy() if k in d else None  # noqa: E731
+        self.ev_dlv, self.prev_peak, self.ev_charge, self.ev_ub = get("dlv"), get("prev_peak"), get("charge"), get("ub")
+        rec = d["recompute"].cpu().numpy() != 0 if self._event_driven else np.ones(self.n_sites, dtype=bool)  # (else it is not bound)
+        return dict(ev_dlv=self.ev_dlv, prev_peak=self.prev_peak, recompute=rec, status=self._ch.status.cpu().numpy() if self._started else None,
+                    ev_charge=self.ev_charge, ev_ub=self.ev_ub, rates=get("rates"))
 
     def summary(self) -> Dict[str, float]:
         s = self._d["stats"].cpu().numpy()

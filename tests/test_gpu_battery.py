@@ -16,9 +16,9 @@ from adacharge_b200.generators import caltech_acn_infrastructure, three_phase_ba
 from adacharge_b200.interface import SessionInfo
 from adacharge_b200.replay import EV
 from adacharge_b200.replay_fast import DeviceFleetReplay, FleetReplay
+from tests.replay_checks import BENCH, assert_as_good_as_cold_oracle, device_equals_host
 
 pytestmark = pytest.mark.gpu
-BENCH = [ab.ObjectiveComponent(ab.tou_energy_cost), ab.ObjectiveComponent(ab.total_energy, 0.3), ab.ObjectiveComponent(ab.demand_charge, 1 / 30)]
 STEPS = list(range(60, 150)) + list(range(288 + 80, 288 + 110))
 
 
@@ -28,27 +28,20 @@ def _fleet(**kw):
 
 
 def _dev_vs_host(steps, **kw):
-    infra = caltech_acn_infrastructure()
-    host, dev = FleetReplay(infra, BENCH, **_fleet(**kw)), DeviceFleetReplay(infra, BENCH, **_fleet(**kw))
-    taper = fired = 0
-    for t in steps:
-        ub0 = None if host.ev_ub is None else host.ev_ub.copy()
-        a = host.step(t)
-        b = dev.step(t, want_first=True)
-        np.testing.assert_array_equal(a, b, err_msg=f"applied pilots at step {t}")
-        np.testing.assert_array_equal(host.rates, dev.rates, err_msg=f"per-EVSE currents at step {t}")
-        if host._event_driven:
-            np.testing.assert_array_equal(host.recompute.astype(np.int32), dev._d["recompute"].cpu().numpy(), err_msg=f"recompute at step {t}")
-        taper += int((host.rates < a).sum())
-        if ub0 is not None:
-            fired += int((host.ev_ub != ub0).sum())
-    dev.run(0, 0)
-    for k in ("ev_dlv", "ev_charge", "ev_ub", "prev_peak"):
-        if getattr(host, k) is not None:
-            np.testing.assert_array_equal(getattr(dev, k), getattr(host, k), err_msg=k)
-    s = dev.summary()
-    assert s["solves"] == sum(host.stats.solved_sites) and s["unsolved"] == sum(host.stats.unsolved)
-    return host, taper, fired
+    """device_equals_host on the fleet, counting the EVSE-steps where a battery took less than its pilot and the
+    EV-steps where the estimate moved."""
+    n, last = dict(taper=0, fired=0), {}
+
+    def on_step(t, host, dev, first):
+        s = host.state()
+        n["taper"] += int((s["rates"] < first).sum())
+        if s["ev_ub"] is not None:
+            before = last.get("ub", np.asarray(host.info.max_pilot, dtype=np.float64)[host.ev_station])  # (the estimates start at max_pilot)
+            n["fired"] += int((s["ev_ub"] != before).sum())
+            last["ub"] = s["ev_ub"]
+
+    host, _ = device_equals_host(caltech_acn_infrastructure(), BENCH, steps, on_step, **_fleet(**kw))
+    return host, n["taper"], n["fired"]
 
 
 @pytest.mark.parametrize("max_recompute", [1, None])
@@ -68,16 +61,18 @@ def test_device_replay_equals_host_replay_with_flags(require_gpu, kw):
 
 
 def _same_as_default(cls, steps, **kw):
+    """The replay with kw against the default one; returns it and its final state."""
     infra = caltech_acn_infrastructure()
     a, b = cls(infra, BENCH, **_fleet()), cls(infra, BENCH, **_fleet(**kw))
     for t in steps:
-        first = b.step(t) if cls is FleetReplay else b.step(t, want_first=True)
-        np.testing.assert_array_equal(a.step(t) if cls is FleetReplay else a.step(t, want_first=True), first, err_msg=f"step {t}")
-        np.testing.assert_array_equal(b.rates, np.where(b.rates > 0, first, 0.0), err_msg=f"currents at step {t}")
-    a.run(0, 0), b.run(0, 0)
-    np.testing.assert_array_equal(a.ev_dlv, b.ev_dlv)
-    np.testing.assert_array_equal(a.prev_peak, b.prev_peak)
-    return b
+        first = b.step(t)
+        np.testing.assert_array_equal(a.step(t), first, err_msg=f"step {t}")
+        rates = b.state()["rates"]
+        np.testing.assert_array_equal(rates, np.where(rates > 0, first, 0.0), err_msg=f"currents at step {t}")
+    sa, sb = a.state(), b.state()
+    for k in ("ev_dlv", "prev_peak"):
+        np.testing.assert_array_equal(sa[k], sb[k], err_msg=k)
+    return b, sb
 
 
 @pytest.mark.parametrize("cls", [FleetReplay, DeviceFleetReplay])
@@ -85,15 +80,15 @@ def test_huge_batteries_are_the_default_replay(require_gpu, monkeypatch, cls):
     """Batteries that never reach their transition (a == p, stated in amperes) and an estimate that therefore never fires:
     the default replay bit for bit."""
     monkeypatch.setattr(replay_fast, "synthetic_batteries", lambda seed, req: (np.full(len(req), 1e9), np.zeros(len(req))))
-    b = _same_as_default(cls, STEPS[:60], battery=True, estimate_max_rate=True)
-    np.testing.assert_array_equal(b.ev_ub, np.asarray(b.info.max_pilot)[b.ev_station])
-    assert (b.ev_charge == b.ev_dlv).all()
+    b, s = _same_as_default(cls, STEPS[:60], battery=True, estimate_max_rate=True)
+    np.testing.assert_array_equal(s["ev_ub"], np.asarray(b.info.max_pilot)[b.ev_station])
+    assert (s["ev_charge"] == s["ev_dlv"]).all()
 
 
 @pytest.mark.parametrize("cls", [FleetReplay, DeviceFleetReplay])
 def test_estimate_without_batteries_is_a_no_op(require_gpu, cls):
-    b = _same_as_default(cls, STEPS[:40], estimate_max_rate=True)
-    np.testing.assert_array_equal(b.ev_ub, np.asarray(b.info.max_pilot)[b.ev_station])
+    b, s = _same_as_default(cls, STEPS[:40], estimate_max_rate=True)
+    np.testing.assert_array_equal(s["ev_ub"], np.asarray(b.info.max_pilot)[b.ev_station])
 
 
 # ---------------------------------------------------------------------------------------------------- semantics
@@ -110,35 +105,35 @@ def test_estimate_caps_the_next_solve(require_gpu, monkeypatch):
     dev, host = _one_ev(monkeypatch, True)
     bound, lowered = float(dev.info.max_pilot[5]), False  # the estimate starts at the EVSE's max_pilot
     for t in range(10, 30):
-        p = dev.step(t, want_first=True)[0, 5]
+        p = dev.step(t)[0, 5]
         np.testing.assert_array_equal(host.step(t)[0, 5], p)
         mx = dev._ch.dev_raw["max_rate"].cpu().numpy()[0, 0]  # the session's maximum rate after the preprocessing
         assert mx == min(32.0, bound), (t, mx, bound)
         if lowered:  # (the solve takes the bound rounded to float32)
             assert p <= np.float32(bound), (t, bound, p)
-        a = dev.rates[0, 5]
+        s = dev.state()
+        a = s["rates"][0, 5]
         assert a == host.rates[0, 5]
         if p - a > 1.0:
             bound, lowered = a + 1.0, True
-        assert dev._d["ub"].cpu().numpy()[0] == bound == host.ev_ub[0]
+        assert s["ev_ub"][0] == bound == host.ev_ub[0]
     assert bound < 9.0  # deep in the taper: the EV takes at most (1 - 0.95) / 0.2 * 32 = 8 A
 
 
 def test_without_the_estimate_the_pilot_stays_above_the_current(require_gpu, monkeypatch):
     dev, host = _one_ev(monkeypatch, False)
     for t in range(10, 30):
-        p = dev.step(t, want_first=True)[0, 5]
+        p = dev.step(t)[0, 5]
         np.testing.assert_array_equal(host.step(t)[0, 5], p)
         assert dev._ch.dev_raw["max_rate"].cpu().numpy()[0, 0] == 32.0
-        assert p > dev.rates[0, 5] + 1.0, (t, p, dev.rates[0, 5])
+        a = dev.state()["rates"][0, 5]
+        assert p > a + 1.0, (t, p, a)
 
 
 # ---------------------------------------------------------------------------------------------------- warm starts
 def test_lowered_bounds_match_a_cold_oracle_solve(require_gpu):
     """Warm-started solves where the estimate lowered some session's maximum rate since the site's previous solve are
     ordinary MPC instances: the schedule is as good as a cold float64 oracle solve of the same step."""
-    from oracle import mpc
-
     spec = [("tou_energy_cost", 1, {}), ("total_energy", 0.3, {}), ("demand_charge", 1 / 30, {})]
     obj = [ab.ObjectiveComponent(getattr(ab, n), c, k) for n, c, k in spec]
     infra = three_phase_balanced_network(3, 30)
@@ -156,35 +151,15 @@ def test_lowered_bounds_match_a_cold_oracle_solve(require_gpu):
         rp.step(t)
         last_mx[idx] = mx
         R = rp._pb.rates.cpu().numpy().astype(np.float64)
-        st = rp._pb.status.cpu().numpy()
+        st = rp.state()["status"]
         for b in range(rp.n_sites):
             if lowered[b] and had[b] and n_sess[b] > 0 and len(cases) < 40:
                 T = max(x.arrival_offset + x.remaining_time for x in sess[b])
                 cases.append((t, b, sess[b], float(peak[b]), R[b][:, :T], int(st[b])))
-    worst, compared, skipped = 0.0, 0, 0
-    for t, b, sess, prev_peak, R, status in cases:
-        assert status == 0, (t, b, status)
-        iface = ab.TestingInterface({"active_sessions": [], "infrastructure_info": infra, "current_time": t, "period": 15,
-                                     "prices": rp.prices, "demand_charge": rp.demand_charge, "prev_peak": prev_peak})
-        I = iface.infrastructure_info()
-        Ro = None
-        for ts in (1.0, 100.0):
-            try:
-                Ro = mpc.solve_mpc(spec, sess, I, iface, "SOC", False, None, prev_peak, tol_scale=ts)
-                break
-            except mpc.OracleInfeasible:
-                pass
-        if Ro is None:
-            skipped += 1
-            continue
-        compared += 1
-        f, fo = (mpc.evaluate_objective(X, spec, I, iface, sess, prev_peak) for X in (R, Ro))
-        mag = sum(abs(mpc.evaluate_objective(Ro, [o], I, iface, sess, prev_peak)) for o in spec)
-        assert abs(f - fo) <= 1e-4 * max(abs(fo), mag) + 1e-7, (t, b, f, fo, mag)
-        worst = max(worst, abs(f - fo) / max(abs(fo), mag))
-        v = mpc.violations(R, sess, I, iface)
-        # a lowered bound (a + up_increment) reaches the solve rounded to float32: the rates keep that bound exactly
-        f32_up = max(max(float(np.float32(x.max_rates[0])) - float(x.max_rates[0]), 0.0) for x in sess)
-        assert v["infrastructure_rel"] <= 1e-5 and v["lb"] <= 0 and v["ub"] <= f32_up and v["energy"] <= 1e-4, (t, b, v, f32_up)
+
+    def f32_up(sess):  # a lowered bound (a + up_increment) reaches the solve rounded to float32: the rates keep that bound exactly
+        return max(max(float(np.float32(x.max_rates[0])) - float(x.max_rates[0]), 0.0) for x in sess)
+
+    compared, skipped, worst = assert_as_good_as_cold_oracle(cases, spec, infra, 15, rp.prices, rp.demand_charge, ub_tol=f32_up)
     assert compared >= 20 and skipped <= 3, (len(cases), compared, skipped)
     print(f"{compared} warm-started solves with lowered bounds compared, worst objective error {worst:.1e} of the term scale")

@@ -12,6 +12,7 @@ from adacharge_b200 import _cabi, engine
 from adacharge_b200.batched import BatchedAdaptiveCharging, sessions_to_arrays
 from adacharge_b200.generators import caltech_acn_infrastructure, config_c2, config_c5, hierarchical_three_phase_network, session_generator
 from oracle import postprocessing as opp
+from tests.replay_checks import device_equals_host
 
 pytestmark = pytest.mark.gpu
 
@@ -153,27 +154,20 @@ def test_batched_reallocation_config_c5(require_gpu):
 
 
 def test_device_fleet_replay_quantized_equals_host(require_gpu):
-    from adacharge_b200.replay_fast import DeviceFleetReplay, FleetReplay
-
-    obj = _components(BENCH_OBJ)
     infra = caltech_acn_infrastructure()
-    kw = dict(n_sites=7, steps_per_day=288, days=2, seed0=40, mean_sessions=12, Tp=160, quantize=True, reallocate=True)
-    host, dev = FleetReplay(infra, obj, **kw), DeviceFleetReplay(infra, obj, **kw)
     sets = [np.asarray(a, dtype=float) for a in infra["allowable_pilots"]]
-    infeasible = 0
-    for t in list(range(80, 125)) + list(range(288 + 90, 288 + 110)):
-        a = host.step(t)
-        b = dev.step(t, want_first=True)
-        np.testing.assert_array_equal(a, b, err_msg=f"first-period pilots at step {t}")
+    n = dict(infeasible=0)
+
+    def on_step(t, host, dev, first):
         for i, s in enumerate(sets):
-            assert np.isin(a[:, i], s).all(), (t, i)
-        infeasible += int((engine.constraints_feasible(host.site, a[:, :, None], 0).cpu().numpy() == 0).sum())
-    dev.run(0, 0)
-    np.testing.assert_array_equal(dev.ev_dlv, host.ev_dlv)
-    np.testing.assert_array_equal(dev.prev_peak, host.prev_peak)
+            assert np.isin(first[:, i], s).all(), (t, i)
+        n["infeasible"] += int((engine.constraints_feasible(host.site, first[:, :, None], 0).cpu().numpy() == 0).sum())
+
+    host, _ = device_equals_host(infra, _components(BENCH_OBJ), list(range(80, 125)) + list(range(288 + 90, 288 + 110)), on_step, n_sites=7,
+                                 steps_per_day=288, days=2, seed0=40, mean_sessions=12, Tp=160, quantize=True, reallocate=True)
     assert min(host.stats.active_sites) < 7 < sum(host.stats.active_sites)  # idle sites occurred
     # floor_to_set rounds up to a member within 0.05 A, so the reference's quantised pilots can exceed a limit by that much
-    print(f"first columns over a network limit (within floor_to_set's 0.05 A): {infeasible} of {65 * 7}")
+    print(f"first columns over a network limit (within floor_to_set's 0.05 A): {n['infeasible']} of {65 * 7}")
 
 
 def test_quantized_quick_charge_day_delivers_energy(require_gpu):

@@ -18,9 +18,9 @@ from adacharge_b200.generators import caltech_acn_infrastructure, three_phase_ba
 from adacharge_b200.interface import SessionInfo
 from adacharge_b200.replay import EV
 from adacharge_b200.replay_fast import DeviceFleetReplay, FleetReplay
+from tests.replay_checks import BENCH, assert_as_good_as_cold_oracle, device_equals_host
 
 pytestmark = pytest.mark.gpu
-BENCH = [ab.ObjectiveComponent(ab.tou_energy_cost), ab.ObjectiveComponent(ab.total_energy, 0.3), ab.ObjectiveComponent(ab.demand_charge, 1 / 30)]
 SENT_F, SENT_I = -7.25, 77
 
 
@@ -106,29 +106,12 @@ def test_per_instance_warm_shifts(require_gpu, path):
 
 
 # ---------------------------------------------------------------------------------------------------- the replays
-def _dev_vs_host(max_recompute, uninterrupted, steps):
-    """Device replay == host replay at every step (applied pilots, recompute mask) and in the final state."""
-    infra = caltech_acn_infrastructure()
-    kw = dict(n_sites=7, steps_per_day=288, days=2, seed0=40, mean_sessions=12, Tp=160, max_recompute=max_recompute,
-              uninterrupted_charging=uninterrupted)
-    host, dev = FleetReplay(infra, BENCH, **kw), DeviceFleetReplay(infra, BENCH, **kw)
-    for t in steps:
-        a = host.step(t)
-        b = dev.step(t, want_first=True)
-        np.testing.assert_array_equal(a, b, err_msg=f"applied pilots at step {t}")
-        np.testing.assert_array_equal(host.recompute.astype(np.int32), dev._d["recompute"].cpu().numpy(), err_msg=f"recompute at step {t}")
-    dev.run(0, 0)
-    np.testing.assert_array_equal(dev.ev_dlv, host.ev_dlv)
-    np.testing.assert_array_equal(dev.prev_peak, host.prev_peak)
-    s = dev.summary()
-    assert s["solves"] == sum(host.stats.solved_sites) and s["unsolved"] == sum(host.stats.unsolved)
-    return host
-
-
 @pytest.mark.parametrize("max_recompute", [None, 3])
 @pytest.mark.parametrize("uninterrupted", [False, True])
 def test_device_replay_equals_host_replay(require_gpu, max_recompute, uninterrupted):
-    host = _dev_vs_host(max_recompute, uninterrupted, list(range(60, 150)) + list(range(288 + 80, 288 + 110)))
+    host, _ = device_equals_host(caltech_acn_infrastructure(), BENCH, list(range(60, 150)) + list(range(288 + 80, 288 + 110)), n_sites=7,
+                                 steps_per_day=288, days=2, seed0=40, mean_sessions=12, Tp=160, max_recompute=max_recompute,
+                                 uninterrupted_charging=uninterrupted)
     st = host.stats
     assert min(st.active_sites) < 7  # idle sites occurred
     assert sum(st.solved_sites) < sum(st.active_sites)  # sites skipped steps
@@ -148,11 +131,12 @@ def test_max_recompute_1_on_the_event_path_equals_the_default(require_gpu, cls):
         f.last_solve, f.recompute, f.shift = (engine._ptr(d[k]) for k in ("last_solve", "recompute", "shift"))
     for t in range(90, 130):
         np.testing.assert_array_equal(a.step(t), b.step(t), err_msg=f"step {t}")
-        if cls is DeviceFleetReplay:
-            assert (b._d["recompute"].cpu().numpy() == 1).all() and (b._d["shift"].cpu().numpy() == (91 if t == 90 else 1)).all()
-    a.run(0, 0), b.run(0, 0)
-    np.testing.assert_array_equal(a.ev_dlv, b.ev_dlv)
-    np.testing.assert_array_equal(a.prev_peak, b.prev_peak)
+        assert b.state()["recompute"].all()
+        if cls is DeviceFleetReplay:  # (each site's warm shift is not part of the state)
+            assert (b._d["shift"].cpu().numpy() == (91 if t == 90 else 1)).all()
+    sa, sb = a.state(), b.state()
+    for k in ("ev_dlv", "prev_peak"):
+        np.testing.assert_array_equal(sa[k], sb[k], err_msg=k)
 
 
 # ---------------------------------------------------------------------------------------------------- semantics
@@ -178,9 +162,9 @@ def test_solve_steps_and_applied_columns(require_gpu, monkeypatch, max_recompute
     dev, host = DeviceFleetReplay(infra, BENCH, **kw), FleetReplay(infra, BENCH, **kw)
     solved, sched, t_last, long_idle = [], None, None, False
     for t in range(288):
-        first = dev.step(t, want_first=True)
+        first = dev.step(t)
         np.testing.assert_array_equal(first, host.step(t), err_msg=f"step {t}")
-        if dev._d["recompute"].cpu().numpy()[0]:
+        if dev.state()["recompute"][0]:
             solved.append(t)
             sched, t_last = dev._ch.pilots[0].cpu().numpy().copy(), t
         c = t - t_last
@@ -189,17 +173,15 @@ def test_solve_steps_and_applied_columns(require_gpu, monkeypatch, max_recompute
         long_idle |= c >= dev.Tp
     assert solved == expect
     assert long_idle == (max_recompute is None)  # 30 -> 70 -> 250: more than Tp = 160 steps without a solve
-    dev.run(0, 0)
-    np.testing.assert_array_equal(dev.ev_dlv, host.ev_dlv)
-    assert dev.ev_dlv[:2].min() > 0
+    dlv = dev.state()["ev_dlv"]
+    np.testing.assert_array_equal(dlv, host.state()["ev_dlv"])
+    assert dlv[:2].min() > 0
 
 
 # ---------------------------------------------------------------------------------------------------- warm starts
 def test_old_warm_starts_match_a_cold_oracle_solve(require_gpu):
     """Solves warm-started from a state two or more columns old (max_recompute None) are ordinary MPC instances: the
     schedule is as good as a cold float64 oracle solve of the same step."""
-    from oracle import mpc
-
     spec = [("tou_energy_cost", 1, {}), ("total_energy", 0.3, {}), ("demand_charge", 1 / 30, {})]
     obj = [ab.ObjectiveComponent(getattr(ab, n), c, k) for n, c, k in spec]
     infra = three_phase_balanced_network(3, 30)
@@ -213,33 +195,11 @@ def test_old_warm_starts_match_a_cold_oracle_solve(require_gpu):
                                    int(rp.ev_dep[e]), current_time=t, max_rates=rp.ev_max[e]) for e in idx[s == b]] for b in range(rp.n_sites)}
         rp.step(t)
         R = rp._pb.rates.cpu().numpy().astype(np.float64)
-        st = rp._pb.status.cpu().numpy()
+        st = rp.state()["status"]
         for b in range(rp.n_sites):
             if rec[b] and since[b] >= 2 and had[b] and n_sess[b] > 0:
                 T = max(x.arrival_offset + x.remaining_time for x in sess[b])
                 cases.append((t, b, sess[b], float(peak[b]), R[b][:, :T], int(st[b])))
-    worst, compared, skipped = 0.0, 0, 0
-    for t, b, sess, prev_peak, R, status in cases:
-        assert status == 0, (t, b, status)
-        iface = ab.TestingInterface({"active_sessions": [], "infrastructure_info": infra, "current_time": t, "period": 15,
-                                     "prices": rp.prices, "demand_charge": rp.demand_charge, "prev_peak": prev_peak})
-        I = iface.infrastructure_info()
-        Ro = None
-        for ts in (1.0, 100.0):
-            try:
-                Ro = mpc.solve_mpc(spec, sess, I, iface, "SOC", False, None, prev_peak, tol_scale=ts)
-                break
-            except mpc.OracleInfeasible:
-                pass
-        if Ro is None:
-            skipped += 1
-            continue
-        compared += 1
-        f, fo = (mpc.evaluate_objective(X, spec, I, iface, sess, prev_peak) for X in (R, Ro))
-        mag = sum(abs(mpc.evaluate_objective(Ro, [o], I, iface, sess, prev_peak)) for o in spec)
-        assert abs(f - fo) <= 1e-4 * max(abs(fo), mag) + 1e-7, (t, b, f, fo, mag)
-        worst = max(worst, abs(f - fo) / max(abs(fo), mag))
-        v = mpc.violations(R, sess, I, iface)
-        assert v["infrastructure_rel"] <= 1e-5 and v["lb"] <= 0 and v["ub"] <= 0 and v["energy"] <= 1e-4, (t, b, v)
+    compared, skipped, worst = assert_as_good_as_cold_oracle(cases, spec, infra, 15, rp.prices, rp.demand_charge)
     assert compared >= 20 and skipped <= 3, (len(cases), compared, skipped)
     print(f"{compared} solves warm-started from states >= 2 columns old compared, worst objective error {worst:.1e} of the term scale")

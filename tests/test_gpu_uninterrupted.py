@@ -14,6 +14,7 @@ from adacharge_b200.algorithms_shim import apply_minimum_charging_rate, apply_up
 from adacharge_b200.batched import BatchedAdaptiveCharging, sessions_to_arrays
 from adacharge_b200.generators import caltech_acn_infrastructure, config_c2, session_generator, three_phase_balanced_network
 from oracle import mpc
+from tests.replay_checks import assert_as_good_as_cold_oracle, device_equals_host
 
 pytestmark = pytest.mark.gpu
 
@@ -269,36 +270,25 @@ def test_device_fleet_replay_equals_host(require_gpu, quantize, reallocate):
     """Two days of a congested fleet: first-period pilots, statuses, delivered energy and peaks of the device replay equal
     the host replay's, bit for bit; no site-step is infeasible; with continuous pilots every admitted EV gets at least
     its minimum."""
-    from adacharge_b200.replay_fast import DeviceFleetReplay, FleetReplay
+    n = dict(adm=0, ref=0)
 
-    infra = caltech_acn_infrastructure(transformer_cap=10)
-    kw = dict(n_sites=7, steps_per_day=288, days=2, seed0=40, mean_sessions=14, Tp=160, quantize=quantize, reallocate=reallocate,
-              uninterrupted_charging=True)
-    host, dev = FleetReplay(infra, _components(BENCH_OBJ), **kw), DeviceFleetReplay(infra, _components(BENCH_OBJ), **kw)
-    assert not dev._ch.lb_zero
-    n_adm = n_ref = 0
-    for t in list(range(80, 130)) + list(range(288 + 90, 288 + 115)):
-        a = host.step(t)
-        b = dev.step(t, want_first=True)
-        np.testing.assert_array_equal(a, b, err_msg=f"first-period pilots at step {t}")
+    def on_step(t, host, dev, first):
         h = {k: v.numpy() for k, v in host._pb.host.items()}
         act = h["n_sessions"] > 0
-        hs, ds = host._pb.status.cpu().numpy(), dev._ch.status.cpu().numpy()
-        np.testing.assert_array_equal(hs[act], ds[act], err_msg=f"statuses at step {t}")
-        assert not (hs[act] == _cabi.ACB_INFEASIBLE).any(), t
+        assert not (host.state()["status"][act] == _cabi.ACB_INFEASIBLE).any(), t
         for s in np.nonzero(act)[0]:
-            n = h["n_sessions"][s]
-            mn0, rows = h["sess_min0"][s, :n], h["sess_row"][s, :n]
-            n_adm += int((mn0 > 0).sum())
-            n_ref += int((h["sess_max0"][s, :n] == 0).sum())
+            k = h["n_sessions"][s]
+            mn0, rows = h["sess_min0"][s, :k], h["sess_row"][s, :k]
+            n["adm"] += int((mn0 > 0).sum())
+            n["ref"] += int((h["sess_max0"][s, :k] == 0).sum())
             if not quantize:
-                assert (a[s, rows] >= mn0 - 1e-4).all(), (t, s, a[s, rows], mn0)
-    dev.run(0, 0)
-    np.testing.assert_array_equal(dev.ev_dlv, host.ev_dlv)
-    np.testing.assert_array_equal(dev.prev_peak, host.prev_peak)
-    s = dev.summary()
-    assert s["site_steps"] == sum(host.stats.active_sites) and s["unsolved"] == sum(host.stats.unsolved)
-    assert n_adm > 0 and n_ref > 0, (n_adm, n_ref)
+                assert (first[s, rows] >= mn0 - 1e-4).all(), (t, s, first[s, rows], mn0)
+
+    _, dev = device_equals_host(caltech_acn_infrastructure(transformer_cap=10), _components(BENCH_OBJ),
+                                list(range(80, 130)) + list(range(288 + 90, 288 + 115)), on_step, n_sites=7, steps_per_day=288, days=2,
+                                seed0=40, mean_sessions=14, Tp=160, quantize=quantize, reallocate=reallocate, uninterrupted_charging=True)
+    assert not dev._ch.lb_zero
+    assert n["adm"] > 0 and n["ref"] > 0, n
 
 
 def test_warm_started_uninterrupted_steps_match_a_cold_oracle_solve(require_gpu):
@@ -312,7 +302,7 @@ def test_warm_started_uninterrupted_steps_match_a_cold_oracle_solve(require_gpu)
     rp = FleetReplay(infra, _components(spec), n_sites=3, steps_per_day=96, days=1, period=15, seed0=5, mean_sessions=7, Tp=64,
                      uninterrupted_charging=True)
     I = rp.info
-    worst, compared, skipped, with_min = 0.0, 0, 0, 0
+    cases, with_min = [], 0
     for t in range(28, 56):
         _, idx, s_of, pos, n_sess = rp._pack(t)
         prev_peak, owed = rp.prev_peak.copy(), rp.ev_req - rp.ev_dlv  # the state the step starts from
@@ -321,7 +311,7 @@ def test_warm_started_uninterrupted_steps_match_a_cold_oracle_solve(require_gpu)
             continue  # cold start
         mn0, mx0 = rp._limits0
         R_all = rp._pb.rates.cpu().numpy().astype(np.float64)
-        st_all = rp._pb.status.cpu().numpy()
+        st_all = rp.state()["status"]
         for site in np.nonzero(n_sess > 0)[0]:
             sess = []
             for j in np.nonzero(s_of == site)[0]:
@@ -331,27 +321,7 @@ def test_warm_started_uninterrupted_steps_match_a_cold_oracle_solve(require_gpu)
                                         current_time=t, min_rates=np.concatenate(([mn0[j]], np.zeros(rem - 1))),
                                         max_rates=np.concatenate(([mx0[j]], np.full(rem - 1, rp.ev_max[e])))))
             with_min += sum(s.min_rates[0] > 0 for s in sess)
-            assert st_all[site] == 0, (t, site, st_all[site])
-            T = mpc.horizon(sess)
-            R = R_all[site, :, :T]
-            iface = ab.TestingInterface({"active_sessions": [], "infrastructure_info": infra, "current_time": t, "period": 15,
-                                         "prices": rp.prices, "demand_charge": rp.demand_charge, "prev_peak": prev_peak[site]})
-            Ro = None
-            for ts in (1.0, 100.0):
-                try:
-                    Ro = mpc.solve_mpc(spec, sess, I, iface, "SOC", False, None, prev_peak[site], tol_scale=ts)
-                    break
-                except mpc.OracleInfeasible:
-                    pass
-            if Ro is None:
-                skipped += 1
-                continue
-            compared += 1
-            f, fo = (mpc.evaluate_objective(X, spec, I, iface, sess, prev_peak[site]) for X in (R, Ro))
-            mag = sum(abs(mpc.evaluate_objective(Ro, [o], I, iface, sess, prev_peak[site])) for o in spec)
-            assert abs(f - fo) <= 1e-4 * max(abs(fo), mag) + 1e-7, (t, site, f, fo, mag)
-            worst = max(worst, abs(f - fo) / max(abs(fo), mag))
-            v = mpc.violations(R, sess, I, iface)
-            assert v["infrastructure_rel"] <= 1e-5 and v["lb"] <= 1e-4 and v["ub"] <= 1e-4 and v["energy"] <= 1e-4, (t, site, v)
+            cases.append((t, site, sess, prev_peak[site], R_all[site, :, :mpc.horizon(sess)], st_all[site]))
+    compared, skipped, worst = assert_as_good_as_cold_oracle(cases, spec, infra, 15, rp.prices, rp.demand_charge, lb_tol=1e-4, ub_tol=1e-4)
     assert compared >= 20 and skipped <= 3 and with_min > 0, (compared, skipped, with_min)
     print(f"{compared} warm-started steps compared, worst objective error {worst:.1e} of the term scale")

@@ -14,7 +14,7 @@ import torch
 import adacharge_b200 as ab
 from adacharge_b200 import _cabi, engine
 from adacharge_b200.generators import session_generator, three_phase_balanced_network
-from tests.test_gpu_replay import device_vs_host_fleet_replay, warm_steps_vs_cold_oracle
+from tests.replay_checks import device_vs_host_fleet_replay, warm_steps_vs_cold_oracle
 
 pytestmark = pytest.mark.gpu
 BENCH = [ab.ObjectiveComponent(ab.tou_energy_cost), ab.ObjectiveComponent(ab.total_energy, 0.3), ab.ObjectiveComponent(ab.demand_charge, 1 / 30)]

@@ -56,16 +56,15 @@ def one_round(n_sites):
             torch.cuda.synchronize()
             ms[k] += a.elapsed_time(b)
             if rp.battery:  # every site solved (max_recompute 1): column 0 of this step's pilots is what was applied
-                w = torch.as_tensor(rp.volt * rp.period / 1e3 / 60, device=rp._d["rates"].device)
-                untaken[k] += float(((rp._ch.pilots[:, :, 0] - rp._d["rates"]) * w).sum())
+                p0 = rp._ch.pilots[:, :, 0].cpu().numpy()
+                untaken[k] += float(((p0 - rp.state()["rates"]) * (rp.volt * rp.period / 1e3 / 60)).sum())
     out = {}
     for k, rp in rps.items():
-        s = rp.summary()
-        st = rp.run(0, 0)
-        req = float(rp.ev_req.sum())
+        s, x = rp.summary(), rp.state()
+        req, dlv, peak_kw = float(rp.ev_req.sum()), float(x["ev_dlv"].sum()), x["prev_peak"] * rp.volt[0] / 1000
         out[k] = dict(solves=s["solves"], unsolved=s["unsolved"], iters_mean=s["iters_mean"], device_ms_per_day=ms[k],
-                      delivered_frac=float(rp.ev_dlv.sum() / req), delivered_kwh=float(rp.ev_dlv.sum()), requested_kwh=req,
-                      peak_kw_mean=float(st.peak_kw.mean()), peak_kw_max=float(st.peak_kw.max()), untaken_pilot_kwh=untaken[k])
+                      delivered_frac=dlv / req, delivered_kwh=dlv, requested_kwh=req,
+                      peak_kw_mean=float(peak_kw.mean()), peak_kw_max=float(peak_kw.max()), untaken_pilot_kwh=untaken[k])
     return out
 
 

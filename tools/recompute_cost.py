@@ -48,29 +48,28 @@ def one_round(n_sites):
     shifts = {k: [] for k in CONFIGS}
     for t in range(288):
         for k, rp in rps.items():
-            had = rp._d["had"].clone()
+            had = rp._d["had"].clone()  # (whether each site's last solve had sessions: solver bookkeeping, not simulator state)
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
             rp.step(t, want_first=False)
             b.record()
             torch.cuda.synchronize()
             ms[k] += a.elapsed_time(b)
-            if rp._event_driven:
-                rec, sh = rp._d["recompute"].cpu().numpy(), rp._d["shift"].cpu().numpy()
-            else:  # max_recompute 1: every site re-solves, from the previous step's state
-                rec, sh = np.ones(rp.n_sites, dtype=np.int32), np.ones(rp.n_sites, dtype=np.int32)
-            warm = (rec != 0) & (had.cpu().numpy() != 0) & (rp._ch.packed["n_sessions"].cpu().numpy() > 0)
+            # (the warm shifts are solver inputs, not simulator state; at max_recompute 1 every solve starts from the step before)
+            sh = rp._d["shift"].cpu().numpy() if rp._event_driven else np.ones(rp.n_sites, dtype=np.int32)
+            warm = rp.state()["recompute"] & (had.cpu().numpy() != 0) & (rp._ch.packed["n_sessions"].cpu().numpy() > 0)
             shifts[k] += sh[warm].tolist()
     out = {}
     for k, rp in rps.items():
-        s = rp.summary()
-        st = rp.run(0, 0)
+        s, x = rp.summary(), rp.state()
         req = float(rp.ev_req.sum())
+        req_site = np.maximum(np.bincount(rp.ev_site, weights=rp.ev_req, minlength=n_sites), 1e-9)
+        frac_site = np.bincount(rp.ev_site, weights=x["ev_dlv"], minlength=n_sites) / req_site
+        peak_kw = x["prev_peak"] * rp.volt[0] / 1000
         out[k] = dict(solves=s["solves"], solves_per_site_day=s["solves"] / n_sites, unsolved=s["unsolved"], device_ms_per_day=ms[k],
                       iters_mean=s["iters_mean"], warm_shift_mean=float(np.mean(shifts[k])) if shifts[k] else 0.0,
-                      warm_solves=len(shifts[k]), delivered_frac=float(rp.ev_dlv.sum() / req),
-                      delivered_frac_min_site=float(st.delivered_frac.min()), peak_kw_mean=float(st.peak_kw.mean()),
-                      peak_kw_max=float(st.peak_kw.max()))
+                      warm_solves=len(shifts[k]), delivered_frac=float(x["ev_dlv"].sum() / req),
+                      delivered_frac_min_site=float(frac_site.min()), peak_kw_mean=float(peak_kw.mean()), peak_kw_max=float(peak_kw.max()))
     return out
 
 

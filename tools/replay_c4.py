@@ -51,7 +51,7 @@ def run(a, b):
     for t in range(a, b):
         for rp, st in zip(rps, streams):
             with torch.cuda.stream(st):
-                rp.step(t, want_first=False) if on_device else rp.step(t)
+                rp.step(t, want_first=False)
 
 
 def summary():
@@ -70,9 +70,10 @@ run(t0 + 3, t1)
 torch.cuda.synchronize()
 wall = time.perf_counter() - w0
 s1 = summary()
+frac = 0.0  # sum over the sites of the delivered fraction of the requested energy
 for rp in rps:
-    rp.run(0, 0)  # (device replay: reads the EV state back; no steps)
-frac = float(np.sum([np.sum(rp.stats.delivered_frac) for rp in rps])) if all(rp.stats.delivered_frac is not None for rp in rps) else float("nan")
+    req = np.bincount(rp.ev_site, weights=rp.ev_req, minlength=rp.n_sites)
+    frac += float(np.sum(np.bincount(rp.ev_site, weights=rp.state()["ev_dlv"], minlength=rp.n_sites) / np.maximum(req, 1e-9)))
 vals = torch.tensor([s1["site_steps"] - s0["site_steps"], s1["unsolved"] - s0["unsolved"], s1["iters"] - s0["iters"], frac], device="cuda", dtype=torch.float64)
 wt = torch.tensor([wall], device="cuda", dtype=torch.float64)
 if world > 1:
